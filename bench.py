@@ -54,7 +54,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip bf16_mode / fp32_mode / torch_b200 / preprocessing / drop-in API legs")
     ap.add_argument("--save-doc0", default="", help="(reference arm) also write the map and the uint8 image of document 0 to this .npz")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="(our arm, rank 0) after the timed steps, write what the last timed step computed as DIR/<name>.npy in float32: "
+                         "image (the dewarped photo that run_device returns, or a fixed seeded sample of it past 64 MiB in all) and "
+                         "map64 (the sampled backward map it was unwarped with: an intermediate result, kept for finer comparison)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return a
 
 
 def workload_name(a):
@@ -125,6 +132,25 @@ def measured_peaks():
 def algorithmic_gflop_per_doc(S, n_batch):
     """SURVEY.md §8(d): live, hoisted FLOPs only."""
     return 101.87 + n_batch * S * 262.52
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes each array as out_dir/<name>.npy in float32, smallest first, whole while it fits in what is left of DUMP_BYTES.  An
+    array that does not fit is written as a 1-D sample at fixed positions (seeded, sorted, identical from run to run), so that two
+    builds of the project can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES // 4 - 1024 * len(arrays)                          # float32 elements, minus room for the .npy headers
+    for name, t in sorted(arrays.items(), key=lambda kv: kv[1].numel()):
+        x = t.detach().float().cpu()
+        if x.numel() > left:
+            idx = torch.randperm(x.numel(), generator=torch.Generator().manual_seed(0))[:left].sort().values
+            x = x.flatten()[idx]
+        left -= x.numel()
+        np.save(os.path.join(out_dir, name + ".npy"), x.numpy())
 
 
 def psnr_db(a: torch.Tensor, b: torch.Tensor) -> float:
@@ -370,7 +396,7 @@ def run_ours(a):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def measure(precision, steps, warmup, with_e2e=True):
+    def measure(precision, steps, warmup, with_e2e=True, keep_last=False):
         pipe = DewarpPipeline(model, diffusion_steps=a.diffusion_steps, n_batch=a.n_batch, docs=a.docs, height=a.height, width=a.width,
                               precision=precision)
 
@@ -413,6 +439,8 @@ def run_ours(a):
 
         ms_dev, launches = timed(lambda i: pipe.run_device(dev_sets[i % n_var]))           # (1) device-resident inputs
         res = {"pipe": pipe, "ms_dev": ms_dev, "launches": launches}
+        if keep_last:                                                      # the e2e legs below overwrite pipe.map64
+            res["last"] = {"map64": pipe.map64.clone(), "image": pipe.out_u8.clone()}
         if with_e2e:
             res["ms_e2e"], _ = timed(lambda i: pipe.run_host(host_sets[i % n_var]))        # (2) synchronous public-API calls: latency
             res["ms_e2e_pipe"] = timed_e2e_pipelined()                                     # (3) two batches outstanding: throughput
@@ -427,8 +455,10 @@ def run_ours(a):
 
     sampler = ClockSampler(local) if rank == 0 else None
     time.sleep(0.05)
-    main = measure(a.precision, a.steps, a.warmup)
+    main = measure(a.precision, a.steps, a.warmup, keep_last=bool(a.dump_outputs) and rank == 0)
     clocks = sampler.stop() if sampler else None
+    if "last" in main:
+        dump_outputs(a.dump_outputs, main.pop("last"))
     pipe = main["pipe"]
     tot_dev, tot_e2e = reduce_max([sum(main["ms_dev"]) / 1e3, min(sum(main["ms_e2e"]), main["ms_e2e_pipe"]) / 1e3])
     docs_total = a.docs * a.steps * world

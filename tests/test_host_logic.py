@@ -166,6 +166,30 @@ def test_bench_reference_arm_contract():
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
 
 
+def test_bench_dump_outputs_whole_or_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: small arrays are written whole in float32; one past the 64 MiB budget becomes the same seeded
+    sample of distinct positions on every call, and the files stay under the budget together."""
+    import bench
+    g = torch.Generator().manual_seed(1)
+    map64 = torch.rand(2, 2, 64, 64, generator=g) * 2 - 1
+    image = torch.randint(0, 256, (2, 1500, 2000, 3), generator=g, dtype=torch.uint8)        # 72 MiB as float32
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"map64": map64, "image": image})
+    m = np.load(tmp_path / "a" / "map64.npy")
+    assert m.dtype == np.float32 and np.array_equal(m, map64.numpy())
+    ia, ib = np.load(tmp_path / "a" / "image.npy"), np.load(tmp_path / "b" / "image.npy")
+    assert ia.dtype == np.float32 and ia.ndim == 1 and np.array_equal(ia, ib)
+    assert set(np.unique(ia)) <= set(range(256)) and len(np.unique(ia)) == 256
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64 << 20
+    ramp = torch.arange(bench.DUMP_BYTES // 4 - 1000, dtype=torch.int32)      # just past the budget, every value exact in float32
+    bench.dump_outputs(str(tmp_path / "r"), {"ramp": ramp})
+    r = np.load(tmp_path / "r" / "ramp.npy")
+    assert r.size < ramp.numel() and np.all(np.diff(r) > 0)                          # sorted positions, none drawn twice
+    small = torch.randint(0, 256, (1, 96, 128, 3), generator=g, dtype=torch.uint8)
+    bench.dump_outputs(str(tmp_path / "c"), {"map64": map64[:1], "image": small})
+    assert np.array_equal(np.load(tmp_path / "c" / "image.npy"), small.float().numpy())
+
+
 def test_committed_bench_lines_carry_the_contract():
     """profiles/r1_bench_lines.jsonl: every line of our arm has value / e2e / roofline / clocks / gpu_launches."""
     import json
