@@ -43,6 +43,10 @@ class Weights(C.Structure):
                 ("fin_ada", Mat), ("fin_ada_b", _vp), ("pyr_h", Mat * 7)]
 
 
+class UnwarpDoc(C.Structure):
+    _fields_ = [("photo", _vp), ("out", _vp), ("H", C.c_int32), ("W", C.c_int32)]
+
+
 # name -> (restype, argtypes); mirrors include/dvd_b200.h one to one
 _i, _f, _sz = C.c_int, C.c_float, C.c_size_t
 _WP = C.POINTER(Weights)
@@ -54,6 +58,9 @@ SIGNATURES = {
     "dvd_unwarp_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _f, _vp]),
     "dvd_unwarp_u8": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _f, _vp]),
     "dvd_unwarp_f32_u8": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _f, _vp]),
+    "dvd_unwarp_table_bytes": (_sz, [_i]),
+    "dvd_unwarp_u8_plan": (_i, [C.POINTER(UnwarpDoc), _i, _i, _i, _i, _f, _vp, _sz, C.POINTER(C.c_longlong)]),
+    "dvd_unwarp_u8_mixed": (_i, [_vp, _i, _vp, _vp]),
     "dvd_grid_sample_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "dvd_fullres_grid_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _f, _vp]),
     "dvd_workspace_bytes": (_sz, [_i, _i, _i]),

@@ -123,29 +123,34 @@ constexpr int TILE_W = 128, TILE_H = 8;   // 32 x 8 threads, 4 px per thread
 // memory (128 + 8 entries), so the per-pixel path is: 8 coarse-map loads, 2 bilinear blends, affine, tap weights and
 // 4*C gathers.  Tiles whose four taps are all inside the photo for every pixel of the warp (the common case) take an
 // unpredicated path so that the 4*C*4 gathers of a thread are issued back to back.
+//
+// The per-tile bodies (unwarp_tile, unwarp_tile_fast) take photo / output / map bases, a geometry and the tile (x, y, image b):
+// the fixed-size kernels pass the batch bases and blockIdx (so their address arithmetic is the one they always had), the
+// persistent mixed-size kernel one document's bases, its own tile walk and b = 0.  A body never returns early (the persistent
+// loop has barriers): rows past the photo skip the work and still reach every __syncthreads.
 template <int IN_U8, int OUT_U8, int C>
-__global__ void __launch_bounds__(256) k_unwarp(const void* __restrict__ photo_, const float* __restrict__ map,
-                                                void* __restrict__ out_, UnwarpGeom g) {
+__device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, const float* __restrict__ map, void* __restrict__ out_,
+                                            const UnwarpGeom& g, unsigned tx, unsigned ty, unsigned b) {
   __shared__ float s_bx[TILE_W], s_lx[TILE_W], s_by[TILE_H], s_ly[TILE_H];
   __shared__ int s_x0[TILE_W], s_y0[TILE_H];
   const int tid = threadIdx.y * 32 + threadIdx.x;
   if (tid < TILE_W) {
-    const int j = min(blockIdx.x * TILE_W + tid, g.W - 1);
+    const int j = min(tx * TILE_W + tid, g.W - 1);
     int x0, xp; float l0, l1;
     up_coeff(g.sx, j, g.mw, x0, xp, l0, l1);
     s_x0[tid] = x0 | (xp << 16); s_lx[tid] = l1; s_bx[tid] = base_ramp(g.bx, j);
   } else if (tid < TILE_W + TILE_H) {
     const int r = tid - TILE_W;
-    const int i = min(blockIdx.y * TILE_H + r, g.H - 1);
+    const int i = min(ty * TILE_H + r, g.H - 1);
     int y0, yp; float l0, l1;
     up_coeff(g.sy, i, g.mh, y0, yp, l0, l1);
     s_y0[r] = y0 | (yp << 16); s_ly[r] = l1; s_by[r] = base_ramp(g.by, i);
   }
   __syncthreads();
-  const int b = blockIdx.z;
-  const int i = blockIdx.y * TILE_H + threadIdx.y;
-  const int j0 = (blockIdx.x * (TILE_W / 4) + threadIdx.x) * 4;
-  if (i >= g.H || j0 >= g.W) return;
+  const int i = ty * TILE_H + threadIdx.y;
+  const int j0 = (tx * (TILE_W / 4) + threadIdx.x) * 4;
+  // a warp is one tile row; its lanes left of the right edge are a prefix of the warp, and only they take part in the vote below
+  if (i < g.H && j0 < g.W) {
   const int W = g.W, H = g.H;
   const int plane = H * W;                                      // < 2^31 elements per image (checked on the host)
   const float* __restrict__ mapb = map + (size_t)b * 2 * g.mh * g.mw;
@@ -177,7 +182,8 @@ __global__ void __launch_bounds__(256) k_unwarp(const void* __restrict__ photo_,
     if (j0 + p >= W) { vmask[p] = 0; off[p] = 0; }
   }
   float res[C][4];
-  if (__all_sync(0xffffffffu, inside) && j0 + 3 < W) {
+  const int live = min(32, (W - (int)tx * TILE_W + 3) / 4);
+  if (__all_sync(live == 32 ? 0xffffffffu : (1u << live) - 1u, inside) && j0 + 3 < W) {
     // ---- fast path: every tap of every pixel of this warp is inside the photo
     if (IN_U8) {
       const uint8_t* __restrict__ ph = (const uint8_t*)photo_ + (size_t)b * plane * C;
@@ -265,6 +271,13 @@ __global__ void __launch_bounds__(256) k_unwarp(const void* __restrict__ photo_,
       }
     }
   }
+  }
+}
+
+template <int IN_U8, int OUT_U8, int C>
+__global__ void __launch_bounds__(256) k_unwarp(const void* __restrict__ photo_, const float* __restrict__ map,
+                                                void* __restrict__ out_, UnwarpGeom g) {
+  unwarp_tile<IN_U8, OUT_U8, C>(photo_, map, out_, g, blockIdx.x, blockIdx.y, blockIdx.z);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -278,16 +291,14 @@ __global__ void __launch_bounds__(256) k_unwarp(const void* __restrict__ photo_,
 constexpr int UW_WIN = 16;
 
 template <int IN_U8, int OUT_U8, int C>
-__global__ void __launch_bounds__(256) k_unwarp_fast(const void* __restrict__ photo_, const float* __restrict__ map,
-                                                     void* __restrict__ out_, UnwarpGeom g) {
+__device__ __forceinline__ void unwarp_tile_fast(const void* __restrict__ photo_, const float* __restrict__ map,
+                                                 void* __restrict__ out_, const UnwarpGeom& g, unsigned tx, unsigned ty, unsigned b) {
   __shared__ float s_bx[TILE_W], s_lx[TILE_W], s_by[TILE_H], s_ly[TILE_H];
   __shared__ int s_kx[TILE_W], s_y0[TILE_H];
   __shared__ float s_v[2][TILE_H][UW_WIN];
-  __shared__ int s_wx0;
   const int tid = threadIdx.y * 32 + threadIdx.x;
-  const int b = blockIdx.z;
   const float* __restrict__ mapb = map + (size_t)b * 2 * g.mh * g.mw;
-  const int jt0 = blockIdx.x * TILE_W;
+  const int jt0 = tx * TILE_W;
   // window of map columns touched by this tile: x0(first column) .. x0(last column) + 1
   int wx0;
   {
@@ -301,7 +312,7 @@ __global__ void __launch_bounds__(256) k_unwarp_fast(const void* __restrict__ ph
     s_kx[tid] = (x0 - wx0) | (xp << 16); s_lx[tid] = l1; s_bx[tid] = base_ramp(g.bx, j);
   } else if (tid < TILE_W + TILE_H) {
     const int r = tid - TILE_W;
-    const int i = min(blockIdx.y * TILE_H + r, g.H - 1);
+    const int i = min(ty * TILE_H + r, g.H - 1);
     int y0, yp; float l0, l1;
     up_coeff(g.sy, i, g.mh, y0, yp, l0, l1);
     s_y0[r] = y0 | (yp << 16); s_ly[r] = l1; s_by[r] = base_ramp(g.by, i);
@@ -316,10 +327,10 @@ __global__ void __launch_bounds__(256) k_unwarp_fast(const void* __restrict__ ph
     s_v[ch][r][k] = l0 * __ldg(m) + l1 * __ldg(m + yp * g.mw);
   }
   __syncthreads();
-  const int i = blockIdx.y * TILE_H + threadIdx.y;
+  const int i = ty * TILE_H + threadIdx.y;
   const int j0 = jt0 + threadIdx.x;                       // pixel p of this thread is column j0 + 32*p: a warp-level
-  if (i >= g.H) return;                                   // load/store then covers 32 CONSECUTIVE pixels (one 128-byte line);
-                                                          // whole warps exit (a warp is one tile row): *_sync masks stay valid
+  if (i < g.H) {                                          // load/store then covers 32 CONSECUTIVE pixels (one 128-byte line);
+                                                          // whole warps skip (a warp is one tile row): *_sync masks stay valid
   const int W = g.W, H = g.H;
   const int plane = H * W;
   const float byv = s_by[threadIdx.y];
@@ -430,6 +441,13 @@ __global__ void __launch_bounds__(256) k_unwarp_fast(const void* __restrict__ ph
         if (j0 + 32 * p < W) __stcs(o + 32 * p, res[c][p]);
     }
   }
+  }
+}
+
+template <int IN_U8, int OUT_U8, int C>
+__global__ void __launch_bounds__(256) k_unwarp_fast(const void* __restrict__ photo_, const float* __restrict__ map,
+                                                     void* __restrict__ out_, UnwarpGeom g) {
+  unwarp_tile_fast<IN_U8, OUT_U8, C>(photo_, map, out_, g, blockIdx.x, blockIdx.y, blockIdx.z);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -828,6 +846,110 @@ static int launch_unwarp(const void* photo, const float* map, void* out, int B, 
   return 0;
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Mixed-size batch (uint8 HWC): one persistent launch walks the 128 x 8 tiles of documents of different sizes.  The caller plans a
+// table on the host (dvd_unwarp_u8_plan) and uploads it; the grid depends only on the device, so a CUDA graph captured once
+// serves every batch composition planned into the same device table.
+struct MixedTableHeader {
+  int32_t n_docs, total_tiles, C, pad;
+};
+struct MixedDoc {                         // 64 bytes
+  const uint8_t* photo;
+  uint8_t* out;
+  UnwarpGeom g;                           // make_geom(): the same coefficients as the fixed-size launch
+  int32_t tiles_x, tile_begin, fast;      // tile_begin: prefix sum of cdiv(W, 128) * cdiv(H, 8)
+};
+static_assert(sizeof(MixedTableHeader) == 16 && sizeof(MixedDoc) == 64, "mixed unwarp table layout");
+constexpr int MIXED_MAX_TILES = 1 << 30;  // tile indices and t + gridDim.x stay inside int32
+
+template <int C>
+__global__ void __launch_bounds__(256) k_unwarp_u8_mixed(const MixedTableHeader* __restrict__ hdr, const MixedDoc* __restrict__ docs,
+                                                         const float* __restrict__ map) {
+  const int n_docs = __ldg(&hdr->n_docs), total = __ldg(&hdr->total_tiles);
+  if (__ldg(&hdr->C) != C) return;        // planned for another channel count: write nothing (uniform over the grid)
+  for (int t = blockIdx.x; t < total; t += gridDim.x) {
+    // the document of tile t: the last one whose tile_begin <= t (empty documents own no tile and are never selected)
+    int lo = 0, hi = n_docs - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (__ldg(&docs[mid].tile_begin) <= t) lo = mid; else hi = mid - 1;
+    }
+    const MixedDoc& d = docs[lo];
+    const UnwarpGeom g = d.g;
+    const int r = t - d.tile_begin, ty = r / d.tiles_x, tx = r - ty * d.tiles_x;
+    const float* mapb = map + (size_t)lo * 2 * g.mh * g.mw;          // document d reads map row d
+    __syncthreads();                      // the previous tile's threads are done reading the shared tables the prologue rewrites
+    if (d.fast) unwarp_tile_fast<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0);
+    else        unwarp_tile<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0);
+  }
+}
+
+static size_t mixed_table_bytes(int max_docs) {
+  return max_docs < 0 ? 0 : sizeof(MixedTableHeader) + (size_t)max_docs * sizeof(MixedDoc);
+}
+
+static int plan_mixed(const dvd_unwarp_doc_t* docs_host, int n_docs, int C, int mh, int mw, float affine, void* table_host,
+                      size_t table_bytes, long long* total_tiles) {
+  DVD_REQUIRE(n_docs >= 0 && (n_docs == 0 || docs_host) && table_host, "unwarp_u8_plan: n_docs=%d, docs %p, table %p", n_docs,
+              (const void*)docs_host, table_host);
+  DVD_REQUIRE(table_bytes >= mixed_table_bytes(n_docs), "unwarp_u8_plan: table of %zu bytes is too small for %d documents (%zu needed)",
+              table_bytes, n_docs, mixed_table_bytes(n_docs));
+  DVD_REQUIRE(C >= 1 && C <= 4, "unwarp_u8_plan: C=%d outside 1..4", C);
+  DVD_REQUIRE(mh >= 1 && mw >= 1 && mh < 65536 && mw < 65536, "unwarp_u8_plan: bad map size %dx%d", mh, mw);
+  MixedTableHeader* hdr = static_cast<MixedTableHeader*>(table_host);
+  MixedDoc* recs = reinterpret_cast<MixedDoc*>(hdr + 1);
+  long long tiles = 0;
+  for (int d = 0; d < n_docs; ++d) {
+    const dvd_unwarp_doc_t& in = docs_host[d];
+    DVD_REQUIRE(in.H >= 0 && in.W >= 0, "unwarp_u8_plan: document %d has a negative size %dx%d", d, in.H, in.W);
+    DVD_REQUIRE((long long)in.H * in.W * C < (1ll << 31), "unwarp_u8_plan: document %d (%dx%dx%d) is too large for 32-bit offsets", d,
+                in.H, in.W, C);
+    const bool empty = in.H == 0 || in.W == 0;
+    DVD_REQUIRE(empty || (in.photo && in.out), "unwarp_u8_plan: document %d has a null photo or output pointer", d);
+    MixedDoc r;
+    r.photo = in.photo; r.out = in.out;
+    r.g = make_geom(in.H, in.W, mh, mw, affine);
+    r.tiles_x = empty ? 0 : cdiv(in.W, TILE_W);
+    r.tile_begin = (int32_t)tiles;
+    r.fast = (int)(127.0f * r.g.sx) + 3 <= UW_WIN && in.W > 1 && in.H > 1;     // the condition launch_unwarp uses
+    tiles += empty ? 0 : (long long)r.tiles_x * cdiv(in.H, TILE_H);
+    DVD_REQUIRE(tiles < MIXED_MAX_TILES, "unwarp_u8_plan: more than %d tiles in one batch", MIXED_MAX_TILES);
+    recs[d] = r;
+  }
+  *hdr = MixedTableHeader{n_docs, (int32_t)tiles, C, 0};
+  if (total_tiles) *total_tiles = tiles;
+  return 0;
+}
+
+static int launch_unwarp_u8_mixed(const void* table, int C, const float* map, cudaStream_t st) {
+  DVD_REQUIRE(table && map, "unwarp_u8_mixed: null pointer");
+  DVD_REQUIRE(C >= 1 && C <= 4, "unwarp_u8_mixed: C=%d outside 1..4", C);
+  const MixedTableHeader* hdr = static_cast<const MixedTableHeader*>(table);
+  const MixedDoc* docs = reinterpret_cast<const MixedDoc*>(hdr + 1);
+  int dev = 0, n_sm = 0;
+  DVD_CUDA(cudaGetDevice(&dev));
+  DVD_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+  DVD_REQUIRE(dev < 64, "unwarp_u8_mixed: device %d", dev);
+#define DVD_UNWARP_MIXED(CC)                                                                                                       \
+  do {                                                                                                                             \
+    static int per_sm[64] = {};                   /* per device: occupancy of this instantiation */                                \
+    if (!per_sm[dev]) {                                                                                                            \
+      DVD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[dev], k_unwarp_u8_mixed<CC>, 256, 0));                        \
+      DVD_REQUIRE(per_sm[dev] >= 1, "unwarp_u8_mixed: kernel does not fit an SM");                                                 \
+    }                                                                                                                              \
+    k_unwarp_u8_mixed<CC><<<n_sm * per_sm[dev], dim3(32, 8), 0, st>>>(hdr, docs, map);                                             \
+  } while (0)
+  switch (C) {
+    case 1: DVD_UNWARP_MIXED(1); break;
+    case 2: DVD_UNWARP_MIXED(2); break;
+    case 3: DVD_UNWARP_MIXED(3); break;
+    default: DVD_UNWARP_MIXED(4); break;
+  }
+#undef DVD_UNWARP_MIXED
+  DVD_LAUNCH_CHECK("k_unwarp_u8_mixed");
+  return 0;
+}
+
 }  // namespace dvd
 
 using namespace dvd;
@@ -843,6 +965,14 @@ extern "C" int dvd_unwarp_u8(const uint8_t* photo, const float* map, uint8_t* ou
 extern "C" int dvd_unwarp_f32_u8(const float* photo, const float* map, uint8_t* out, int B, int C, int H, int W, int mh, int mw,
                                  float affine, void* stream) {
   return launch_unwarp<0, 1>(photo, map, out, B, C, H, W, mh, mw, affine, (cudaStream_t)stream);
+}
+extern "C" size_t dvd_unwarp_table_bytes(int max_docs) { return mixed_table_bytes(max_docs); }
+extern "C" int dvd_unwarp_u8_plan(const dvd_unwarp_doc_t* docs_host, int n_docs, int C, int mh, int mw, float affine, void* table_host,
+                                  size_t table_bytes, long long* total_tiles) {
+  return plan_mixed(docs_host, n_docs, C, mh, mw, affine, table_host, table_bytes, total_tiles);
+}
+extern "C" int dvd_unwarp_u8_mixed(const void* table, int C, const float* map, void* stream) {
+  return launch_unwarp_u8_mixed(table, C, map, (cudaStream_t)stream);
 }
 extern "C" int dvd_fullres_grid_f32(const float* map, float* grid, int B, int H, int W, int mh, int mw, float affine,
                                     void* stream) {

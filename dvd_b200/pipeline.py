@@ -4,6 +4,10 @@
 (train_settings/dvd/evaluation.py:245-268 sampling, :300-306 upsample/affine, :317-318 unwarp) for
 a fixed batch of ``docs`` documents per call.  Everything between the inputs and the dewarped
 image runs in libdvd_b200; torch only owns the buffers and the stream.
+
+With ``max_pixels=P`` the pipeline takes photos of different sizes in one batch (mixed-size mode): ``photo_u8`` is then a list of
+uint8 HWC tensors whose pixel counts sum to at most P, the results are a list of uint8 HWC images, and one unwarp launch, captured
+once per set of buffers, serves every composition of sizes.
 """
 from __future__ import annotations
 
@@ -16,13 +20,16 @@ import torch
 from . import _lib
 from .model import DiT
 from .sampler import create_gaussian_diffusion
-from .unwarp import AFFINE
+from .unwarp import AFFINE, plan_mixed, table_bytes
 
 
 class DewarpPipeline:
     def __init__(self, model: DiT, diffusion_steps: int = 3, n_batch: int = 2, docs: int = 1, height: int = 1500, width: int = 2000,
-                 noise_schedule: str = "cosine", precision: str | None = None):
+                 noise_schedule: str = "cosine", precision: str | None = None, max_pixels: int | None = None):
         self.model, self.docs, self.n_batch, self.H, self.W = model, docs, n_batch, height, width
+        self.max_pixels = max_pixels
+        if max_pixels is not None and max_pixels < 1:
+            raise ValueError(f"max_pixels must be positive, got {max_pixels}")
         self.precision = precision or model.precision
         self.dev = model.device
         if self.dev.type != "cuda":
@@ -33,13 +40,19 @@ class DewarpPipeline:
         with torch.cuda.device(self.dev):
             self._bind_engine()
             z = lambda *s, dt=torch.float32: torch.zeros(s, dtype=dt, device=self.dev)
+            # mixed-size mode: photos and outputs live in byte arenas, each document at a 16-byte aligned offset
+            img = (docs, height, width, 3) if max_pixels is None else (3 * max_pixels + 16 * docs,)
             self.buf = {"y512": z(docs, 3, 512, 512), "mask_cat": z(docs, 1, 512, 512), "mask_y512": z(docs, 384, 64, 64),
                         "line_msk": z(docs, 64, 64, 64), "x_T": z(docs * n_batch, 2, 64, 64),
-                        "photo_u8": z(docs, height, width, 3, dt=torch.uint8)}
+                        "photo_u8": z(*img, dt=torch.uint8)}
             self.init_flow0 = z(docs, 2, 64, 64)                       # evaluation.py:180 (use_init_flow=False)
             self.map64 = z(docs, 2, 64, 64)
-            self.out_u8 = z(docs, height, width, 3, dt=torch.uint8)
-            self.out_host = torch.empty((docs, height, width, 3), dtype=torch.uint8).pin_memory()
+            self.out_u8 = z(*img, dt=torch.uint8)
+            self.out_host = torch.empty(img, dtype=torch.uint8).pin_memory()
+            if max_pixels is not None:                                # run_device's unwarp table (host plan -> device copy)
+                self._table = z(table_bytes(docs), dt=torch.uint8)
+                self._table_host = torch.empty(table_bytes(docs), dtype=torch.uint8).pin_memory()
+                self._ev_table = torch.cuda.Event()
         self.h2d_bytes = sum(v.numel() * v.element_size() for v in self.buf.values())
         self.d2h_bytes = self.out_u8.numel()
         self.use_graph = os.environ.get("DVD_NO_GRAPH", "0") != "1"
@@ -74,6 +87,39 @@ class DewarpPipeline:
         _lib.check(self.lib.dvd_unwarp_u8(_lib.ptr(d["photo_u8"]), _lib.ptr(self.map64), _lib.ptr(out), self.docs, 3,
                                           self.H, self.W, 64, 64, AFFINE, _lib.stream_ptr()), "dvd_unwarp_u8")
 
+    def _enqueue_unwarp_mixed(self, d: dict):
+        """mixed-size unwarp of the batch planned into the device table d["table"] (one launch whatever the composition)."""
+        _lib.check(self.lib.dvd_unwarp_u8_mixed(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), "dvd_unwarp_u8_mixed")
+
+    def _check_photos(self, photos, device: torch.device, lo: int) -> list:
+        """Validates the photos of a mixed-size batch (lo..docs uint8 HWC RGB tensors on `device`, at most max_pixels in all)."""
+        if not isinstance(photos, (list, tuple)):
+            raise ValueError("mixed-size mode (max_pixels) takes photo_u8 as a list of uint8 HWC tensors")
+        if not lo <= len(photos) <= self.docs:
+            raise ValueError(f"{len(photos)} photos: this call takes {lo}..{self.docs}" if lo < self.docs else
+                             f"{len(photos)} photos: this call takes exactly {self.docs}")
+        for i, p in enumerate(photos):
+            if not isinstance(p, torch.Tensor) or p.dtype != torch.uint8 or p.dim() != 3 or p.shape[2] != 3:
+                raise ValueError(f"photo {i}: expected a uint8 HWC tensor with 3 channels, got "
+                                 f"{getattr(p, 'dtype', type(p))} {tuple(getattr(p, 'shape', ()))}")
+            if not p.is_contiguous():
+                raise ValueError(f"photo {i} is not contiguous")
+            if p.device != device:
+                raise ValueError(f"photo {i} is on {p.device}, this call takes photos on {device}")
+        px = sum(p.shape[0] * p.shape[1] for p in photos)
+        if px > self.max_pixels:
+            raise ValueError(f"the batch has {px} pixels, more than max_pixels={self.max_pixels}")
+        return list(photos)
+
+    @staticmethod
+    def _arena_views(arena: torch.Tensor, photos) -> list:
+        """one [H,W,3] view per photo, packed at 16-byte aligned offsets"""
+        views, off = [], 0
+        for p in photos:
+            views.append(arena[off:off + p.numel()].view(p.shape))
+            off = (off + p.numel() + 15) & ~15
+        return views
+
     def _graph(self, which: str, d: dict, keys, fn):
         """CUDA graph of `fn(d)` for this set of input buffers (captured once, replayed afterwards)."""
         key = (which,) + tuple(d[k].data_ptr() for k in keys)
@@ -101,14 +147,31 @@ class DewarpPipeline:
 
     SAMPLING_KEYS = ("y512", "mask_cat", "mask_y512", "line_msk", "x_T")
 
-    def run_device(self, d: dict) -> torch.Tensor:
+    def run_device(self, d: dict):
         """The ~230 kernel launches of one batch are captured once per set of input buffers into two CUDA graphs (sampling,
-        unwarp) and replayed (the library never allocates or synchronises, so every entry point is capturable)."""
+        unwarp) and replayed (the library never allocates or synchronises, so every entry point is capturable).
+
+        Mixed-size mode: d["photo_u8"] is a list of exactly `docs` uint8 HWC photos on the pipeline's device (read in place);
+        returns a list of views into the device output arena, overwritten by the next call."""
         self._check_weights()
+        if self.max_pixels is not None:
+            return self._run_device_mixed(d)
         with torch.cuda.device(self.dev):
             self._run("sampling", d, self.SAMPLING_KEYS, self._enqueue_sampling)
             self._run("unwarp", d, ("photo_u8",), self._enqueue_unwarp)
         return self.out_u8
+
+    def _run_device_mixed(self, d: dict) -> list:
+        photos = self._check_photos(d["photo_u8"], self.dev, self.docs)
+        with torch.cuda.device(self.dev):
+            self._run("sampling", d, self.SAMPLING_KEYS, self._enqueue_sampling)
+            outs = self._arena_views(self.out_u8, photos)
+            self._ev_table.synchronize()                               # the previous upload has read the pinned table
+            plan_mixed(self._table_host, photos, outs, 64, 64)
+            self._table.copy_(self._table_host, non_blocking=True)
+            self._ev_table.record()
+            self._run("unwarp", {"table": self._table}, ("table",), self._enqueue_unwarp_mixed)
+        return outs
 
     # ---- pinned-host inputs -> host uint8 image (H2D and D2H inside the call)
     def _make_slots(self):
@@ -120,16 +183,24 @@ class DewarpPipeline:
         for _ in range(2):
             buf = {k: torch.empty_like(v) for k, v in self.buf.items()}
             buf["out_u8"] = torch.empty_like(self.out_u8)
-            self._slots.append({"buf": buf, "out_host": torch.empty_like(self.out_host).pin_memory(), "used": False,
-                                "ev_in": torch.cuda.Event(), "ev_photo": torch.cuda.Event(), "ev_done": torch.cuda.Event(),
-                                "ev_out": torch.cuda.Event()})
+            slot = {"buf": buf, "out_host": torch.empty_like(self.out_host).pin_memory(), "used": False,
+                    "ev_in": torch.cuda.Event(), "ev_photo": torch.cuda.Event(), "ev_done": torch.cuda.Event(), "ev_out": torch.cuda.Event()}
+            if self.max_pixels is not None:
+                buf["table"] = torch.empty_like(self._table)
+                slot.update(table_host=torch.empty_like(self._table_host).pin_memory(), ev_table=torch.cuda.Event(), views=None)
+            self._slots.append(slot)
         self._submitted = 0
 
     def submit_host(self, h: dict) -> int:
         """Enqueue one batch (pinned host inputs) without waiting for it; returns a ticket for `wait`.  At most two batches may be
         outstanding (a ticket must be waited for before the second-next submit).  The photo is only needed by the last kernel, so
-        its upload also runs underneath this batch's own sampling."""
+        its upload also runs underneath this batch's own sampling.
+
+        Mixed-size mode: h["photo_u8"] is a list of 1..docs uint8 HWC host photos and the other inputs have that many documents
+        (x_T that many times n_batch); document slots past the list keep their earlier inputs, are sampled and not unwarped."""
         self._check_weights()
+        if self.max_pixels is not None:
+            return self._submit_host_mixed(h)
         with torch.cuda.device(self.dev):
             if self._slots is None:
                 self._make_slots()
@@ -159,13 +230,62 @@ class DewarpPipeline:
             s["used"] = True
         return ticket
 
-    def wait(self, ticket: int) -> torch.Tensor:
-        """Block until the batch of `ticket` is on the host; the returned pinned tensor is reused by the second-next submit."""
+    def _submit_host_mixed(self, h: dict) -> int:
+        photos = self._check_photos(h["photo_u8"], torch.device("cpu"), 1)
+        n = len(photos)
+        for k in self.SAMPLING_KEYS:
+            want = (n * self.n_batch if k == "x_T" else n,) + tuple(self.buf[k].shape[1:])
+            if tuple(h[k].shape) != want:
+                raise ValueError(f"{k}: expected shape {want} for {n} photos, got {tuple(h[k].shape)}")
+        with torch.cuda.device(self.dev):
+            if self._slots is None:
+                self._make_slots()
+            main = torch.cuda.current_stream()
+            ticket = self._submitted
+            self._submitted += 1
+            s = self._slots[ticket % 2]
+            buf = s["buf"]
+            photo_dev = self._arena_views(buf["photo_u8"], photos)
+            out_dev = self._arena_views(buf["out_u8"], photos)
+            with torch.cuda.stream(self._h2d):
+                if s["used"]:
+                    self._h2d.wait_event(s["ev_done"])             # the kernels of batch ticket-2 have read this slot's inputs
+                for k in self.SAMPLING_KEYS:
+                    buf[k][:h[k].shape[0]].copy_(h[k], non_blocking=True)
+                s["ev_in"].record()
+                for dst, src in zip(photo_dev, photos):
+                    dst.copy_(src, non_blocking=True)
+                s["ev_photo"].record()
+            main.wait_event(s["ev_in"])
+            if s["used"]:
+                main.wait_event(s["ev_out"])                       # the download of batch ticket-2 has read this slot's output
+            self._run("sampling", buf, self.SAMPLING_KEYS, self._enqueue_sampling)
+            # the device only waits for batch ticket-2 through events; the HOST rewrites the pinned table now, so the upload of
+            # ticket-2 must have read it (normally long done)
+            s["ev_table"].synchronize()
+            plan_mixed(s["table_host"], photo_dev, out_dev, 64, 64)
+            buf["table"].copy_(s["table_host"], non_blocking=True)
+            s["ev_table"].record(main)
+            main.wait_event(s["ev_photo"])
+            self._run("unwarp", buf, ("table",), self._enqueue_unwarp_mixed)
+            s["ev_done"].record(main)
+            end = out_dev[-1].data_ptr() - buf["out_u8"].data_ptr() + out_dev[-1].numel()
+            with torch.cuda.stream(self._d2h):
+                self._d2h.wait_event(s["ev_done"])
+                s["out_host"][:end].copy_(buf["out_u8"][:end], non_blocking=True)
+                s["ev_out"].record()
+            s["views"] = self._arena_views(s["out_host"], photos)
+            s["used"] = True
+        return ticket
+
+    def wait(self, ticket: int):
+        """Block until the batch of `ticket` is on the host; the returned pinned tensor (mixed-size mode: list of views into a
+        pinned arena) is reused by the second-next submit."""
         s = self._slots[ticket % 2]
         s["ev_out"].synchronize()
-        return s["out_host"]
+        return s["out_host"] if self.max_pixels is None else s["views"]
 
-    def run_host(self, h: dict) -> torch.Tensor:
+    def run_host(self, h: dict):
         """Synchronous form: host inputs in, host uint8 image(s) out."""
         return self.wait(self.submit_host(h))
 

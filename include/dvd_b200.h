@@ -128,6 +128,24 @@ DVD_API int dvd_unwarp_u8(const uint8_t* photo, const float* map, uint8_t* out, 
 /* fp32 NCHW photo in, uint8 HWC out (the reference's tensor types at both ends of visualize_dewarping). */
 DVD_API int dvd_unwarp_f32_u8(const float* photo, const float* map, uint8_t* out, int B, int C, int H, int W,
                       int mh, int mw, float affine, void* stream);
+/* Mixed-size uint8 HWC batch: documents of different sizes in ONE launch (same result, byte for byte, as dvd_unwarp_u8 on each
+ * document alone).  The caller owns a table in device memory: dvd_unwarp_u8_plan fills it in HOST memory (pinned, for an async
+ * upload; no CUDA call, so it can run while earlier work is in flight), the caller copies it to the device, and dvd_unwarp_u8_mixed
+ * launches.  The launch reads the table on the device only, so a CUDA graph captured once serves every composition planned into
+ * the same device table.  Document d reads map row d of map [n_docs,2,mh,mw]; empty documents (H or W = 0) are allowed. */
+typedef struct dvd_unwarp_doc {
+  const uint8_t* photo;                 /* [H,W,C] uint8, device (NULL allowed when H or W is 0) */
+  uint8_t* out;                         /* [H,W,C] uint8, device                                 */
+  int32_t H, W;
+} dvd_unwarp_doc_t;
+/* bytes of a table for up to max_docs documents */
+DVD_API size_t dvd_unwarp_table_bytes(int max_docs);
+/* host only: validates (C in 1..4, H,W >= 0, H*W*C < 2^31, non-NULL pointers of non-empty documents, table_bytes large enough) and
+ * fills table_host; *total_tiles (may be NULL) = the number of 128x8 tiles of the batch. */
+DVD_API int dvd_unwarp_u8_plan(const dvd_unwarp_doc_t* docs_host, int n_docs, int C, int mh, int mw, float affine,
+                               void* table_host, size_t table_bytes, long long* total_tiles);
+/* one launch; table = the uploaded plan; C must equal the planned C (a table planned for another C is ignored: nothing is written) */
+DVD_API int dvd_unwarp_u8_mixed(const void* table, int C, const float* map, void* stream);
 /* WP:14-23,50-73 register_model2 / SpatialTransformer2: generic bilinear grid_sample,
  * align_corners=True, zeros padding.  img [B,C,H,W], grid [B,2,Ho,Wo] (ch0=x, ch1=y), out [B,C,Ho,Wo]. */
 DVD_API int dvd_grid_sample_f32(const float* img, const float* grid, float* out, int B, int C, int H, int W,
