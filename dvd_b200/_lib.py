@@ -27,7 +27,7 @@ class DecLayer(C.Structure):
     _fields_ = [("n1_w", _vp), ("n1_b", _vp), ("qkv", Mat), ("fc", Mat), ("n2_w", _vp), ("n2_b", _vp),
                 ("conv1", Mat), ("bn1_scale", _vp), ("bn1_shift", _vp), ("dw_w", _vp), ("bn2_scale", _vp),
                 ("bn2_shift", _vp), ("conv2", Mat), ("bn3_scale", _vp), ("bn3_shift", _vp),
-                ("qkv_h", Mat), ("qkv_ln", Mat), ("qkv_colsum", _vp), ("qkv_cvec", _vp), ("conv1_ln", Mat), ("conv1_colsum", _vp), ("conv1_cvec", _vp)]
+                ("qkv_ln", Mat), ("qkv_colsum", _vp), ("qkv_cvec", _vp), ("conv1_ln", Mat), ("conv1_colsum", _vp), ("conv1_cvec", _vp)]
 
 
 class Weights(C.Structure):

@@ -11,7 +11,6 @@
 #include "gemm_simt.cuh"
 #include "gemm_tc.cuh"
 #include "misc.cuh"
-#include <stdlib.h>
 #include <string.h>
 #include <vector>
 
@@ -224,52 +223,44 @@ static int static_forward(const Ctx& c, const float* y512, const float* mask_cat
     // level_0 (Cin = 4): the 3x3x4 patch of every pixel is written once as a K = 64 (36 valid + zero padding) 16-bit row
     // (im2col, 128 B per pixel) and multiplied by the K-padded weight on tcgen05; the six wide convs run as implicit GEMMs
     // directly on the NHWC activations; the last pool writes the fp32 feature map the rest of the model consumes.
-    // pyrP / pyrQ are fp32-sized: the first half holds the bf16 activation, the second half its low part (split-precision mode).
-    // DVD_PREC_BF16X3 with fp16 weight pairs (dvd_weights_t::pyr_h): the activations are ONE fp16 value per element and every conv runs
-    // two tensor passes instead of three (oracle/precision_study.py --two-pass: "only pyramid: fp16 activation x weight pair" moves the
-    // final map by nothing measurable, 1.25e-6 vs 1.44e-6).  DVD_PYR_3PASS=1 restores the bf16 pairs.
-    const bool a16 = x3 && w.pyr_h[0].bf16 && w.pyr_h[0].bf16_lo && w.pyr_h[6].bf16 && w.pyr_h[6].bf16_lo &&
-                     !(getenv("DVD_PYR_3PASS") && atoi(getenv("DVD_PYR_3PASS")));
-    const int passes = x3 ? (a16 ? 2 : 3) : 1;
-    const size_t half = (size_t)B * 512 * 512 * 64;
-    B16 P, Q;
-    P.hi = (__nv_bfloat16*)s.pyrP; P.lo = (x3 && !a16) ? P.hi + half : nullptr;
-    Q.hi = (__nv_bfloat16*)s.pyrQ; Q.lo = (x3 && !a16) ? Q.hi + half : nullptr;
-    auto op = [&](const B16& b) { TcMat m; m.hi = b.hi; m.lo = b.lo; m.ld = 64; m.f16 = a16; return m; };
+    // DVD_PREC_BF16X3 runs on the fp16 weight pairs (dvd_weights_t::pyr_h): the activations are ONE fp16 value per element and every
+    // conv runs two tensor passes (oracle/precision_study.py --two-pass: "only pyramid: fp16 activation x weight pair" moves the final
+    // map by nothing measurable, 1.25e-6 vs 1.44e-6 for bf16 pairs on both sides).
+    const int passes = x3 ? 2 : 1, pf = x3 ? 1 : 0;
+    __nv_bfloat16* P = (__nv_bfloat16*)s.pyrP;
+    __nv_bfloat16* Q = (__nv_bfloat16*)s.pyrQ;
+    auto op = [&](__nv_bfloat16* a) { TcMat m; m.hi = a; m.ld = 64; m.f16 = x3; return m; };
     auto wop = [&](int layer) {
-      if (!a16) return weight_op(c, w.pyr[layer]);
+      if (!x3) return weight_op(c, w.pyr[layer]);
       TcMat m; m.hi = (const __nv_bfloat16*)w.pyr_h[layer].bf16; m.lo = (const __nv_bfloat16*)w.pyr_h[layer].bf16_lo; m.ld = w.pyr_h[layer].k;
       return m;
     };
-    auto out16 = [&](Epilogue& e, const B16& dst, int ld) {
-      if (a16) { e.out_bf16 = dst.hi; e.out_lo = nullptr; e.ldc_bf16 = ld; e.out_f16 = 1; }
-      else out_operand(e, dst, ld);
-    };
+    auto out16 = [&](Epilogue& e, __nv_bfloat16* dst, int ld) { e.out_bf16 = dst; e.ldc_bf16 = ld; e.out_f16 = pf; };
     {
       ProfScope ps(PC_CONV, st, 2.0 * B * 512 * 512 * 64 * 36.0, passes);
-      DVD_REQUIRE(w.pyr[0].bf16 && (!x3 || w.pyr[0].bf16_lo), "pyramid level_0 16-bit (K-padded) weight missing");
-      DVD_TRY(im2col3x3_c4_bf16(s.y4, Q.hi, Q.lo, B, 512, 512, st, a16 ? 1 : 0));     // Q: [B*512*512, 64]
-      Epilogue e; e.bias = w.pyr_b[0]; e.act = ACT_RELU; out16(e, P, 64);
       TcMat wt = wop(0); wt.ld = 64;
+      DVD_REQUIRE(wt.hi && (!x3 || wt.lo), "pyramid level_0 16-bit (K-padded) weight missing");
+      DVD_TRY(im2col3x3_c4_bf16(s.y4, Q, B, 512, 512, st, pf));     // Q: [B*512*512, 64]
+      Epilogue e; e.bias = w.pyr_b[0]; e.act = ACT_RELU; out16(e, P, 64);
       DVD_TRY(gemm_tc(op(Q), wt, B * 512 * 512, 64, 64, e, st));
     }
-    auto conv = [&](const B16& in, const B16& out, int H, int Cin, int layer) -> int {
+    auto conv = [&](__nv_bfloat16* in, __nv_bfloat16* out, int H, int Cin, int layer) -> int {
       const int Cout = w.pyr[layer].n;
       ProfScope ps(PC_CONV, st, 2.0 * B * H * H * Cout * 9.0 * Cin, passes);
       Epilogue e; e.bias = w.pyr_b[layer]; e.act = ACT_RELU; out16(e, out, Cout);
-      DVD_REQUIRE(w.pyr[layer].bf16 && (!x3 || w.pyr[layer].bf16_lo), "pyramid 16-bit weights missing");
-      return conv3x3_tc(op(in), wop(layer), B, H, H, Cin, Cout, e, st);
+      const TcMat wt = wop(layer);
+      DVD_REQUIRE(wt.hi && (!x3 || wt.lo), "pyramid 16-bit weights missing");
+      return conv3x3_tc(op(in), wt, B, H, H, Cin, Cout, e, st);
     };
-    const int pf = a16 ? 1 : 0;
     DVD_TRY(conv(P, Q, 512, 64, 1));
-    DVD_TRY(maxpool2_nhwc_bf16(Q.hi, Q.lo, P.hi, P.lo, nullptr, B, 512, 512, 64, st, pf));
+    DVD_TRY(maxpool2_nhwc_bf16(Q, P, nullptr, B, 512, 512, 64, st, pf));
     DVD_TRY(conv(P, Q, 256, 64, 2));
     DVD_TRY(conv(Q, P, 256, 128, 3));
-    DVD_TRY(maxpool2_nhwc_bf16(P.hi, P.lo, Q.hi, Q.lo, nullptr, B, 256, 256, 128, st, pf));
+    DVD_TRY(maxpool2_nhwc_bf16(P, Q, nullptr, B, 256, 256, 128, st, pf));
     DVD_TRY(conv(Q, P, 128, 128, 4));
     DVD_TRY(conv(P, Q, 128, 256, 5));
     DVD_TRY(conv(Q, P, 128, 256, 6));
-    DVD_TRY(maxpool2_nhwc_bf16(P.hi, P.lo, nullptr, nullptr, s.feat, B, 128, 128, 256, st, pf));
+    DVD_TRY(maxpool2_nhwc_bf16(P, nullptr, s.feat, B, 128, 128, 256, st, pf));
   } else {
     DVD_TRY(conv3x3(c, s.y4, s.pyrP, B, 512, 512, 4, w.pyr[0], w.pyr_b[0]));
     DVD_TRY(conv3x3(c, s.pyrP, s.pyrQ, B, 512, 512, 64, w.pyr[1], w.pyr_b[1]));
@@ -317,22 +308,15 @@ static int denoise_step(const Ctx& c, const float* x_t, const float* init_flow, 
   const dvd_weights_t& w = *c.w; const Workspace& s = c.ws; cudaStream_t st = c.st;
   const int N = c.docs * c.n_hyp, M = N * 1024;
   const bool tc = c.tc();
-  // LayerNorm folded into the decoder GEMMs (producers emit row statistics + the raw rows as a 16-bit operand, the consumer normalises
-  // in its epilogue).  DVD_LN_FUSION = 1 (default): norm2 -> conv1 (raw rows as a bf16 pair, three passes) AND norm1 -> q|k|v (raw rows
-  // as ONE fp16 value, two passes; oracle: 1.2e-6 -> 1.8e-6 mean map error): no LayerNorm kernel left in the decoder; 2: norm2 -> conv1
-  // only; 0: separate LayerNorm kernels.  Measured in profiles/r2_ln_fusion.txt.  Before the GEMM epilogue's cold-code fix the fused variants lost: every instruction added to an
-  // epilogue that ran cold cost several times its warm price.
-  const int want_lnf = getenv("DVD_LN_FUSION") ? atoi(getenv("DVD_LN_FUSION")) : 1;
-  const bool lnf_c1 = c.x3() && want_lnf && w.dec[0].conv1_ln.bf16 && w.dec[0].conv1_ln.bf16_lo && w.dec[0].conv1_colsum;   // norm2 -> conv1
-  const bool lnf = lnf_c1 && want_lnf == 1 && w.dec[0].qkv_ln.bf16 && w.dec[0].qkv_ln.bf16_lo && w.dec[0].qkv_colsum;         // + norm1 -> q|k|v
-  // The decoder's q|k|v GEMM (the largest of the step) takes its activation as ONE fp16 value: q, k and v are rounded to fp16 for the
-  // attention anyway, and what moves the map is weight rounding, not activation rounding (oracle/precision_study.py
-  // --decoder-breakdown: 1.44e-6 -> 1.52e-6 mean map error).  Two tensor passes instead of three.  DVD_QKV_3PASS=1 restores the pair.
-  const bool qkv_a16 = c.x3() && !lnf && w.dec[0].qkv_h.bf16 && w.dec[0].qkv_h.bf16_lo && !(getenv("DVD_QKV_3PASS") && atoi(getenv("DVD_QKV_3PASS")));
-  // (with norm1 folded the q|k|v GEMM is always two-pass: qkv_ln is packed as an fp16 pair and the raw rows arrive as ONE fp16 value)
+  // DVD_PREC_BF16X3 folds every LayerNorm of the decoder into the GEMM that consumes it (producers emit row statistics + the raw rows as
+  // a 16-bit operand, the consumer normalises in its epilogue): norm2 -> conv1 (raw rows as a bf16 pair, three passes) and norm1 ->
+  // q|k|v (raw rows as ONE fp16 value against the fp16 pair qkv_ln, two passes; q, k and v are rounded to fp16 for the attention anyway;
+  // oracle: 1.2e-6 -> 1.8e-6 mean map error).  Measured against separate LayerNorm kernels in profiles/r2_ln_fusion.txt.  Before the
+  // GEMM epilogue's cold-code fix the fused variants lost: every instruction added to an epilogue that ran cold cost several times its
+  // warm price.
+  const bool lnf = c.x3();
   const float* ada = trow + 384;                 // shift_msa, scale_msa, gate_msa, shift_mlp, scale_mlp, gate_mlp
   const float* fin = trow + 384 + 2304;          // shift[1536], scale[1536]
-  auto off16 = [](const B16& b, size_t n) { B16 r; r.hi = b.hi + n; r.lo = b.lo ? b.lo + n : nullptr; return r; };
   // ---- obs embed (CM:571) and r embed (CM:602-603) with the fused feature warp (GD:618-624)
   DVD_TRY(obs_embed(x_t, w.emb[0].f32, w.emb_b[0], w.pos, s.xe, N, st));
   const int lda_r = 1032;                       // 258*4; TMA zero-fills the K tail of the last 64-wide box
@@ -407,19 +391,18 @@ static int denoise_step(const Ctx& c, const float* x_t, const float* init_flow, 
     // h- and w-branch side by side: conv1x1 + ReLU, then conv1x1 + sigmoid (CA:143-157)
     DVD_TRY(gemv_pair(mean, mean, 1536, w.h_scale0.f32, w.w_scale0.f32, w.h_scale0_b, w.w_scale0_b, hs1, ws1, 1536, N, 1536, 1536, 1, st));
     DVD_TRY(gemv_pair(hs1, ws1, 1536, w.h_scale2.f32, w.w_scale2.f32, w.h_scale2_b, w.w_scale2_b, hs, wsv, 1536, N, 1536, 1536, 3, st));
-    // DVD_LN_FUSION=1: all twelve LayerNorms of the decoder are folded into the GEMMs that consume them (no LN kernel, no normalised copy):
-    // every producer of the residual stream X also writes X as an operand pair and the rows' partial (sum, sum of squares); the QKV /
+    // bf16x3: all twelve LayerNorms of the decoder are folded into the GEMMs that consume them (no LN kernel, no normalised copy):
+    // every producer of the residual stream X also writes X as a 16-bit operand and the rows' partial (sum, sum of squares); the QKV /
     // conv1 GEMMs multiply the RAW rows by gamma-scaled weights and normalise in the epilogue (Epilogue::ln_*).  Accuracy checked on
     // the oracle first (oracle/precision_study.py --ln-fusion: 1.44e-6 -> 1.53e-6 mean map error).
-    if (lnf) DVD_TRY(posenc_add_ln(s.X, hs, wsv, w.dec_hpe, w.dec_wpe, N, 1536, s.X16.hi, nullptr, s.lnstats, 48, st, 1));
+    if (lnf) DVD_TRY(posenc_add_ln(s.X, hs, wsv, w.dec_hpe, w.dec_wpe, N, 1536, s.X16.hi, s.lnstats, 48, st));
     else DVD_TRY(posenc_add(s.X, hs, wsv, w.dec_hpe, w.dec_wpe, N, 1536, st));
   }
   if (g_stop_after == 2) return 0;
   // ---- 6 decoder layers (CA:377-396)
   for (int l = 0; l < 6; ++l) {
     const dvd_dec_layer_t& L = w.dec[l];
-    if (!lnf) DVD_TRY(layernorm(s.X, 1536, tc ? nullptr : s.hd, 1536, s.hd16.hi, s.hd16.lo, 1536, M, 1536, 1e-5f, L.n1_w, L.n1_b, nullptr, nullptr, st,
-                                qkv_a16 ? 1 : 0));
+    if (!lnf) DVD_TRY(layernorm(s.X, 1536, tc ? nullptr : s.hd, 1536, s.hd16.hi, s.hd16.lo, 1536, M, 1536, 1e-5f, L.n1_w, L.n1_b, nullptr, nullptr, st));
     {
       Epilogue e; e.out = tc ? nullptr : s.qkv_d; e.ldc = 4608;
       if (tc) { out_attn(c, e, s.qkv_d16, 4608); e.vt_out = s.vt_d16; e.vt_col0 = 3072; }
@@ -427,21 +410,21 @@ static int denoise_step(const Ctx& c, const float* x_t, const float* init_flow, 
         e.ln_stats = s.lnstats; e.ln_colsum = L.qkv_colsum; e.ln_chunks = 48; e.ln_eps = 1e-5f; e.bias = L.qkv_cvec;
         DVD_TRY(linear(c, nullptr, s.X16, 1536, L.qkv_ln, 0, M, 4608, e, true));
       } else {
-        DVD_TRY(linear(c, s.hd, s.hd16, 1536, qkv_a16 ? L.qkv_h : L.qkv, 0, M, 4608, e, qkv_a16));
+        DVD_TRY(linear(c, s.hd, s.hd16, 1536, L.qkv, 0, M, 4608, e));
       }
     }
     DVD_TRY(attention(c, s.qkv_d, s.qkv_d16, 4608, s.qkv_d + 1536, tc ? s.qkv_d16 + 1536 : nullptr, 4608, s.qkv_d + 3072, s.vt_d16, 4608,
                       s.att_d, s.att_d16, 1536, N, 256, 0.0625f, 1));
     {
       Epilogue e; e.resid = s.X; e.ldr = 1536; e.out = s.X; e.ldc = 1536;
-      if (lnf_c1) { out_operand(e, s.X16, 1536); e.stats_out = s.lnstats; }
+      if (lnf) { out_operand(e, s.X16, 1536); e.stats_out = s.lnstats; }
       DVD_TRY(linear(c, s.att_d, s.att_d16, 1536, L.fc, 0, M, 1536, e));
     }
-    if (!lnf_c1) DVD_TRY(layernorm(s.X, 1536, tc ? nullptr : s.hd, 1536, s.hd16.hi, s.hd16.lo, 1536, M, 1536, 1e-5f, L.n2_w, L.n2_b, nullptr, nullptr, st));
+    if (!lnf) DVD_TRY(layernorm(s.X, 1536, tc ? nullptr : s.hd, 1536, s.hd16.hi, s.hd16.lo, 1536, M, 1536, 1e-5f, L.n2_w, L.n2_b, nullptr, nullptr, st));
     {
       Epilogue e; e.scale = L.bn1_scale; e.shift = L.bn1_shift; e.act = ACT_RELU; e.out = tc ? nullptr : s.f1; e.ldc = 2048;
       if (tc) out_operand(e, s.f116, 2048);
-      if (lnf_c1) {
+      if (lnf) {
         e.ln_stats = s.lnstats; e.ln_colsum = L.conv1_colsum; e.ln_chunks = 48; e.ln_eps = 1e-5f; e.bias = L.conv1_cvec;
         DVD_TRY(linear(c, nullptr, s.X16, 1536, L.conv1_ln, 0, M, 2048, e));
       } else {
@@ -459,7 +442,6 @@ static int denoise_step(const Ctx& c, const float* x_t, const float* init_flow, 
   }
   // ---- final layer + unpatchify + init_flow + DDIM update (one kernel)
   DVD_TRY(final_layer(s.X, w.dec_ln_w, w.dec_ln_b, fin, fin + 1536, w.fin.f32, w.fin_b, init_flow, x_t, da, db, pred, x_prev, N, st));
-  (void)off16;
   return 0;
 }
 
@@ -468,6 +450,20 @@ static int make_ctx(Ctx& c, const dvd_weights_t* w, void* workspace, size_t byte
   DVD_REQUIRE(docs > 0 && n_hyp > 0, "docs and n_hyp must be positive");
   DVD_REQUIRE(precision == DVD_PREC_FP32 || precision == DVD_PREC_BF16 || precision == DVD_PREC_BF16X3, "bad precision %d", precision);
   DVD_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "workspace must be 256-byte aligned");
+  if (precision == DVD_PREC_BF16X3) {            // the packs only this precision reads (include/dvd_b200.h)
+    for (int i = 0; i < 7; ++i) {
+      DVD_REQUIRE(w->pyr_h[i].bf16, "bf16x3 weight table: pyr_h[%d].bf16 is NULL", i);
+      DVD_REQUIRE(w->pyr_h[i].bf16_lo, "bf16x3 weight table: pyr_h[%d].bf16_lo is NULL", i);
+    }
+    for (int l = 0; l < 6; ++l) {
+      const dvd_dec_layer_t& L = w->dec[l];
+      const struct { const void* p; const char* name; } need[] = {
+          {L.qkv_ln.bf16, "qkv_ln.bf16"}, {L.qkv_ln.bf16_lo, "qkv_ln.bf16_lo"}, {L.qkv_colsum, "qkv_colsum"}, {L.qkv_cvec, "qkv_cvec"},
+          {L.conv1_ln.bf16, "conv1_ln.bf16"}, {L.conv1_ln.bf16_lo, "conv1_ln.bf16_lo"}, {L.conv1_colsum, "conv1_colsum"},
+          {L.conv1_cvec, "conv1_cvec"}};
+      for (const auto& f : need) DVD_REQUIRE(f.p, "bf16x3 weight table: dec[%d].%s is NULL", l, f.name);
+    }
+  }
   c.w = w; c.docs = docs; c.n_hyp = n_hyp; c.prec = precision; c.st = (cudaStream_t)stream;
   c.ws = carve(workspace, docs, n_hyp, precision);
   if (c.ws.total_bytes > bytes) {

@@ -722,10 +722,10 @@ int gemm_pair_dispatch(const TcMat& A, const TcMat& W, int M, int N, int K, cons
   DVD_REQUIRE(!e.out_bf16 || (e.ldc_bf16 % 8 == 0 && e.group_col_stride % 8 == 0 && (reinterpret_cast<uintptr_t>(e.out_bf16) & 15) == 0 &&
                               (reinterpret_cast<uintptr_t>(e.out_lo) & 15) == 0),
               "gemm_pair: 16-bit outputs are stored 16 bytes at a time (ld %% 8, 16-byte aligned bases)");
+  DVD_REQUIRE(!conv || mode != 1, "gemm_pair: the implicit convolution takes a bf16 activation or an fp16 one, not a split pair");
   const int bn = pick_bn(M, N, K, mode, sm_count() / 2);
-  if (conv && mode == 2) return launch_pair_bn<2, true>(bn, A, W, M, N, K, e, conv_b, conv_h, conv_w, conv_cin, st);
-  if (conv) return mode ? launch_pair_bn<1, true>(bn, A, W, M, N, K, e, conv_b, conv_h, conv_w, conv_cin, st)
-                        : launch_pair_bn<0, true>(bn, A, W, M, N, K, e, conv_b, conv_h, conv_w, conv_cin, st);
+  if (conv) return mode == 2 ? launch_pair_bn<2, true>(bn, A, W, M, N, K, e, conv_b, conv_h, conv_w, conv_cin, st)
+                             : launch_pair_bn<0, true>(bn, A, W, M, N, K, e, conv_b, conv_h, conv_w, conv_cin, st);
   if (mode == 2) return launch_pair_bn<2, false>(bn, A, W, M, N, K, e, 0, 0, 0, 0, st);
   return mode ? launch_pair_bn<1, false>(bn, A, W, M, N, K, e, 0, 0, 0, 0, st)
               : launch_pair_bn<0, false>(bn, A, W, M, N, K, e, 0, 0, 0, 0, st);

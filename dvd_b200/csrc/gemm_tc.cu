@@ -385,12 +385,13 @@ int gemm_tc(const TcMat& A, const TcMat& W, int M, int N, int K, const Epilogue&
 }
 
 // 3x3 / pad 1 / stride 1 convolution as an implicit GEMM: in NHWC [B,H,W,Cin], Wt [Cout, 9*Cin] ([ky][kx][Cin]),
-// out NHWC [B,H,W,Cout] through the Epilogue (bias + ReLU, 16-bit and/or fp32).
+// out NHWC [B,H,W,Cout] through the Epilogue (bias + ReLU, 16-bit and/or fp32).  Two operand forms: a bf16 activation with a bf16
+// weight (one pass), or an fp16 activation with an fp16 weight pair (two passes).
 int conv3x3_tc(const TcMat& in, const TcMat& Wt, int B, int H, int Wd, int Cin, int Cout, const Epilogue& e, cudaStream_t st) {
   DVD_REQUIRE(in.hi && Wt.hi && (e.out || e.out_bf16), "conv3x3_tc: null pointer");
   DVD_REQUIRE(Cin % 64 == 0 && Wd % 128 == 0 && (Cout == 64 || Cout % 128 == 0), "conv3x3_tc: unsupported shape Cin=%d W=%d Cout=%d", Cin, Wd, Cout);
-  DVD_REQUIRE(in.f16 ? (!in.lo && Wt.lo) : ((in.lo != nullptr) == (Wt.lo != nullptr)),
-              "conv3x3_tc: activation and weight must both be split pairs or both plain (or: fp16 activation with an fp16 weight pair)");
+  DVD_REQUIRE(!in.lo && (in.f16 ? Wt.lo != nullptr : Wt.lo == nullptr),
+              "conv3x3_tc: bf16 activation with a bf16 weight, or fp16 activation with an fp16 weight pair");
   const int M = B * H * Wd, K = 9 * Cin;
   int rc = check_epilogue(e, Cout); if (rc) return rc;
   if (!use_v1() && gemm_pair_supported(M, Cout, K, true)) {
@@ -398,19 +399,12 @@ int conv3x3_tc(const TcMat& in, const TcMat& Wt, int B, int H, int Wd, int Cin, 
     return gemm_pair_dispatch(in, w, M, Cout, K, e, B, H, Wd, Cin, st);
   }
   DVD_REQUIRE(!in.f16, "conv3x3_tc: the fp16-activation mode needs the CTA-pair kernel");
-  const bool x3 = in.lo != nullptr;
   const int bn = Cout == 64 ? 64 : ((Cout % 256 == 0 && (long long)(M / 128) * (Cout / 256) >= 2LL * sm_count()) ? 256 : 128);
-  CUtensorMap tmA, tmB, tmAl, tmBl;
+  CUtensorMap tmA, tmB;
   rc = make_tmap_bf16_nhwc(&tmA, in.hi, (uint64_t)B, (uint64_t)H, (uint64_t)Wd, (uint64_t)Cin); if (rc) return rc;
   rc = make_tmap_bf16_2d(&tmB, Wt.hi, (uint64_t)Cout, (uint64_t)K, (uint64_t)K, bn == 64 ? 64 : 128, 64); if (rc) return rc;
-  tmAl = tmA; tmBl = tmB;
-  if (x3) {
-    rc = make_tmap_bf16_nhwc(&tmAl, in.lo, (uint64_t)B, (uint64_t)H, (uint64_t)Wd, (uint64_t)Cin); if (rc) return rc;
-    rc = make_tmap_bf16_2d(&tmBl, Wt.lo, (uint64_t)Cout, (uint64_t)K, (uint64_t)K, bn == 64 ? 64 : 128, 64); if (rc) return rc;
-  }
   ConvGeom cg{H, Wd, Cin};
-  return x3 ? launch_tc_bn<true, true>(bn, tmA, tmAl, tmB, tmBl, M, Cout, K, e, cg, st)
-            : launch_tc_bn<true, false>(bn, tmA, tmAl, tmB, tmBl, M, Cout, K, e, cg, st);
+  return launch_tc_bn<true, false>(bn, tmA, tmA, tmB, tmB, M, Cout, K, e, cg, st);
 }
 
 }  // namespace dvd

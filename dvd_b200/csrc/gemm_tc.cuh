@@ -26,7 +26,8 @@ inline int gemm_tc_bf16(const __nv_bfloat16* A, int lda, const __nv_bfloat16* W,
 }
 
 // 3x3 / pad 1 conv as implicit GEMM on tcgen05 (TMA boxes over the NHWC activation, zero padding by OOB fill):
-// in [B,H,W,Cin] (pair or plain), Wt [Cout, 9*Cin] ordered [ky][kx][Cin]; output through the Epilogue as [B*H*W, Cout].
+// in [B,H,W,Cin] (plain bf16 with a plain bf16 Wt, or fp16 with an fp16 pair Wt), Wt [Cout, 9*Cin] ordered [ky][kx][Cin]; output
+// through the Epilogue as [B*H*W, Cout].
 int conv3x3_tc(const TcMat& in, const TcMat& Wt, int B, int H, int Wd, int Cin, int Cout, const Epilogue& e, cudaStream_t st);
 
 // softmax(scale * Q K^T) V per (sample, head); 16-bit in/out (bf16, or fp16 when f16 != 0), fp32 softmax statistics and accumulation.

@@ -9,7 +9,7 @@ template <int NV>   // float4 per lane: C = 128 * NV
 __global__ void __launch_bounds__(256) k_layernorm(const float* __restrict__ in, int ldin, float* __restrict__ out, int ldo,
                                                    __nv_bfloat16* __restrict__ out16, __nv_bfloat16* __restrict__ out16_lo, int ldo16,
                                                    int rows, float eps, const float* __restrict__ w, const float* __restrict__ b,
-                                                   const float* __restrict__ msh, const float* __restrict__ msc, int f16) {
+                                                   const float* __restrict__ msh, const float* __restrict__ msc) {
   pdl_trigger();
   pdl_wait();
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -44,26 +44,22 @@ __global__ void __launch_bounds__(256) k_layernorm(const float* __restrict__ in,
     if (out) *reinterpret_cast<float4*>(out + (size_t)row * ldo + c0) = make_float4(y[0], y[1], y[2], y[3]);
     if (out16) {
       uint2 u, l;
-      if (f16) {                               // single IEEE fp16 operand (two-pass GEMM: fp16 activation x weight pair)
-        u.x = pack_f16x2(y[0], y[1]); u.y = pack_f16x2(y[2], y[3]);
-      } else {
-        split_bf16x2(y[0], y[1], u.x, l.x);
-        split_bf16x2(y[2], y[3], u.y, l.y);
-      }
+      split_bf16x2(y[0], y[1], u.x, l.x);
+      split_bf16x2(y[2], y[3], u.y, l.y);
       *reinterpret_cast<uint2*>(out16 + (size_t)row * ldo16 + c0) = u;
-      if (out16_lo && !f16) *reinterpret_cast<uint2*>(out16_lo + (size_t)row * ldo16 + c0) = l;
+      if (out16_lo) *reinterpret_cast<uint2*>(out16_lo + (size_t)row * ldo16 + c0) = l;
     }
   }
 }
 
 int layernorm(const float* in, int ldin, float* out, int ldo, __nv_bfloat16* out16, __nv_bfloat16* out16_lo, int ldo16, int rows, int C,
-              float eps, const float* w, const float* b, const float* msh, const float* msc, cudaStream_t st, int out_f16) {
+              float eps, const float* w, const float* b, const float* msh, const float* msc, cudaStream_t st) {
   DVD_REQUIRE(in && (out || out16) && rows > 0, "layernorm: bad args");
   DVD_REQUIRE(C == 384 || C == 1536, "layernorm: C must be 384 or 1536 (got %d)", C);
   DVD_REQUIRE(ldin % 4 == 0 && ldo % 4 == 0 && ldo16 % 4 == 0, "layernorm: ld %% 4");
   dim3 grid(cdiv(rows, 8));
-  if (C == 384) DVD_CUDA(launch_pdl(4, k_layernorm<3>, grid, dim3(256), (size_t)0, st, in, ldin, out, ldo, out16, out16_lo, ldo16, rows, eps, w, b, msh, msc, out_f16));
-  else          DVD_CUDA(launch_pdl(4, k_layernorm<12>, grid, dim3(256), (size_t)0, st, in, ldin, out, ldo, out16, out16_lo, ldo16, rows, eps, w, b, msh, msc, out_f16));
+  if (C == 384) DVD_CUDA(launch_pdl(4, k_layernorm<3>, grid, dim3(256), (size_t)0, st, in, ldin, out, ldo, out16, out16_lo, ldo16, rows, eps, w, b, msh, msc));
+  else          DVD_CUDA(launch_pdl(4, k_layernorm<12>, grid, dim3(256), (size_t)0, st, in, ldin, out, ldo, out16, out16_lo, ldo16, rows, eps, w, b, msh, msc));
   DVD_LAUNCH_CHECK("k_layernorm");
   return 0;
 }
@@ -108,8 +104,7 @@ int maxpool2_nhwc(const float* in, float* out, int B, int H, int W, int C, cudaS
 
 // one thread = one (pixel, tap pair): 8 of the 16-byte chunks of a 128-byte output row; chunks 5..7 (k >= 40) are zero and
 // chunk 4 holds tap 8 + zeros
-__global__ void __launch_bounds__(256) k_im2col_c4(const float4* __restrict__ in, uint4* __restrict__ out, uint4* __restrict__ out_lo, int H, int W,
-                                                   size_t total, int f16) {
+__global__ void __launch_bounds__(256) k_im2col_c4(const float4* __restrict__ in, uint4* __restrict__ out, int H, int W, size_t total, int f16) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;          // total = B*H*W*8 chunks
   if (i >= total) return;
   const int chunk = i & 7; const size_t pix = i >> 3;
@@ -124,29 +119,23 @@ __global__ void __launch_bounds__(256) k_im2col_c4(const float4* __restrict__ in
       if (yy >= 0 && yy < H && xx >= 0 && xx < W) v[t] = __ldg(in + (b * H + yy) * W + xx);
     }
   }
-  uint4 o, l;
-  if (f16) {                                   // one IEEE fp16 value per element (two-pass mode of the pyramid)
-    o = make_uint4(pack_f16x2(v[0].x, v[0].y), pack_f16x2(v[0].z, v[0].w), pack_f16x2(v[1].x, v[1].y), pack_f16x2(v[1].z, v[1].w));
-    out[i] = o;
-    return;
-  }
-  split_bf16x2(v[0].x, v[0].y, o.x, l.x); split_bf16x2(v[0].z, v[0].w, o.y, l.y);
-  split_bf16x2(v[1].x, v[1].y, o.z, l.z); split_bf16x2(v[1].z, v[1].w, o.w, l.w);
-  out[i] = o;
-  if (out_lo) out_lo[i] = l;
+  if (f16)                                     // one IEEE fp16 value per element (two-pass mode of the pyramid)
+    out[i] = make_uint4(pack_f16x2(v[0].x, v[0].y), pack_f16x2(v[0].z, v[0].w), pack_f16x2(v[1].x, v[1].y), pack_f16x2(v[1].z, v[1].w));
+  else
+    out[i] = make_uint4(pack_bf16x2(v[0].x, v[0].y), pack_bf16x2(v[0].z, v[0].w), pack_bf16x2(v[1].x, v[1].y), pack_bf16x2(v[1].z, v[1].w));
 }
-int im2col3x3_c4_bf16(const float* in, __nv_bfloat16* out, __nv_bfloat16* out_lo, int B, int H, int W, cudaStream_t st, int out_f16) {
+int im2col3x3_c4_bf16(const float* in, __nv_bfloat16* out, int B, int H, int W, cudaStream_t st, int out_f16) {
   DVD_REQUIRE(in && out && B > 0, "im2col: bad args");
   size_t total = (size_t)B * H * W * 8;
-  k_im2col_c4<<<cdiv(total, 256), 256, 0, st>>>((const float4*)in, (uint4*)out, (uint4*)out_lo, H, W, total, out_f16);
+  k_im2col_c4<<<cdiv(total, 256), 256, 0, st>>>((const float4*)in, (uint4*)out, H, W, total, out_f16);
   DVD_LAUNCH_CHECK("k_im2col_c4");
   return 0;
 }
 
-// 2x2 max pool on bf16 NHWC (8 channels = 16 bytes per thread); the input may be a split pair (value = hi + lo), the output is
-// written as bf16 (hi + optional lo) and / or fp32
-__global__ void k_maxpool2_bf16(const uint4* __restrict__ in, const uint4* __restrict__ in_lo, uint4* __restrict__ out16,
-                                uint4* __restrict__ out16_lo, float* __restrict__ out32, int B, int H, int W, int C8, int f16) {
+// 2x2 max pool on 16-bit NHWC (8 channels = 16 bytes per thread): bf16, or IEEE fp16 when f16; the output is written in the input's
+// 16-bit type and / or as fp32
+__global__ void k_maxpool2_bf16(const uint4* __restrict__ in, uint4* __restrict__ out16, float* __restrict__ out32, int B, int H, int W,
+                                int C8, int f16) {
   const int Ho = H / 2, Wo = W / 2;
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   size_t total = (size_t)B * Ho * Wo * C8;
@@ -168,23 +157,13 @@ __global__ void k_maxpool2_bf16(const uint4* __restrict__ in, const uint4* __res
 #pragma unroll
       for (int k = 0; k < 4; ++k) { const float2 t2 = __half22float2(g[k]); f[2 * k] = t2.x; f[2 * k + 1] = t2.y; }
     }
-    if (in_lo && !f16) {
-      const uint4 ql = __ldg(in_lo + base + offs[t]);
-      const __nv_bfloat162* hl = reinterpret_cast<const __nv_bfloat162*>(&ql);
-#pragma unroll
-      for (int k = 0; k < 4; ++k) { f[2 * k] += __low2float(hl[k]); f[2 * k + 1] += __high2float(hl[k]); }
-    }
 #pragma unroll
     for (int k = 0; k < 8; ++k) m[k] = t == 0 ? f[k] : fmaxf(m[k], f[k]);
   }
-  if (out16 && f16) {                          // (the maximum of fp16 values is an fp16 value: exact)
+  if (out16 && f16) {                          // (the maximum of 16-bit values is a 16-bit value: exact)
     out16[i] = make_uint4(pack_f16x2(m[0], m[1]), pack_f16x2(m[2], m[3]), pack_f16x2(m[4], m[5]), pack_f16x2(m[6], m[7]));
   } else if (out16) {
-    uint4 o, l;
-    split_bf16x2(m[0], m[1], o.x, l.x); split_bf16x2(m[2], m[3], o.y, l.y);
-    split_bf16x2(m[4], m[5], o.z, l.z); split_bf16x2(m[6], m[7], o.w, l.w);
-    out16[i] = o;
-    if (out16_lo) out16_lo[i] = l;
+    out16[i] = make_uint4(pack_bf16x2(m[0], m[1]), pack_bf16x2(m[2], m[3]), pack_bf16x2(m[4], m[5]), pack_bf16x2(m[6], m[7]));
   }
   if (out32) {
     float4* o = reinterpret_cast<float4*>(out32 + i * 8);
@@ -192,11 +171,10 @@ __global__ void k_maxpool2_bf16(const uint4* __restrict__ in, const uint4* __res
     o[1] = make_float4(m[4], m[5], m[6], m[7]);
   }
 }
-int maxpool2_nhwc_bf16(const __nv_bfloat16* in, const __nv_bfloat16* in_lo, __nv_bfloat16* out16, __nv_bfloat16* out16_lo, float* out32, int B,
-                       int H, int W, int C, cudaStream_t st, int f16) {
+int maxpool2_nhwc_bf16(const __nv_bfloat16* in, __nv_bfloat16* out16, float* out32, int B, int H, int W, int C, cudaStream_t st, int f16) {
   DVD_REQUIRE(in && (out16 || out32) && C % 8 == 0 && H % 2 == 0 && W % 2 == 0, "maxpool2_bf16: bad args");
   size_t total = (size_t)B * (H / 2) * (W / 2) * (C / 8);
-  k_maxpool2_bf16<<<cdiv(total, 256), 256, 0, st>>>((const uint4*)in, (const uint4*)in_lo, (uint4*)out16, (uint4*)out16_lo, out32, B, H, W, C / 8, f16);
+  k_maxpool2_bf16<<<cdiv(total, 256), 256, 0, st>>>((const uint4*)in, (uint4*)out16, out32, B, H, W, C / 8, f16);
   DVD_LAUNCH_CHECK("k_maxpool2_bf16");
   return 0;
 }
@@ -572,11 +550,12 @@ int posenc_add(float* X, const float* hs, const float* ws, const float* hpe, con
   return 0;
 }
 
-// posenc_add for the fused-LayerNorm path: one warp per token row; also writes the row as the 16-bit operand of the next GEMM (bf16 or
-// pair) and its (sum, sum of squares) for the LayerNorm that GEMM's epilogue applies (slot 0 = whole row, the other chunk slots zero).
+// posenc_add for the fused-LayerNorm path: one warp per token row; also writes the row as ONE fp16 value per element (the operand of
+// the two-pass q|k|v GEMM) and its (sum, sum of squares) for the LayerNorm that GEMM's epilogue applies (slot 0 = whole row, the other
+// chunk slots zero).
 __global__ void __launch_bounds__(256) k_posenc_ln(float* __restrict__ X, const float4* __restrict__ hs, const float4* __restrict__ ws,
-                                                   const float4* __restrict__ hpe, const float4* __restrict__ wpe, __nv_bfloat16* __restrict__ hi,
-                                                   __nv_bfloat16* __restrict__ lo, float* __restrict__ stats, int chunks, int rows, int f16) {
+                                                   const float4* __restrict__ hpe, const float4* __restrict__ wpe, __nv_bfloat16* __restrict__ x16,
+                                                   float* __restrict__ stats, int chunks, int rows) {
   pdl_trigger();                                    // programmatic dependent launch: the successor may be scheduled now,
   pdl_wait();                                       // and this kernel was possibly scheduled before its predecessor finished
   constexpr int C4 = 384;                       // 1536 / 4
@@ -595,15 +574,7 @@ __global__ void __launch_bounds__(256) k_posenc_ln(float* __restrict__ X, const 
     x.x = (x.x + a.x * hp.x) + b.x * wp.x; x.y = (x.y + a.y * hp.y) + b.y * wp.y;
     x.z = (x.z + a.z * hp.z) + b.z * wp.z; x.w = (x.w + a.w * hp.w) + b.w * wp.w;
     xr[c] = x;
-    uint2 u, l;
-    if (f16) {                                  // ONE fp16 value per element (operand of the two-pass q|k|v GEMM)
-      u.x = pack_f16x2(x.x, x.y); u.y = pack_f16x2(x.z, x.w);
-    } else {
-      split_bf16x2(x.x, x.y, u.x, l.x);
-      split_bf16x2(x.z, x.w, u.y, l.y);
-    }
-    *reinterpret_cast<uint2*>(hi + ((size_t)row * C4 + c) * 4) = u;
-    if (lo && !f16) *reinterpret_cast<uint2*>(lo + ((size_t)row * C4 + c) * 4) = l;
+    *reinterpret_cast<uint2*>(x16 + ((size_t)row * C4 + c) * 4) = make_uint2(pack_f16x2(x.x, x.y), pack_f16x2(x.z, x.w));
     s1 += (x.x + x.y) + (x.z + x.w);
     s2 += (x.x * x.x + x.y * x.y) + (x.z * x.z + x.w * x.w);
   }
@@ -612,11 +583,11 @@ __global__ void __launch_bounds__(256) k_posenc_ln(float* __restrict__ X, const 
   for (int k = lane; k < chunks; k += 32) sr[k] = k == 0 ? make_float2(s1, s2) : make_float2(0.f, 0.f);
 }
 int posenc_add_ln(float* X, const float* hs, const float* ws, const float* hpe, const float* wpe, int N, int C, __nv_bfloat16* x16,
-                  __nv_bfloat16* x16_lo, float* stats, int chunks, cudaStream_t st, int x16_f16) {
+                  float* stats, int chunks, cudaStream_t st) {
   DVD_REQUIRE(X && hs && ws && hpe && wpe && x16 && stats && C == 1536 && chunks == C / 32, "posenc_add_ln: bad args");
   const int rows = N * 1024;
   DVD_CUDA(launch_pdl(16, k_posenc_ln, dim3(cdiv(rows, 8)), dim3(256), (size_t)0, st, X, (const float4*)hs, (const float4*)ws, (const float4*)hpe,
-                      (const float4*)wpe, x16, x16_lo, stats, chunks, rows, x16_f16));
+                      (const float4*)wpe, x16, stats, chunks, rows));
   DVD_LAUNCH_CHECK("k_posenc_ln");
   return 0;
 }

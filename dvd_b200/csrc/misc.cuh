@@ -10,18 +10,17 @@ namespace dvd {
 // bf16 destinations throughout this header: `x16` alone is plain bf16; with a non-null `x16_lo` the value is stored as the split
 // pair hi = bf16(v), lo = bf16(v - hi) (operand of a 3-pass GEMM in DVD_PREC_BF16X3).
 int layernorm(const float* in, int ldin, float* out, int ldo, __nv_bfloat16* out_bf16, __nv_bfloat16* out_bf16_lo, int ldo16, int rows, int C,
-              float eps, const float* w, const float* b, const float* mod_shift, const float* mod_scale, cudaStream_t st, int out_f16 = 0);
-// (out_f16 != 0: out_bf16 receives ONE IEEE fp16 value per element instead of bf16 / a bf16 pair)
+              float eps, const float* w, const float* b, const float* mod_shift, const float* mod_scale, cudaStream_t st);
 
 // y512 [B,3,512,512] + mask [B,1,512,512] (NCHW) -> NHWC [B,512,512,4]        (CM:586-587)
 int pack_y4(const float* y512, const float* mask, float* out, int B, cudaStream_t st);
 // 2x2 max pool on NHWC fp32
 int maxpool2_nhwc(const float* in, float* out, int B, int H, int W, int C, cudaStream_t st);
 // 3x3 / pad 1 im2col of a 4-channel NHWC fp32 image into bf16 rows of 64 (k = tap*4 + c, k >= 36 zero): [B*H*W, 64]
-// (out_f16 != 0: ONE IEEE fp16 value per element in `out` instead of bf16 / a bf16 pair)
-int im2col3x3_c4_bf16(const float* in, __nv_bfloat16* out, __nv_bfloat16* out_lo, int B, int H, int W, cudaStream_t st, int out_f16 = 0);
-int maxpool2_nhwc_bf16(const __nv_bfloat16* in, const __nv_bfloat16* in_lo, __nv_bfloat16* out16, __nv_bfloat16* out16_lo, float* out32, int B,
-                       int H, int W, int C, cudaStream_t st, int f16 = 0);      // f16: input and 16-bit output are single fp16 values
+// (out_f16 != 0: ONE IEEE fp16 value per element instead of bf16)
+int im2col3x3_c4_bf16(const float* in, __nv_bfloat16* out, int B, int H, int W, cudaStream_t st, int out_f16);
+int maxpool2_nhwc_bf16(const __nv_bfloat16* in, __nv_bfloat16* out16, float* out32, int B, int H, int W, int C, cudaStream_t st,
+                       int f16);      // f16: input and 16-bit output are single fp16 values (else bf16)
 // fp32 NHWC -> NCHW (feat for the drop-in model() return value) and back
 int nhwc_to_nchw(const float* in, float* out, int B, int H, int W, int C, cudaStream_t st);
 
@@ -62,10 +61,11 @@ int token_mean(const float* X, float* out, int N, int C, cudaStream_t st);
 // X[n,tok,c] += hs[n,c]*hpe[tok/32,c] + ws[n,c]*wpe[tok%32,c]              (CA:148-153)
 int posenc_add(float* X, const float* hs, const float* ws, const float* hpe, const float* wpe, int N, int C, cudaStream_t st);
 
-// same + the row as 16-bit GEMM operand (x16 [+ x16_lo]) + per-row (sum, sum of squares) in `stats` [N*1024][chunks][2] (slot 0), for the
-// LayerNorm fused into the next GEMM's epilogue (Epilogue::ln_stats).  C = 1536, chunks = C / 32.
+// same + the row as ONE IEEE fp16 value per element in x16 (the raw-row operand of the two-pass q|k|v GEMM) + per-row (sum, sum of
+// squares) in `stats` [N*1024][chunks][2] (slot 0), for the LayerNorm fused into that GEMM's epilogue (Epilogue::ln_stats).
+// C = 1536, chunks = C / 32.
 int posenc_add_ln(float* X, const float* hs, const float* ws, const float* hpe, const float* wpe, int N, int C, __nv_bfloat16* x16,
-                  __nv_bfloat16* x16_lo, float* stats, int chunks, cudaStream_t st, int x16_f16 = 0);
+                  float* stats, int chunks, cudaStream_t st);
 
 // depthwise 3x3 (pad 1) over the 32x32 token grid + folded BN + ReLU, token-major [N,1024,C]  (CA:33-41)
 int dwconv3x3_bn_relu(const float* in, const float* w9c, const float* scale, const float* shift, float* out,

@@ -87,15 +87,17 @@ class PackedWeights:
     def _vec(self, t):
         return C.c_void_p(self._dev(t).data_ptr())
 
-    def _mat(self, w2d: torch.Tensor, bf16: bool = True) -> _lib.Mat:
+    def _mat(self, w2d: torch.Tensor, bf16: bool = True, lo: bool = True) -> _lib.Mat:
+        """fp32 W, plus bf16(W) for the tensor modes when ``bf16``, plus bf16(W - bf16(W)) when ``lo`` (the matrices bf16x3 runs on
+        bf16 pairs)."""
         w = self._dev(w2d)
         m = _lib.Mat()
         m.f32 = w.data_ptr()
         m.n, m.k = int(w.shape[0]), int(w.shape[1])
         if bf16 and self.with_bf16:
             h, l = split_bf16(w)
-            self.keep += [h, l]
-            m.bf16, m.bf16_lo = h.data_ptr(), l.data_ptr()
+            self.keep += [h, l] if lo else [h]
+            m.bf16, m.bf16_lo = h.data_ptr(), (l.data_ptr() if lo else None)
         return m
 
     def _ln_fold(self, w64: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, f16: bool = False):
@@ -121,17 +123,17 @@ class PackedWeights:
         T = self.table
         T.pos = self._vec(sd["noised_obs_pos_embed"].reshape(1024, 384))
         for i, p in enumerate(PYR_KEYS):
-            w = sd[p + ".weight"].float()                                  # [Cout, Cin, 3, 3] -> [Cout, ky, kx, Cin]
-            T.pyr[i] = self._mat(w.permute(0, 2, 3, 1).reshape(w.shape[0], -1), bf16=(i > 0))
-            if i == 0 and self.with_bf16:                                   # level_0: K = 36 zero-padded to 64 for the tcgen05 im2col GEMM
-                pad = torch.zeros((w.shape[0], 64), dtype=torch.float32, device=self.device)
-                pad[:, :36] = w.permute(0, 2, 3, 1).reshape(w.shape[0], -1).to(self.device)
-                h, l = split_bf16(pad)
-                self.keep += [h, l]
-                T.pyr[0].bf16, T.pyr[0].bf16_lo = h.data_ptr(), l.data_ptr()
-            if self.with_bf16:                                              # the same matrices as fp16 pairs (two-pass pyramid of bf16x3)
-                w2 = pad if i == 0 else self.keep[-3]                       # level 0: the K-padded copy; else the fp32 copy _mat made
-                h16, l16 = split_f16(w2)
+            w = sd[p + ".weight"].float()
+            wk = w.permute(0, 2, 3, 1).reshape(w.shape[0], -1).to(self.device)    # [Cout, Cin, 3, 3] -> [Cout, ky, kx, Cin]
+            T.pyr[i] = self._mat(wk, bf16=(i > 0), lo=False)                # bf16 reads the hi; bf16x3 reads pyr_h
+            if self.with_bf16:
+                w2 = wk
+                if i == 0:                                                  # level_0: K = 36 zero-padded to 64 for the tcgen05 im2col GEMM
+                    w2 = torch.nn.functional.pad(wk, (0, 64 - wk.shape[1]))
+                    h = w2.to(torch.bfloat16).contiguous()
+                    self.keep.append(h)
+                    T.pyr[0].bf16 = h.data_ptr()
+                h16, l16 = split_f16(w2)                                    # the same matrices as fp16 pairs (two-pass pyramid of bf16x3)
                 self.keep += [h16, l16]
                 T.pyr_h[i].f32, T.pyr_h[i].bf16, T.pyr_h[i].bf16_lo = T.pyr[i].f32, h16.data_ptr(), l16.data_ptr()
                 T.pyr_h[i].n, T.pyr_h[i].k = int(w2.shape[0]), int(w2.shape[1])
@@ -163,16 +165,10 @@ class PackedWeights:
             L.n1_w, L.n1_b = self._vec(sd[p + "norm1.weight"]), self._vec(sd[p + "norm1.bias"])
             L.n2_w, L.n2_b = self._vec(sd[p + "norm2.weight"]), self._vec(sd[p + "norm2.bias"])
             L.qkv = self._mat(torch.cat([sd[p + "attn.linear_q.weight"], sd[p + "attn.linear_k.weight"],
-                                         sd[p + "attn.linear_v.weight"]], 0))
-            if self.with_bf16:                                    # fp16 pair of the same weights (two-pass q|k|v GEMM of bf16x3)
-                wq32 = self.keep[-3]                              # the fp32 copy _mat just made (keep = [..., f32, hi, lo])
-                h16, l16 = split_f16(wq32)
-                self.keep += [h16, l16]
-                L.qkv_h.f32, L.qkv_h.bf16, L.qkv_h.bf16_lo = wq32.data_ptr(), h16.data_ptr(), l16.data_ptr()
-                L.qkv_h.n, L.qkv_h.k = 4608, 1536
+                                         sd[p + "attn.linear_v.weight"]], 0), lo=False)          # bf16x3 reads qkv_ln
             L.fc = self._mat(sd[p + "attn.fc.weight"])
             f = p + "feed_forward."
-            L.conv1 = self._mat(sd[f + "conv1.conv.weight"].reshape(2048, 1536))
+            L.conv1 = self._mat(sd[f + "conv1.conv.weight"].reshape(2048, 1536), lo=False)         # bf16x3 reads conv1_ln
             L.bn1_scale, L.bn1_shift = self._bn(sd, f + "conv1.")
             L.dw_w = self._vec(sd[f + "depthwise_conv.conv.weight"].reshape(2048, 9).t())   # tap-major [9, 2048]
             L.bn2_scale, L.bn2_shift = self._bn(sd, f + "depthwise_conv.")

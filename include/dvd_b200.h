@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define DVD_ABI_VERSION 4
+#define DVD_ABI_VERSION 5
 
 #if defined(__GNUC__)
 #define DVD_API __attribute__((visibility("default")))
@@ -46,14 +46,15 @@ extern "C" {
 /* precision of the denoiser's dense contractions */
 #define DVD_PREC_FP32  0      /* fp32 FFMA reference mode (bit-for-bit reproducible)   */
 #define DVD_PREC_BF16  1      /* bf16 operands, fp32 accumulate on tcgen05 / TMEM (fast, reduced accuracy)        */
-#define DVD_PREC_BF16X3 2     /* fp32-accurate tensor-core mode: every GEMM operand is a bf16 pair hi+lo and runs */
-                              /* three tcgen05 passes (hi*hi + lo*hi + hi*lo, error ~2^-16); attention in fp16     */
+#define DVD_PREC_BF16X3 2     /* fp32-accurate tensor-core mode: GEMM operands are bf16 pairs hi+lo and run three */
+                              /* tcgen05 passes (hi*hi + lo*hi + hi*lo, error ~2^-16); the pyramid and the        */
+                              /* decoder's q|k|v run two (fp16 activation x fp16 weight pair); attention in fp16   */
 
 /* One dense weight matrix W[n][k] (row-major, K contiguous == torch Linear layout). */
 typedef struct dvd_mat {
   const float* f32;           /* always present                                       */
   const void*  bf16;          /* bf16(W) for the tensor modes (may be NULL in fp32)    */
-  const void*  bf16_lo;       /* bf16(W - bf16(W)) for DVD_PREC_BF16X3 (else NULL)     */
+  const void*  bf16_lo;       /* bf16(W - bf16(W)) where a precision runs this matrix on bf16 pairs (DVD_PREC_BF16X3), else NULL */
   int32_t n, k;
 } dvd_mat_t;
 
@@ -68,12 +69,9 @@ typedef struct dvd_dec_layer {          /* CA:343-396 DecoderLayer, CA:13-57 fee
   const float *bn2_scale, *bn2_shift;
   dvd_mat_t conv2;                      /* [1536,2048]                                    */
   const float *bn3_scale, *bn3_shift;
-  /* LayerNorm folded into the consumer GEMM (DVD_PREC_BF16X3): W' = W * gamma (per input channel), colsum[n] = sum_k W'[n][k] of the
-   * ROUNDED pair, cvec = W beta.  The epilogue computes rstd * (x W'^T - mean * colsum) + cvec from the raw residual rows. */
-  /* The q|k|v GEMM of DVD_PREC_BF16X3 takes ONE fp16 activation value per element (two tensor passes instead of three; q, k, v are
-   * rounded to fp16 for the attention anyway).  tcgen05 kind::f16 cannot mix fp16 and bf16 operands, so these weights are ALSO
-   * packed as an IEEE fp16 pair: qkv_h.bf16 = fp16(W), qkv_h.bf16_lo = fp16(W - fp16(W)).  NULL pointers: the three-pass path runs. */
-  dvd_mat_t qkv_h;                      /* [4608,1536], fp16 hi / lo in the bf16 / bf16_lo slots */
+  /* LayerNorm folded into the consumer GEMM, required for DVD_PREC_BF16X3 (which reads these instead of qkv / conv1): W' = W * gamma
+   * (per input channel), colsum[n] = sum_k W'[n][k] of the ROUNDED pair, cvec = W beta.  The epilogue computes
+   * rstd * (x W'^T - mean * colsum) + cvec from the raw residual rows. */
   dvd_mat_t qkv_ln;                     /* [4608,1536] = qkv * norm1.weight, as an IEEE fp16 hi / lo pair (two-pass GEMM on fp16 raw rows) */
   const float *qkv_colsum, *qkv_cvec;   /* [4608]                                         */
   dvd_mat_t conv1_ln;                   /* [2048,1536] = conv1 * norm2.weight             */
@@ -103,9 +101,9 @@ typedef struct dvd_weights {
   const float *dec_ln_w, *dec_ln_b;     /* decoder.layer_norm (eps 1e-5)                   */
   dvd_mat_t fin;             const float* fin_b;                       /* [8,1536]         */
   dvd_mat_t fin_ada;         const float* fin_ada_b;                   /* [3072,1536]      */
-  /* DVD_PREC_BF16X3, optional: the pyramid weights (same packing as pyr[], level 0 K-padded to 64) as IEEE fp16 hi / lo pairs in the
-   * bf16 / bf16_lo slots.  When present the pyramid runs two tensor passes (ONE fp16 activation x weight pair; the oracle study finds no
-   * measurable map error from fp16 pyramid activations); NULL pointers: three passes on bf16 pairs. */
+  /* Required for DVD_PREC_BF16X3: the pyramid weights (same packing as pyr[], level 0 K-padded to 64) as IEEE fp16 hi / lo pairs in
+   * the bf16 / bf16_lo slots.  That precision runs the pyramid in two tensor passes (ONE fp16 activation x weight pair; the oracle study
+   * finds no measurable map error from fp16 pyramid activations) and reads pyr[].bf16 / .bf16_lo not at all. */
   dvd_mat_t pyr_h[7];
 } dvd_weights_t;
 

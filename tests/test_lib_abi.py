@@ -29,7 +29,7 @@ def test_library_exports_every_declared_symbol():
     for name in _declared():
         assert hasattr(lib, name), f"{name} declared in dvd_b200.h but not exported"
         assert name in _lib.SIGNATURES, f"{name} has no ctypes signature in dvd_b200/_lib.py"
-    assert lib.dvd_version() == 4
+    assert lib.dvd_version() == 5
     assert lib.dvd_workspace_bytes(0, 2, 0) == 0
     assert lib.dvd_workspace_bytes(1, 2, 0) > 100 << 20
 
