@@ -73,6 +73,7 @@ SIGNATURES = {
     "dvd_workspace_tensor": (_vp, [_vp, _i, _i, _i, C.c_char_p, C.POINTER(C.c_longlong)]),
     "dvd_test_gemm": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _sz, _vp]),
     "dvd_test_attention": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _vp, _sz, _vp]),
+    "dvd_test_dwconv": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp]),
     "dvd_gemm_bf16": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "dvd_gemm_tune": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "dvd_debug_stop_after": (_i, [_i]),

@@ -144,6 +144,14 @@ extern "C" int dvd_test_attention(const float* q, const float* k, const float* v
   return pair_to_f32(o16, x3 ? olo : nullptr, o, n, st);
 }
 
+// The decoder's depthwise 3x3 + folded BN + ReLU of the tensor modes on its own: [N,1024,C] bf16 (in_lo non-NULL: bf16 pairs) in and
+// out, the same launch dvd_denoise_step makes.
+extern "C" int dvd_test_dwconv(const void* in_hi, const void* in_lo, const float* w9, const float* scale, const float* shift, void* out_hi,
+                               void* out_lo, int N, int C, void* stream) {
+  return dwconv3x3_bn_relu_bf16((const __nv_bfloat16*)in_hi, (const __nv_bfloat16*)in_lo, w9, scale, shift, (__nv_bfloat16*)out_hi,
+                                (__nv_bfloat16*)out_lo, N, C, (cudaStream_t)stream);
+}
+
 // Plain tensor-core GEMM entry point (tuning / micro-benchmarks): out = A W^T + bias, bf16 output (and optional fp32 output).
 // A16_lo / W16_lo non-null: split-precision pairs (three passes).
 extern "C" int dvd_gemm_bf16(const void* A16, const void* A16_lo, int lda, const void* W16, const void* W16_lo, int ldw, const float* bias,

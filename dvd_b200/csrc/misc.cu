@@ -618,37 +618,68 @@ __global__ void __launch_bounds__(256) k_dwconv(const float4* __restrict__ in, c
   float r0 = fmaxf(acc.x * s.x + t.x, 0.f), r1 = fmaxf(acc.y * s.y + t.y, 0.f), r2 = fmaxf(acc.z * s.z + t.z, 0.f), r3 = fmaxf(acc.w * s.w + t.w, 0.f);
   store4(out, Out16{out16, nullptr}, i * 4, r0, r1, r2, r3);
 }
-// bf16 in / bf16 out variant for the tensor path: 8 channels (16 bytes) per thread, fp32 accumulation.
-// CTA = 8 x-positions (one per warp) x 256 channels (8 per lane) x a vertical strip of RS output rows.  The 9 x 256 tap weights and
-// the BN scale / shift of the CTA's channels are staged once in shared memory (they do not depend on the previous kernel, so this runs
-// ahead of griddepcontrol.wait); a thread walks the strip column by column (kx outer): 3 weight rows (ky) in registers, every input
-// row of the strip loaded once and fed to up to three output rows -> (RS+2)*3 activation loads + 18 LDS.128 per RS outputs, ~80
-// registers, one wave of 512 CTAs.
-template <int RS, int NW>
-__global__ void __launch_bounds__(32 * NW) k_dwconv_bf16(const uint4* __restrict__ in, const uint4* __restrict__ in_lo, const float* __restrict__ w9,
-                                                     const float* __restrict__ sc, const float* __restrict__ sh, uint4* __restrict__ out,
-                                                     uint4* __restrict__ out_lo, int C8) {
-  __shared__ __align__(16) float s_w[9][256];
-  __shared__ __align__(16) float s_sc[256], s_sh[256];
+// bf16 / bf16-pair variant for the tensor path.  CTA = one sample x one 64-channel slice x a band of kDwRows output rows across all
+// 32 x positions.  The kDwRows + 2 input rows of the band are loaded once from global memory (all ten 16-byte loads per thread and
+// array issued before any is used), converted to fp32 (hi + lo) and staged in shared memory; a thread then computes 8 channels of one
+// x position for the whole band from there, walking the input column by column (kx outer) like the fp32 kernel: per output the taps
+// are accumulated kx-major, ky-minor, and taps outside the image are skipped.  At batch 1 (N = 2) the 256 CTAs of 80 KB each run as
+// one wave at 2 CTAs per SM; larger batches just add CTAs (one flat grid index).
+constexpr int kDwRows = 8, kDwCh = 64, kDwThreads = 256;
+constexpr int kDwSmem = (kDwRows + 2) * 32 * kDwCh * 4;
+// float4 slot of channel quad q (0..15) inside a 64-channel row: the upper half is shifted by one slot so that the 8 threads of a
+// quarter-warp (8 channel groups reading quads 2g, 2g + 1) hit 8 distinct 4-bank groups
+__device__ __forceinline__ int dw_slot(int q) { return q ^ (q >> 3); }
+
+__global__ void __launch_bounds__(kDwThreads, 2) k_dwconv_band(const uint4* __restrict__ in, const uint4* __restrict__ in_lo,
+                                                               const float4* __restrict__ w9, const float4* __restrict__ sc,
+                                                               const float4* __restrict__ sh, uint4* __restrict__ out,
+                                                               uint4* __restrict__ out_lo, int C8) {
+  extern __shared__ float4 s_in[];                        // [kDwRows + 2][32 x][16 slots]: fp32 hi + lo of input rows y0-1 .. y0+kDwRows
+  __shared__ float4 s_w[9][16], s_sc[16], s_sh[16];
   pdl_trigger();
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int c8 = blockIdx.x * 32 + lane;                  // 8-channel group of this thread
-  const int x = blockIdx.y * NW + warp;
-  const int strips = 32 / RS;
-  const size_t n = blockIdx.z / strips;
-  const int y0 = (blockIdx.z % strips) * RS;
-  const int C = C8 * 8, cb = blockIdx.x * 256;            // first channel of the CTA
-  for (int e = threadIdx.x; e < 9 * 256; e += 32 * NW) s_w[e >> 8][e & 255] = (cb + (e & 255) < C) ? __ldg(w9 + (size_t)(e >> 8) * C + cb + (e & 255)) : 0.f;
-  for (int e = threadIdx.x; e < 256; e += 32 * NW) {
-    s_sc[e] = (cb + e < C) ? __ldg(sc + cb + e) : 0.f;
-    s_sh[e] = (cb + e < C) ? __ldg(sh + cb + e) : 0.f;
+  constexpr int bands = 32 / kDwRows;
+  const int slices = C8 / 8;                              // 64-channel slices
+  const int slice = blockIdx.x % slices, band = (blockIdx.x / slices) % bands;
+  const size_t n = blockIdx.x / slices / bands;
+  const int y0 = band * kDwRows, C4 = C8 * 2;
+  const int g = threadIdx.x & 7, x = threadIdx.x >> 3;    // this thread's 8 channels (quads 2g, 2g + 1) and x position
+  // taps and BN of the slice do not depend on the previous kernel: staged before griddepcontrol.wait
+  for (int e = threadIdx.x; e < 11 * 16; e += kDwThreads) {
+    const int q = e & 15, c4 = slice * 16 + q;
+    if (e < 9 * 16) s_w[e >> 4][dw_slot(q)] = __ldg(w9 + (size_t)(e >> 4) * C4 + c4);
+    else if (e < 10 * 16) s_sc[dw_slot(q)] = __ldg(sc + c4);
+    else s_sh[dw_slot(q)] = __ldg(sh + c4);
+  }
+  pdl_wait();
+  const size_t base = n * 1024 * C8 + slice * 8 + g;     // 16-byte lane (sample n, token 0, this thread's channel group)
+  uint4 vh[kDwRows + 2], vl[kDwRows + 2];
+#pragma unroll
+  for (int i = 0; i < kDwRows + 2; ++i) {                 // staged row i = input row y0 - 1 + i
+    const int yy = y0 - 1 + i;
+    if (yy < 0 || yy >= 32) continue;
+    vh[i] = __ldg(in + base + (size_t)(yy * 32 + x) * C8);
+    if (in_lo) vl[i] = __ldg(in_lo + base + (size_t)(yy * 32 + x) * C8);
+  }
+#pragma unroll
+  for (int i = 0; i < kDwRows + 2; ++i) {
+    const int yy = y0 - 1 + i;
+    if (yy < 0 || yy >= 32) continue;
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&vh[i]);
+    float f[8] = {__low2float(h[0]), __high2float(h[0]), __low2float(h[1]), __high2float(h[1]),
+                  __low2float(h[2]), __high2float(h[2]), __low2float(h[3]), __high2float(h[3])};
+    if (in_lo) {                                          // split pair: value = hi + lo
+      const __nv_bfloat162* hl = reinterpret_cast<const __nv_bfloat162*>(&vl[i]);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) { f[2 * k] += __low2float(hl[k]); f[2 * k + 1] += __high2float(hl[k]); }
+    }
+    float4* row = s_in + (i * 32 + x) * 16;
+    row[dw_slot(2 * g)] = make_float4(f[0], f[1], f[2], f[3]);
+    row[dw_slot(2 * g + 1)] = make_float4(f[4], f[5], f[6], f[7]);
   }
   __syncthreads();
-  pdl_wait();
-  if (c8 >= C8) return;
-  float acc[RS][8];
+  float acc[kDwRows][8];
 #pragma unroll
-  for (int o = 0; o < RS; ++o)
+  for (int o = 0; o < kDwRows; ++o)
 #pragma unroll
     for (int k = 0; k < 8; ++k) acc[o][k] = 0.f;
 #pragma unroll 1                                             // (one copy of the column body: the kernel's code is fetched cold on every launch)
@@ -658,57 +689,52 @@ __global__ void __launch_bounds__(32 * NW) k_dwconv_bf16(const uint4* __restrict
     float w[3][8];
 #pragma unroll
     for (int ky = 0; ky < 3; ++ky) {
-      const float4 w0 = *reinterpret_cast<const float4*>(&s_w[ky * 3 + kx][lane * 8]);
-      const float4 w1 = *reinterpret_cast<const float4*>(&s_w[ky * 3 + kx][lane * 8 + 4]);
+      const float4 w0 = s_w[ky * 3 + kx][dw_slot(2 * g)], w1 = s_w[ky * 3 + kx][dw_slot(2 * g + 1)];
       w[ky][0] = w0.x; w[ky][1] = w0.y; w[ky][2] = w0.z; w[ky][3] = w0.w; w[ky][4] = w1.x; w[ky][5] = w1.y; w[ky][6] = w1.z; w[ky][7] = w1.w;
     }
 #pragma unroll
-    for (int r = -1; r <= RS; ++r) {
+    for (int r = -1; r <= kDwRows; ++r) {
       const int yy = y0 + r;
       if (yy < 0 || yy >= 32) continue;
-      const uint4 v = __ldg(in + (n * 1024 + yy * 32 + xx) * C8 + c8);
-      const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&v);
-      float f[8] = {__low2float(h[0]), __high2float(h[0]), __low2float(h[1]), __high2float(h[1]),
-                    __low2float(h[2]), __high2float(h[2]), __low2float(h[3]), __high2float(h[3])};
-      if (in_lo) {                                         // split pair: value = hi + lo
-        const uint4 vl = __ldg(in_lo + (n * 1024 + yy * 32 + xx) * C8 + c8);
-        const __nv_bfloat162* hl = reinterpret_cast<const __nv_bfloat162*>(&vl);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) { f[2 * k] += __low2float(hl[k]); f[2 * k + 1] += __high2float(hl[k]); }
-      }
+      const float4* p = s_in + ((r + 1) * 32 + xx) * 16;
+      const float4 a = p[dw_slot(2 * g)], b = p[dw_slot(2 * g + 1)];
+      const float f[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
 #pragma unroll
       for (int ky = 0; ky < 3; ++ky) {
-        const int o = r + 1 - ky;                          // output row (inside the strip) that sees input row r through tap row ky
-        if (o < 0 || o >= RS) continue;
+        const int o = r + 1 - ky;                          // output row (inside the band) that sees input row r through tap row ky
+        if (o < 0 || o >= kDwRows) continue;
 #pragma unroll
         for (int k = 0; k < 8; ++k) acc[o][k] = fmaf(f[k], w[ky][k], acc[o][k]);
       }
     }
   }
-  const float4 s0 = *reinterpret_cast<const float4*>(&s_sc[lane * 8]), s1 = *reinterpret_cast<const float4*>(&s_sc[lane * 8 + 4]);
-  const float4 t0 = *reinterpret_cast<const float4*>(&s_sh[lane * 8]), t1 = *reinterpret_cast<const float4*>(&s_sh[lane * 8 + 4]);
+  const float4 s0 = s_sc[dw_slot(2 * g)], s1 = s_sc[dw_slot(2 * g + 1)];
+  const float4 t0 = s_sh[dw_slot(2 * g)], t1 = s_sh[dw_slot(2 * g + 1)];
 #pragma unroll
-  for (int o = 0; o < RS; ++o) {
+  for (int o = 0; o < kDwRows; ++o) {
     const float r8[8] = {fmaxf(acc[o][0] * s0.x + t0.x, 0.f), fmaxf(acc[o][1] * s0.y + t0.y, 0.f), fmaxf(acc[o][2] * s0.z + t0.z, 0.f),
                          fmaxf(acc[o][3] * s0.w + t0.w, 0.f), fmaxf(acc[o][4] * s1.x + t1.x, 0.f), fmaxf(acc[o][5] * s1.y + t1.y, 0.f),
                          fmaxf(acc[o][6] * s1.z + t1.z, 0.f), fmaxf(acc[o][7] * s1.w + t1.w, 0.f)};
     uint4 ov, ol;
     split_bf16x2(r8[0], r8[1], ov.x, ol.x); split_bf16x2(r8[2], r8[3], ov.y, ol.y);
     split_bf16x2(r8[4], r8[5], ov.z, ol.z); split_bf16x2(r8[6], r8[7], ov.w, ol.w);
-    out[(n * 1024 + (size_t)(y0 + o) * 32 + x) * C8 + c8] = ov;
-    if (out_lo) out_lo[(n * 1024 + (size_t)(y0 + o) * 32 + x) * C8 + c8] = ol;
+    const size_t at = base + (size_t)((y0 + o) * 32 + x) * C8;
+    out[at] = ov;
+    if (out_lo) out_lo[at] = ol;
   }
 }
 int dwconv3x3_bn_relu_bf16(const __nv_bfloat16* in, const __nv_bfloat16* in_lo, const float* w9c, const float* scale, const float* shift,
                            __nv_bfloat16* out, __nv_bfloat16* out_lo, int N, int C, cudaStream_t st) {
-  DVD_REQUIRE(in && w9c && scale && shift && out && C % 8 == 0, "dwconv_bf16: bad args");
-  // 4 warps (4 columns) per CTA: at ~93 registers a 256-thread CTA fits twice per SM, and the 512 CTAs of one document then run as
-  // 1.7 waves of 296; the 1024 CTAs of 128 threads (5 per SM) backfill much more evenly.
-  constexpr int RS = 4, NW = 4;
-  DVD_REQUIRE((long long)N * (32 / RS) <= 65535, "dwconv_bf16: batch too large for the grid");
-  DVD_CUDA(launch_pdl(8, k_dwconv_bf16<RS, NW>, dim3(cdiv(C / 8, 32), 32 / NW, N * (32 / RS)), dim3(32 * NW), (size_t)0, st, (const uint4*)in, (const uint4*)in_lo, w9c, scale,
-                      shift, (uint4*)out, (uint4*)out_lo, C / 8));
-  DVD_LAUNCH_CHECK("k_dwconv_bf16");
+  DVD_REQUIRE(in && w9c && scale && shift && out, "dwconv_bf16: null pointer");
+  DVD_REQUIRE(N > 0 && C > 0 && C % kDwCh == 0, "dwconv_bf16: N = %d, C = %d (C must be a positive multiple of %d)", N, C, kDwCh);
+  DVD_REQUIRE((((uintptr_t)in | (uintptr_t)in_lo | (uintptr_t)w9c | (uintptr_t)scale | (uintptr_t)shift | (uintptr_t)out | (uintptr_t)out_lo) & 15) == 0,
+              "dwconv_bf16: pointers must be 16-byte aligned");
+  const long long ctas = (long long)N * (32 / kDwRows) * (C / kDwCh);
+  DVD_REQUIRE(ctas <= 0x7fffffffLL, "dwconv_bf16: batch too large for the grid");
+  DVD_SET_MAX_SMEM(k_dwconv_band, kDwSmem);
+  DVD_CUDA(launch_pdl(8, k_dwconv_band, dim3((unsigned)ctas), dim3(kDwThreads), (size_t)kDwSmem, st, (const uint4*)in, (const uint4*)in_lo,
+                      (const float4*)w9c, (const float4*)scale, (const float4*)shift, (uint4*)out, (uint4*)out_lo, C / 8));
+  DVD_LAUNCH_CHECK("k_dwconv_band");
   return 0;
 }
 

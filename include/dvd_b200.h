@@ -213,6 +213,11 @@ DVD_API int dvd_test_gemm(const float* A, const float* W, const float* bias, flo
 DVD_API int dvd_test_attention(const float* q, const float* k, const float* v, float* o, int batch, int heads,
                        int T, int d, float scale, int precision, void* scratch, size_t scratch_bytes,
                        void* stream);
+/* Depthwise 3x3 (pad 1) over the 32x32 token grid + folded BN + ReLU as the decoder runs it in the tensor modes: in_hi / in_lo
+ * [N,1024,C] bf16 (value = hi + lo; in_lo NULL: hi alone), w9 [9,C] fp32 (tap ky*3+kx), scale / shift [C] fp32, out_hi / out_lo
+ * [N,1024,C] bf16 pair of the result (out_lo may be NULL).  C must be a multiple of 64, N > 0, every pointer 16-byte aligned. */
+DVD_API int dvd_test_dwconv(const void* in_hi, const void* in_lo, const float* w9, const float* scale, const float* shift,
+                            void* out_hi, void* out_lo, int N, int C, void* stream);
 /* Plain tensor-core GEMM (tuning / micro-benchmarks): out = A[M,K] W[N,K]^T + bias; bf16 operands (A16_lo / W16_lo non-NULL:
  * split pairs, three passes; A16_lo NULL next to a weight pair: A16, W16 and W16_lo hold IEEE fp16, two passes), bf16 and/or fp32 output.
  * dvd_test_gemm accepts precision 3 for the same two-pass mode (fp16 activation x fp16 weight pair). */
