@@ -17,6 +17,9 @@
 //                  and the vertically pre-blended coarse-map window in shared memory, gathers through L1;
 //   k_unwarp       fully general fallback (tiny photos / huge maps).
 // The 64x64 coarse map (32 KB) is read through the read-only path and stays L1/L2 resident.
+// k_unwarp_u8_mixed and k_unwarp_u8_sized run the uint8 tile bodies over a host-planned table of documents.  The sized kernel writes an
+// Ho x Wo page: EV:301,304 with size=(s*Ho, s*Wo) instead of the photo's (H, W), WP:73 at that grid, then the mean of each s x s block
+// (box supersampling when shrinking; s = 1 is the reference chain at the output size) before the .astype(uint8) truncation.
 #include "common.cuh"
 #include "tc_common.cuh"
 #include <stdlib.h>
@@ -126,11 +129,13 @@ constexpr int TILE_W = 128, TILE_H = 8;   // 32 x 8 threads, 4 px per thread
 //
 // The per-tile bodies (unwarp_tile, unwarp_tile_fast) take photo / output / map bases, a geometry and the tile (x, y, image b):
 // the fixed-size kernels pass the batch bases and blockIdx (so their address arithmetic is the one they always had), the
-// persistent mixed-size kernel one document's bases, its own tile walk and b = 0.  A body never returns early (the persistent
-// loop has barriers): rows past the photo skip the work and still reach every __syncthreads.
+// persistent mixed-size and sized kernels one document's bases, their own tile walk and b = 0.  A body never returns early (the
+// persistent loop has barriers): rows past the output skip the work and still reach every __syncthreads.
+// The geometry g is the OUTPUT's (coordinate chain, tile walk, output rows); Hi x Wi is the photo the taps read.  Every caller but
+// the sized kernel passes Hi = g.H, Wi = g.W.
 template <int IN_U8, int OUT_U8, int C>
 __device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, const float* __restrict__ map, void* __restrict__ out_,
-                                            const UnwarpGeom& g, unsigned tx, unsigned ty, unsigned b) {
+                                            const UnwarpGeom& g, unsigned tx, unsigned ty, unsigned b, int Hi, int Wi) {
   __shared__ float s_bx[TILE_W], s_lx[TILE_W], s_by[TILE_H], s_ly[TILE_H];
   __shared__ int s_x0[TILE_W], s_y0[TILE_H];
   const int tid = threadIdx.y * 32 + threadIdx.x;
@@ -152,7 +157,7 @@ __device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, con
   // a warp is one tile row; its lanes left of the right edge are a prefix of the warp, and only they take part in the vote below
   if (i < g.H && j0 < g.W) {
   const int W = g.W, H = g.H;
-  const int plane = H * W;                                      // < 2^31 elements per image (checked on the host)
+  const int plane = H * W, pplane = Hi * Wi;                    // output / photo: < 2^31 elements per image (checked on the host)
   const float* __restrict__ mapb = map + (size_t)b * 2 * g.mh * g.mw;
   const int y0m = s_y0[threadIdx.y] & 0xffff, dy = (s_y0[threadIdx.y] >> 16) * g.mw;
   const float ly1 = s_ly[threadIdx.y], ly0 = 1.0f - ly1, byv = s_by[threadIdx.y];
@@ -174,8 +179,8 @@ __device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, con
     const float sy = ly0 * (lx0 * __ldg(m1) + lx1 * __ldg(m1 + xp)) + ly1 * (lx0 * __ldg(m1 + dy) + lx1 * __ldg(m1 + dy + xp));
     const float gx = ((sx + s_bx[cj]) * 2.0f - 1.0f) * g.affine;
     const float gy = ((sy + byv) * 2.0f - 1.0f) * g.affine;
-    const Taps t = make_taps(gx, gy, H, W);
-    off[p] = t.y0 * W + t.x0;
+    const Taps t = make_taps(gx, gy, Hi, Wi);
+    off[p] = t.y0 * Wi + t.x0;
     wnw[p] = t.nw; wne[p] = t.ne; wsw[p] = t.sw; wse[p] = t.se;
     vmask[p] = (int)t.vx0 | ((int)t.vx1 << 1) | ((int)t.vy0 << 2) | ((int)t.vy1 << 3);
     inside = inside && (vmask[p] == 15 || j0 + p >= W);
@@ -186,7 +191,7 @@ __device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, con
   if (__all_sync(live == 32 ? 0xffffffffu : (1u << live) - 1u, inside) && j0 + 3 < W) {
     // ---- fast path: every tap of every pixel of this warp is inside the photo
     if (IN_U8) {
-      const uint8_t* __restrict__ ph = (const uint8_t*)photo_ + (size_t)b * plane * C;
+      const uint8_t* __restrict__ ph = (const uint8_t*)photo_ + (size_t)b * pplane * C;
 #pragma unroll
       for (int p = 0; p < 4; ++p) {
         const uint8_t* q = ph + (size_t)off[p] * C;
@@ -194,23 +199,23 @@ __device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, con
         for (int c = 0; c < C; ++c) {
           float v = (float)__ldg(q + c) * wnw[p];
           v += (float)__ldg(q + C + c) * wne[p];
-          v += (float)__ldg(q + (size_t)W * C + c) * wsw[p];
-          v += (float)__ldg(q + (size_t)(W + 1) * C + c) * wse[p];
+          v += (float)__ldg(q + (size_t)Wi * C + c) * wsw[p];
+          v += (float)__ldg(q + (size_t)(Wi + 1) * C + c) * wse[p];
           res[c][p] = v;
         }
       }
     } else {
-      const float* __restrict__ ph = (const float*)photo_ + (size_t)b * C * plane;
+      const float* __restrict__ ph = (const float*)photo_ + (size_t)b * C * pplane;
 #pragma unroll
       for (int c = 0; c < C; ++c) {
-        const float* pc = ph + (size_t)c * plane;
+        const float* pc = ph + (size_t)c * pplane;
 #pragma unroll
         for (int p = 0; p < 4; ++p) {
           const float* q = pc + off[p];
           float v = __ldg(q) * wnw[p];
           v += __ldg(q + 1) * wne[p];
-          v += __ldg(q + W) * wsw[p];
-          v += __ldg(q + W + 1) * wse[p];
+          v += __ldg(q + Wi) * wsw[p];
+          v += __ldg(q + Wi + 1) * wse[p];
           res[c][p] = v;
         }
       }
@@ -226,17 +231,17 @@ __device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, con
       for (int c = 0; c < C; ++c) {
         float v = 0.f;
         if (IN_U8) {
-          const uint8_t* q = (const uint8_t*)photo_ + ((size_t)b * plane + off[p]) * C + c;
+          const uint8_t* q = (const uint8_t*)photo_ + ((size_t)b * pplane + off[p]) * C + c;
           if (t.vy0 & t.vx0) v += (float)__ldg(q) * t.nw;
           if (t.vy0 & t.vx1) v += (float)__ldg(q + C) * t.ne;
-          if (t.vy1 & t.vx0) v += (float)__ldg(q + (long long)W * C) * t.sw;
-          if (t.vy1 & t.vx1) v += (float)__ldg(q + (long long)(W + 1) * C) * t.se;
+          if (t.vy1 & t.vx0) v += (float)__ldg(q + (long long)Wi * C) * t.sw;
+          if (t.vy1 & t.vx1) v += (float)__ldg(q + (long long)(Wi + 1) * C) * t.se;
         } else {
-          const float* q = (const float*)photo_ + ((size_t)b * C + c) * plane + off[p];
+          const float* q = (const float*)photo_ + ((size_t)b * C + c) * pplane + off[p];
           if (t.vy0 & t.vx0) v += __ldg(q) * t.nw;
           if (t.vy0 & t.vx1) v += __ldg(q + 1) * t.ne;
-          if (t.vy1 & t.vx0) v += __ldg(q + W) * t.sw;
-          if (t.vy1 & t.vx1) v += __ldg(q + W + 1) * t.se;
+          if (t.vy1 & t.vx0) v += __ldg(q + Wi) * t.sw;
+          if (t.vy1 & t.vx1) v += __ldg(q + Wi + 1) * t.se;
         }
         res[c][p] = v;
       }
@@ -277,7 +282,7 @@ __device__ __forceinline__ void unwarp_tile(const void* __restrict__ photo_, con
 template <int IN_U8, int OUT_U8, int C>
 __global__ void __launch_bounds__(256) k_unwarp(const void* __restrict__ photo_, const float* __restrict__ map,
                                                 void* __restrict__ out_, UnwarpGeom g) {
-  unwarp_tile<IN_U8, OUT_U8, C>(photo_, map, out_, g, blockIdx.x, blockIdx.y, blockIdx.z);
+  unwarp_tile<IN_U8, OUT_U8, C>(photo_, map, out_, g, blockIdx.x, blockIdx.y, blockIdx.z, g.H, g.W);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -292,7 +297,8 @@ constexpr int UW_WIN = 16;
 
 template <int IN_U8, int OUT_U8, int C>
 __device__ __forceinline__ void unwarp_tile_fast(const void* __restrict__ photo_, const float* __restrict__ map,
-                                                 void* __restrict__ out_, const UnwarpGeom& g, unsigned tx, unsigned ty, unsigned b) {
+                                                 void* __restrict__ out_, const UnwarpGeom& g, unsigned tx, unsigned ty, unsigned b,
+                                                 int Hi, int Wi) {
   __shared__ float s_bx[TILE_W], s_lx[TILE_W], s_by[TILE_H], s_ly[TILE_H];
   __shared__ int s_kx[TILE_W], s_y0[TILE_H];
   __shared__ float s_v[2][TILE_H][UW_WIN];
@@ -332,9 +338,9 @@ __device__ __forceinline__ void unwarp_tile_fast(const void* __restrict__ photo_
   if (i < g.H) {                                          // load/store then covers 32 CONSECUTIVE pixels (one 128-byte line);
                                                           // whole warps skip (a warp is one tile row): *_sync masks stay valid
   const int W = g.W, H = g.H;
-  const int plane = H * W;
+  const int plane = H * W, pplane = Hi * Wi;                  // output / photo
   const float byv = s_by[threadIdx.y];
-  const float fw = (float)(W - 1), fh = (float)(H - 1);
+  const float fw = (float)(Wi - 1), fh = (float)(Hi - 1);
   int off[4];
   float wnw[4], wne[4], wsw[4], wse[4];
   int x0s[4], y0s[4];
@@ -354,16 +360,16 @@ __device__ __forceinline__ void unwarp_tile_fast(const void* __restrict__ photo_
     const float ax = ix - fx, ay = iy - fy, bx = (fx + 1.f) - ix, byw = (fy + 1.f) - iy;
     wnw[p] = bx * byw; wne[p] = ax * byw; wsw[p] = bx * ay; wse[p] = ax * ay;
     x0s[p] = x0; y0s[p] = y0;
-    off[p] = y0 * W + x0;
-    inside = inside && (((unsigned)x0 < (unsigned)(W - 1)) & ((unsigned)y0 < (unsigned)(H - 1)));
+    off[p] = y0 * Wi + x0;
+    inside = inside && (((unsigned)x0 < (unsigned)(Wi - 1)) & ((unsigned)y0 < (unsigned)(Hi - 1)));
   }
   float res[C][4];
   if (__all_sync(0xffffffffu, inside) && jt0 + TILE_W <= W) {
     // all-inside path.  Address arithmetic is kept to one 64-bit pointer per pixel plus one add per channel / row: the tap
     // loads then use immediate offsets (profiles/r1_ncu_unwarp.txt showed ~6 integer instructions per load before this).
     if (IN_U8) {
-      const uint8_t* __restrict__ ph = (const uint8_t*)photo_ + (size_t)b * plane * C;
-      const size_t rowb = (size_t)W * C;
+      const uint8_t* __restrict__ ph = (const uint8_t*)photo_ + (size_t)b * pplane * C;
+      const size_t rowb = (size_t)Wi * C;
 #pragma unroll
       for (int p = 0; p < 4; ++p) {
         const uint8_t* q0 = ph + (size_t)off[p] * C;
@@ -378,15 +384,15 @@ __device__ __forceinline__ void unwarp_tile_fast(const void* __restrict__ photo_
         }
       }
     } else {
-      const float* __restrict__ ph = (const float*)photo_ + (size_t)b * C * plane;
+      const float* __restrict__ ph = (const float*)photo_ + (size_t)b * C * pplane;
 #pragma unroll
       for (int p = 0; p < 4; ++p) {
         const float* q0 = ph + off[p];
-        const float* q1 = q0 + W;
+        const float* q1 = q0 + Wi;
 #pragma unroll
         for (int c = 0; c < C; ++c) {
-          const float* a = q0 + (size_t)c * plane;
-          const float* d = q1 + (size_t)c * plane;
+          const float* a = q0 + (size_t)c * pplane;
+          const float* d = q1 + (size_t)c * pplane;
           float v = __ldg(a) * wnw[p];
           v += __ldg(a + 1) * wne[p];
           v += __ldg(d) * wsw[p];
@@ -401,23 +407,23 @@ __device__ __forceinline__ void unwarp_tile_fast(const void* __restrict__ photo_
     for (int p = 0; p < 4; ++p) {
       const int x0 = x0s[p], y0 = y0s[p];
       const bool px_ok = (j0 + 32 * p < W);
-      const bool vx0 = px_ok && x0 >= 0 && x0 < W, vx1 = px_ok && x0 >= -1 && x0 < W - 1;
-      const bool vy0 = y0 >= 0 && y0 < H, vy1 = y0 >= -1 && y0 < H - 1;
+      const bool vx0 = px_ok && x0 >= 0 && x0 < Wi, vx1 = px_ok && x0 >= -1 && x0 < Wi - 1;
+      const bool vy0 = y0 >= 0 && y0 < Hi, vy1 = y0 >= -1 && y0 < Hi - 1;
 #pragma unroll
       for (int c = 0; c < C; ++c) {
         float v = 0.f;
         if (IN_U8) {
-          const uint8_t* base = (const uint8_t*)photo_ + (size_t)b * plane * C + c;
-          if (vy0 && vx0) v += (float)__ldg(base + ((long long)y0 * W + x0) * C) * wnw[p];
-          if (vy0 && vx1) v += (float)__ldg(base + ((long long)y0 * W + x0 + 1) * C) * wne[p];
-          if (vy1 && vx0) v += (float)__ldg(base + ((long long)(y0 + 1) * W + x0) * C) * wsw[p];
-          if (vy1 && vx1) v += (float)__ldg(base + ((long long)(y0 + 1) * W + x0 + 1) * C) * wse[p];
+          const uint8_t* base = (const uint8_t*)photo_ + (size_t)b * pplane * C + c;
+          if (vy0 && vx0) v += (float)__ldg(base + ((long long)y0 * Wi + x0) * C) * wnw[p];
+          if (vy0 && vx1) v += (float)__ldg(base + ((long long)y0 * Wi + x0 + 1) * C) * wne[p];
+          if (vy1 && vx0) v += (float)__ldg(base + ((long long)(y0 + 1) * Wi + x0) * C) * wsw[p];
+          if (vy1 && vx1) v += (float)__ldg(base + ((long long)(y0 + 1) * Wi + x0 + 1) * C) * wse[p];
         } else {
-          const float* base = (const float*)photo_ + ((size_t)b * C + c) * plane;
-          if (vy0 && vx0) v += __ldg(base + (long long)y0 * W + x0) * wnw[p];
-          if (vy0 && vx1) v += __ldg(base + (long long)y0 * W + x0 + 1) * wne[p];
-          if (vy1 && vx0) v += __ldg(base + (long long)(y0 + 1) * W + x0) * wsw[p];
-          if (vy1 && vx1) v += __ldg(base + (long long)(y0 + 1) * W + x0 + 1) * wse[p];
+          const float* base = (const float*)photo_ + ((size_t)b * C + c) * pplane;
+          if (vy0 && vx0) v += __ldg(base + (long long)y0 * Wi + x0) * wnw[p];
+          if (vy0 && vx1) v += __ldg(base + (long long)y0 * Wi + x0 + 1) * wne[p];
+          if (vy1 && vx0) v += __ldg(base + (long long)(y0 + 1) * Wi + x0) * wsw[p];
+          if (vy1 && vx1) v += __ldg(base + (long long)(y0 + 1) * Wi + x0 + 1) * wse[p];
         }
         res[c][p] = v;
       }
@@ -447,7 +453,7 @@ __device__ __forceinline__ void unwarp_tile_fast(const void* __restrict__ photo_
 template <int IN_U8, int OUT_U8, int C>
 __global__ void __launch_bounds__(256) k_unwarp_fast(const void* __restrict__ photo_, const float* __restrict__ map,
                                                      void* __restrict__ out_, UnwarpGeom g) {
-  unwarp_tile_fast<IN_U8, OUT_U8, C>(photo_, map, out_, g, blockIdx.x, blockIdx.y, blockIdx.z);
+  unwarp_tile_fast<IN_U8, OUT_U8, C>(photo_, map, out_, g, blockIdx.x, blockIdx.y, blockIdx.z, g.H, g.W);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -879,8 +885,8 @@ __global__ void __launch_bounds__(256) k_unwarp_u8_mixed(const MixedTableHeader*
     const int r = t - d.tile_begin, ty = r / d.tiles_x, tx = r - ty * d.tiles_x;
     const float* mapb = map + (size_t)lo * 2 * g.mh * g.mw;          // document d reads map row d
     __syncthreads();                      // the previous tile's threads are done reading the shared tables the prologue rewrites
-    if (d.fast) unwarp_tile_fast<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0);
-    else        unwarp_tile<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0);
+    if (d.fast) unwarp_tile_fast<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0, g.H, g.W);
+    else        unwarp_tile<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0, g.H, g.W);
   }
 }
 
@@ -950,6 +956,249 @@ static int launch_unwarp_u8_mixed(const void* table, int C, const float* map, cu
   return 0;
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Sized batch (uint8 HWC): document d dewarps its Hi x Wi photo into an Ho x Wo output.  With supersampling factor s, output pixel
+// (i, j) is the mean of the s x s block (s*i + a, s*j + b) of the reference chain evaluated on the VIRTUAL s*Ho x s*Wo grid:
+//   out = trunc(avg_pool2d(grid_sample(photo, fullres_grid(map[d], s*Ho, s*Wo)), s))
+// s = 1 documents run the fixed-size bodies on their output geometry (fast body under the same window rule as plan_mixed), so a
+// same-size s = 1 document is dvd_unwarp_u8 byte for byte.  s > 1 documents run unwarp_tile_ss.  The table design (host plan,
+// device table, grid independent of the table) is the mixed-size batch's; a separate kernel keeps k_unwarp_u8_mixed's registers.
+struct SizedDoc {                         // 88 bytes
+  const uint8_t* photo;
+  uint8_t* out;
+  UnwarpGeom g;                           // s = 1: make_geom(Ho, Wo); s > 1: make_geom(s*Ho, s*Wo), the virtual grid
+  int32_t Hi, Wi, Ho, Wo;                 // photo, output
+  int32_t s, win;                         // supersampling factor; win: fast body (s = 1) / pre-blended map window (s > 1)
+  int32_t tiles_x, tile_begin;            // tile_begin: prefix sum of the tiles of the documents before
+};
+static_assert(sizeof(SizedDoc) == 88, "sized unwarp table layout");
+constexpr int SS_TW = 32, SS_TH = 8, SS_MAX = 8;   // output tile of the supersampling body (one pixel per thread); largest factor
+
+// One 32 x 8 output tile of an s > 1 document: thread (x, y) owns output pixel (ty*8 + y, tx*32 + x) and accumulates its s*s
+// subsamples a-major, b-minor, in fp32; the mean is truncated like .astype(uint8).  Each subsample runs the coordinate chain of an
+// s = 1 pixel of the virtual grid from per-tile column / row tables (8*s rows, 32*s columns); the coarse map is blended
+// vertically once per virtual row when the tile touches at most UW_WIN map columns (fast body's order), else it is read per
+// subsample in the general body's order.
+// One thread per output pixel rather than one lane per subsample column + a shuffle reduction over groups of s lanes: the
+// reduction would idle 32 mod s lanes for s in {3,5,6,7} and sum in a tree order, while here every lane is busy for every s, the
+// order is a plain sequential sum, and the s-pixel stride between neighbouring lanes' taps costs more L1 wavefronts per load, not
+// more bytes: the b loop re-reads the same lines from L1 a few instructions later.
+template <int C>
+__device__ __forceinline__ void unwarp_tile_ss(const uint8_t* __restrict__ photo, const float* __restrict__ map, uint8_t* __restrict__ out,
+                                               const UnwarpGeom& g, int s, bool win, int Ho, int Wo, int Hi, int Wi, unsigned tx,
+                                               unsigned ty) {
+  __shared__ float s_bx[SS_TW * SS_MAX], s_lx[SS_TW * SS_MAX], s_by[SS_TH * SS_MAX], s_ly[SS_TH * SS_MAX];
+  __shared__ int s_kx[SS_TW * SS_MAX], s_y0[SS_TH * SS_MAX];
+  __shared__ float s_v[2][SS_TH * SS_MAX][UW_WIN];
+  const int tid = threadIdx.y * 32 + threadIdx.x;
+  const int vw = SS_TW * s, vh = SS_TH * s;               // virtual columns / rows of the tile
+  const int jt0 = tx * vw, it0 = ty * vh;
+  int wx0 = 0;                                            // first map column of the window (0: absolute column indices)
+  if (win) {
+    int xp; float l0, l1;
+    up_coeff(g.sx, min(jt0, g.W - 1), g.mw, wx0, xp, l0, l1);
+  }
+  for (int e = tid; e < vw + vh; e += SS_TW * SS_TH) {    // virtual columns / rows past the edge repeat the last one
+    if (e < vw) {
+      const int j = min(jt0 + e, g.W - 1);
+      int x0, xp; float l0, l1;
+      up_coeff(g.sx, j, g.mw, x0, xp, l0, l1);
+      s_kx[e] = (x0 - wx0) | (xp << 16); s_lx[e] = l1; s_bx[e] = base_ramp(g.bx, j);
+    } else {
+      const int r = e - vw, i = min(it0 + r, g.H - 1);
+      int y0, yp; float l0, l1;
+      up_coeff(g.sy, i, g.mh, y0, yp, l0, l1);
+      s_y0[r] = y0 | (yp << 16); s_ly[r] = l1; s_by[r] = base_ramp(g.by, i);
+    }
+  }
+  __syncthreads();
+  if (win) {                                              // vertical blend of the map window: [channel][virtual row][window column]
+    for (int e = tid; e < 2 * vh * UW_WIN; e += SS_TW * SS_TH) {
+      const int k = e % UW_WIN, r = (e / UW_WIN) % vh, ch = e / (UW_WIN * vh);
+      const int col = min(wx0 + k, g.mw - 1);
+      const int y0 = s_y0[r] & 0xffff, yp = s_y0[r] >> 16;
+      const float l1 = s_ly[r], l0 = 1.0f - l1;
+      const float* m = map + (size_t)ch * g.mh * g.mw + (size_t)y0 * g.mw + col;
+      s_v[ch][r][k] = l0 * __ldg(m) + l1 * __ldg(m + yp * g.mw);
+    }
+  }
+  __syncthreads();
+  const int io = ty * SS_TH + threadIdx.y, jo = tx * SS_TW + threadIdx.x;
+  if (io < Ho && jo < Wo) {
+    const float fw = (float)(Wi - 1), fh = (float)(Hi - 1);
+    const int mplane = g.mh * g.mw;
+    float acc[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) acc[c] = 0.f;
+#pragma unroll 1
+    for (int a = 0; a < s; ++a) {
+      const int rr = threadIdx.y * s + a;
+      const int dy = (s_y0[rr] >> 16) * g.mw;
+      const float ly1 = s_ly[rr], ly0 = 1.0f - ly1, byv = s_by[rr];
+      const float* __restrict__ mrow = map + (s_y0[rr] & 0xffff) * g.mw;
+#pragma unroll 1
+      for (int b = 0; b < s; ++b) {
+        const int cj = threadIdx.x * s + b;
+        const int k = s_kx[cj] & 0xffff, xp = s_kx[cj] >> 16;
+        const float lx1 = s_lx[cj], lx0 = 1.0f - lx1;
+        float sx, sy;
+        if (win) {
+          sx = lx0 * s_v[0][rr][k] + lx1 * s_v[0][rr][k + xp];
+          sy = lx0 * s_v[1][rr][k] + lx1 * s_v[1][rr][k + xp];
+        } else {
+          const float* m0 = mrow + k;
+          const float* m1 = m0 + mplane;
+          sx = ly0 * (lx0 * __ldg(m0) + lx1 * __ldg(m0 + xp)) + ly1 * (lx0 * __ldg(m0 + dy) + lx1 * __ldg(m0 + dy + xp));
+          sy = ly0 * (lx0 * __ldg(m1) + lx1 * __ldg(m1 + xp)) + ly1 * (lx0 * __ldg(m1 + dy) + lx1 * __ldg(m1 + dy + xp));
+        }
+        const float gx = ((sx + s_bx[cj]) * 2.0f - 1.0f) * g.affine;
+        const float gy = ((sy + byv) * 2.0f - 1.0f) * g.affine;
+        const float ix = ((gx + 1.f) / 2.f) * fw, iy = ((gy + 1.f) / 2.f) * fh;      // grid_sampler_unnormalize, align_corners=True
+        const int x0 = __float2int_rd(ix), y0 = __float2int_rd(iy);
+        const float fx = (float)x0, fy = (float)y0;
+        const float ax = ix - fx, ay = iy - fy, bxw = (fx + 1.f) - ix, byw = (fy + 1.f) - iy;
+        const float wnw = bxw * byw, wne = ax * byw, wsw = bxw * ay, wse = ax * ay;
+        if (((unsigned)x0 < (unsigned)(Wi - 1)) & ((unsigned)y0 < (unsigned)(Hi - 1))) {
+          const uint8_t* q0 = photo + ((size_t)y0 * Wi + x0) * C;
+          const uint8_t* q1 = q0 + (size_t)Wi * C;
+#pragma unroll
+          for (int c = 0; c < C; ++c) {
+            float v = (float)__ldg(q0 + c) * wnw;
+            v += (float)__ldg(q0 + C + c) * wne;
+            v += (float)__ldg(q1 + c) * wsw;
+            v += (float)__ldg(q1 + C + c) * wse;
+            acc[c] += v;
+          }
+        } else {
+          // per-tap validity (zeros padding); coordinates may be wild, so validity is tested before any address is formed
+          const bool vx0 = x0 >= 0 && x0 < Wi, vx1 = x0 >= -1 && x0 < Wi - 1;
+          const bool vy0 = y0 >= 0 && y0 < Hi, vy1 = y0 >= -1 && y0 < Hi - 1;
+#pragma unroll
+          for (int c = 0; c < C; ++c) {
+            float v = 0.f;
+            if (vy0 && vx0) v += (float)__ldg(photo + ((long long)y0 * Wi + x0) * C + c) * wnw;
+            if (vy0 && vx1) v += (float)__ldg(photo + ((long long)y0 * Wi + x0 + 1) * C + c) * wne;
+            if (vy1 && vx0) v += (float)__ldg(photo + ((long long)(y0 + 1) * Wi + x0) * C + c) * wsw;
+            if (vy1 && vx1) v += (float)__ldg(photo + ((long long)(y0 + 1) * Wi + x0 + 1) * C + c) * wse;
+            acc[c] += v;
+          }
+        }
+      }
+    }
+    const float n = (float)(s * s);
+    uint8_t* o = out + ((size_t)io * Wo + jo) * C;
+#pragma unroll
+    for (int c = 0; c < C; ++c) o[c] = to_u8_trunc(acc[c] / n);
+  }
+}
+
+// At least 3 CTAs per SM (80 registers) for C <= 3 and 2 for C = 4: the most that compile without spills (ptxas's own choice,
+// 64 registers for C <= 3, spills a few bytes; 3 CTAs at C = 4 spill 8 bytes)
+template <int C>
+__global__ void __launch_bounds__(256, C < 4 ? 3 : 2) k_unwarp_u8_sized(const MixedTableHeader* __restrict__ hdr, const SizedDoc* __restrict__ docs,
+                                                         const float* __restrict__ map) {
+  const int n_docs = __ldg(&hdr->n_docs), total = __ldg(&hdr->total_tiles);
+  if (__ldg(&hdr->C) != C) return;        // planned for another channel count: write nothing (uniform over the grid)
+  for (int t = blockIdx.x; t < total; t += gridDim.x) {
+    int lo = 0, hi = n_docs - 1;          // the document of tile t (see k_unwarp_u8_mixed)
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (__ldg(&docs[mid].tile_begin) <= t) lo = mid; else hi = mid - 1;
+    }
+    const SizedDoc& d = docs[lo];
+    const UnwarpGeom g = d.g;
+    const int r = t - d.tile_begin, ty = r / d.tiles_x, tx = r - ty * d.tiles_x;
+    const float* mapb = map + (size_t)lo * 2 * g.mh * g.mw;
+    __syncthreads();                      // the previous tile's threads are done reading the shared tables the prologue rewrites
+    if (d.s > 1)    unwarp_tile_ss<C>(d.photo, mapb, d.out, g, d.s, d.win, d.Ho, d.Wo, d.Hi, d.Wi, tx, ty);
+    else if (d.win) unwarp_tile_fast<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0, d.Hi, d.Wi);
+    else            unwarp_tile<1, 1, C>(d.photo, mapb, d.out, g, tx, ty, 0, d.Hi, d.Wi);
+  }
+}
+
+static size_t sized_table_bytes(int max_docs) {
+  return max_docs < 0 ? 0 : sizeof(MixedTableHeader) + (size_t)max_docs * sizeof(SizedDoc);
+}
+
+static int plan_sized(const dvd_unwarp_sized_doc_t* docs_host, int n_docs, int C, int mh, int mw, float affine, void* table_host,
+                      size_t table_bytes, long long* total_tiles, int32_t* s_out) {
+  DVD_REQUIRE(n_docs >= 0 && (n_docs == 0 || docs_host) && table_host, "unwarp_u8_sized_plan: n_docs=%d, docs %p, table %p", n_docs,
+              (const void*)docs_host, table_host);
+  DVD_REQUIRE(table_bytes >= sized_table_bytes(n_docs),
+              "unwarp_u8_sized_plan: table of %zu bytes is too small for %d documents (%zu needed)", table_bytes, n_docs,
+              sized_table_bytes(n_docs));
+  DVD_REQUIRE(C >= 1 && C <= 4, "unwarp_u8_sized_plan: C=%d outside 1..4", C);
+  DVD_REQUIRE(mh >= 1 && mw >= 1 && mh < 65536 && mw < 65536, "unwarp_u8_sized_plan: bad map size %dx%d", mh, mw);
+  MixedTableHeader* hdr = static_cast<MixedTableHeader*>(table_host);
+  SizedDoc* recs = reinterpret_cast<SizedDoc*>(hdr + 1);
+  long long tiles = 0;
+  for (int d = 0; d < n_docs; ++d) {
+    const dvd_unwarp_sized_doc_t& in = docs_host[d];
+    DVD_REQUIRE(in.H >= 0 && in.W >= 0 && in.Ho >= 0 && in.Wo >= 0,
+                "unwarp_u8_sized_plan: document %d has a negative size (photo %dx%d, output %dx%d)", d, in.H, in.W, in.Ho, in.Wo);
+    DVD_REQUIRE(in.supersample >= 0 && in.supersample <= 8, "unwarp_u8_sized_plan: document %d has supersample=%d outside 0..8", d,
+                in.supersample);
+    DVD_REQUIRE((long long)in.H * in.W * C < (1ll << 31), "unwarp_u8_sized_plan: document %d photo (%dx%dx%d) is too large for 32-bit offsets",
+                d, in.H, in.W, C);
+    DVD_REQUIRE((long long)in.Ho * in.Wo * C < (1ll << 31),
+                "unwarp_u8_sized_plan: document %d output (%dx%dx%d) is too large for 32-bit offsets", d, in.Ho, in.Wo, C);
+    const bool empty = in.H == 0 || in.W == 0 || in.Ho == 0 || in.Wo == 0;
+    DVD_REQUIRE(empty || (in.photo && in.out), "unwarp_u8_sized_plan: document %d has a null photo or output pointer", d);
+    int s = in.supersample;
+    if (s == 0) s = empty ? 1 : std::min(8, std::max({1, cdiv(in.H, in.Ho), cdiv(in.W, in.Wo)}));
+    DVD_REQUIRE((long long)s * in.Ho < (1ll << 31) && (long long)s * in.Wo < (1ll << 31),
+                "unwarp_u8_sized_plan: document %d output %dx%d at supersample %d is too large for 32-bit coordinates", d, in.Ho, in.Wo, s);
+    SizedDoc r;
+    r.photo = in.photo; r.out = in.out;
+    r.g = make_geom(s * in.Ho, s * in.Wo, mh, mw, affine);
+    r.Hi = in.H; r.Wi = in.W; r.Ho = in.Ho; r.Wo = in.Wo; r.s = s;
+    if (s == 1) {                         // the rule of launch_unwarp / plan_mixed, on the output geometry
+      r.win = (int)(127.0f * r.g.sx) + 3 <= UW_WIN && in.Wo > 1 && in.Ho > 1;
+      r.tiles_x = empty ? 0 : cdiv(in.Wo, TILE_W);
+    } else {                              // map columns a 32*s-column virtual tile can touch
+      r.win = (int)((float)(SS_TW * s - 1) * r.g.sx) + 3 <= UW_WIN;
+      r.tiles_x = empty ? 0 : cdiv(in.Wo, SS_TW);
+    }
+    r.tile_begin = (int32_t)tiles;
+    tiles += empty ? 0 : (long long)r.tiles_x * cdiv(in.Ho, s == 1 ? TILE_H : SS_TH);
+    DVD_REQUIRE(tiles < MIXED_MAX_TILES, "unwarp_u8_sized_plan: more than %d tiles in one batch", MIXED_MAX_TILES);
+    recs[d] = r;
+    if (s_out) s_out[d] = s;
+  }
+  *hdr = MixedTableHeader{n_docs, (int32_t)tiles, C, 0};
+  if (total_tiles) *total_tiles = tiles;
+  return 0;
+}
+
+static int launch_unwarp_u8_sized(const void* table, int C, const float* map, cudaStream_t st) {
+  DVD_REQUIRE(table && map, "unwarp_u8_sized: null pointer");
+  DVD_REQUIRE(C >= 1 && C <= 4, "unwarp_u8_sized: C=%d outside 1..4", C);
+  const MixedTableHeader* hdr = static_cast<const MixedTableHeader*>(table);
+  const SizedDoc* docs = reinterpret_cast<const SizedDoc*>(hdr + 1);
+  int dev = 0, n_sm = 0;
+  DVD_CUDA(cudaGetDevice(&dev));
+  DVD_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+  DVD_REQUIRE(dev < 64, "unwarp_u8_sized: device %d", dev);
+#define DVD_UNWARP_SIZED(CC)                                                                                                       \
+  do {                                                                                                                             \
+    static int per_sm[64] = {};                   /* per device: occupancy of this instantiation */                                \
+    if (!per_sm[dev]) {                                                                                                            \
+      DVD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm[dev], k_unwarp_u8_sized<CC>, 256, 0));                        \
+      DVD_REQUIRE(per_sm[dev] >= 1, "unwarp_u8_sized: kernel does not fit an SM");                                                 \
+    }                                                                                                                              \
+    k_unwarp_u8_sized<CC><<<n_sm * per_sm[dev], dim3(32, 8), 0, st>>>(hdr, docs, map);                                             \
+  } while (0)
+  switch (C) {
+    case 1: DVD_UNWARP_SIZED(1); break;
+    case 2: DVD_UNWARP_SIZED(2); break;
+    case 3: DVD_UNWARP_SIZED(3); break;
+    default: DVD_UNWARP_SIZED(4); break;
+  }
+#undef DVD_UNWARP_SIZED
+  DVD_LAUNCH_CHECK("k_unwarp_u8_sized");
+  return 0;
+}
+
 }  // namespace dvd
 
 using namespace dvd;
@@ -973,6 +1222,14 @@ extern "C" int dvd_unwarp_u8_plan(const dvd_unwarp_doc_t* docs_host, int n_docs,
 }
 extern "C" int dvd_unwarp_u8_mixed(const void* table, int C, const float* map, void* stream) {
   return launch_unwarp_u8_mixed(table, C, map, (cudaStream_t)stream);
+}
+extern "C" size_t dvd_unwarp_sized_table_bytes(int max_docs) { return sized_table_bytes(max_docs); }
+extern "C" int dvd_unwarp_u8_sized_plan(const dvd_unwarp_sized_doc_t* docs_host, int n_docs, int C, int mh, int mw, float affine,
+                                        void* table_host, size_t table_bytes, long long* total_tiles, int32_t* supersample_out) {
+  return plan_sized(docs_host, n_docs, C, mh, mw, affine, table_host, table_bytes, total_tiles, supersample_out);
+}
+extern "C" int dvd_unwarp_u8_sized(const void* table, int C, const float* map, void* stream) {
+  return launch_unwarp_u8_sized(table, C, map, (cudaStream_t)stream);
 }
 extern "C" int dvd_fullres_grid_f32(const float* map, float* grid, int B, int H, int W, int mh, int mw, float affine,
                                     void* stream) {

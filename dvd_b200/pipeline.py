@@ -8,6 +8,10 @@ image runs in libdvd_b200; torch only owns the buffers and the stream.
 With ``max_pixels=P`` the pipeline takes photos of different sizes in one batch (mixed-size mode): ``photo_u8`` is then a list of
 uint8 HWC tensors whose pixel counts sum to at most P, the results are a list of uint8 HWC images, and one unwarp launch, captured
 once per set of buffers, serves every composition of sizes.
+
+With ``out_size`` the dewarped pages come out at a requested size instead of the photo's: a ``(Ho, Wo)`` tuple, or a callable
+``(H, W) -> (Ho, Wo)`` evaluated per photo.  The unwarp step is then the sized launch (supersampled when shrinking), so only the
+smaller pages are written and downloaded.
 """
 from __future__ import annotations
 
@@ -20,16 +24,26 @@ import torch
 from . import _lib
 from .model import DiT
 from .sampler import create_gaussian_diffusion
-from .unwarp import AFFINE, plan_mixed, table_bytes
+from .unwarp import AFFINE, plan_mixed, plan_sized, size_arg, sized_table_bytes, supersample_arg, table_bytes
 
 
 class DewarpPipeline:
     def __init__(self, model: DiT, diffusion_steps: int = 3, n_batch: int = 2, docs: int = 1, height: int = 1500, width: int = 2000,
-                 noise_schedule: str = "cosine", precision: str | None = None, max_pixels: int | None = None):
+                 noise_schedule: str = "cosine", precision: str | None = None, max_pixels: int | None = None, out_size=None,
+                 supersample="auto", max_out_pixels: int | None = None):
         self.model, self.docs, self.n_batch, self.H, self.W = model, docs, n_batch, height, width
         self.max_pixels = max_pixels
         if max_pixels is not None and max_pixels < 1:
             raise ValueError(f"max_pixels must be positive, got {max_pixels}")
+        # output size (None: the photo's).  Fixed-size mode: one (Ho, Wo) for the batch; mixed-size mode: per photo, into an arena
+        # of max_out_pixels (default max_pixels)
+        self.out_size, self.supersample = out_size, supersample_arg(supersample)
+        if out_size is not None and not callable(out_size):
+            size_arg(out_size, "out_size")
+        if max_out_pixels is not None and (out_size is None or max_pixels is None or max_out_pixels < 1):
+            raise ValueError("max_out_pixels takes a positive count and applies to mixed-size mode (max_pixels) with out_size")
+        self.max_out_pixels = max_out_pixels if max_out_pixels is not None else max_pixels
+        self.HWo = self._out_hw(height, width) if out_size is not None and max_pixels is None else (height, width)
         self.precision = precision or model.precision
         self.dev = model.device
         if self.dev.type != "cuda":
@@ -42,17 +56,20 @@ class DewarpPipeline:
             z = lambda *s, dt=torch.float32: torch.zeros(s, dtype=dt, device=self.dev)
             # mixed-size mode: photos and outputs live in byte arenas, each document at a 16-byte aligned offset
             img = (docs, height, width, 3) if max_pixels is None else (3 * max_pixels + 16 * docs,)
+            oimg = (docs,) + self.HWo + (3,) if max_pixels is None else (3 * self.max_out_pixels + 16 * docs,)
             self.buf = {"y512": z(docs, 3, 512, 512), "mask_cat": z(docs, 1, 512, 512), "mask_y512": z(docs, 384, 64, 64),
                         "line_msk": z(docs, 64, 64, 64), "x_T": z(docs * n_batch, 2, 64, 64),
                         "photo_u8": z(*img, dt=torch.uint8)}
             self.init_flow0 = z(docs, 2, 64, 64)                       # evaluation.py:180 (use_init_flow=False)
             self.map64 = z(docs, 2, 64, 64)
-            self.out_u8 = z(*img, dt=torch.uint8)
-            self.out_host = torch.empty(img, dtype=torch.uint8).pin_memory()
+            self.out_u8 = z(*oimg, dt=torch.uint8)
+            self.out_host = torch.empty(oimg, dtype=torch.uint8).pin_memory()
             if max_pixels is not None:                                # run_device's unwarp table (host plan -> device copy)
-                self._table = z(table_bytes(docs), dt=torch.uint8)
-                self._table_host = torch.empty(table_bytes(docs), dtype=torch.uint8).pin_memory()
+                tb = table_bytes(docs) if out_size is None else sized_table_bytes(docs)
+                self._table = z(tb, dt=torch.uint8)
+                self._table_host = torch.empty(tb, dtype=torch.uint8).pin_memory()
                 self._ev_table = torch.cuda.Event()
+            self._fixed_tables = {}            # fixed-size mode with out_size: (photo, out) pointers -> sized table, planned once
         self.h2d_bytes = sum(v.numel() * v.element_size() for v in self.buf.values())
         self.d2h_bytes = self.out_u8.numel()
         self.use_graph = os.environ.get("DVD_NO_GRAPH", "0") != "1"
@@ -91,6 +108,45 @@ class DewarpPipeline:
         """mixed-size unwarp of the batch planned into the device table d["table"] (one launch whatever the composition)."""
         _lib.check(self.lib.dvd_unwarp_u8_mixed(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), "dvd_unwarp_u8_mixed")
 
+    def _enqueue_unwarp_sized(self, d: dict):
+        """sized unwarp of the batch planned into the device table d["table"] (one launch whatever the composition)."""
+        _lib.check(self.lib.dvd_unwarp_u8_sized(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), "dvd_unwarp_u8_sized")
+
+    def _out_hw(self, H: int, W: int) -> tuple:
+        """output size of an H x W photo"""
+        return size_arg(self.out_size(H, W) if callable(self.out_size) else self.out_size, f"out_size for a {H}x{W} photo")
+
+    def _fixed_table(self, photo: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+        """device table of the sized launch photo [docs,H,W,3] -> out [docs,Ho,Wo,3], planned and uploaded once per buffer pair
+        (a graph captured with it keeps it alive through its input dict)"""
+        key = (photo.data_ptr(), out.data_ptr())
+        if key not in self._fixed_tables:
+            nb = sized_table_bytes(self.docs)
+            host = torch.empty(nb, dtype=torch.uint8).pin_memory()
+            plan_sized(host, list(photo.unbind(0)), list(out.unbind(0)), 64, 64, self.supersample)
+            table = torch.empty(nb, dtype=torch.uint8, device=self.dev)
+            table.copy_(host, non_blocking=True)
+            if len(self._fixed_tables) >= 16:
+                self._fixed_tables.pop(next(iter(self._fixed_tables)))
+            self._fixed_tables[key] = (table, host)                  # the pinned block stays alive until its upload has run
+        return self._fixed_tables[key][0]
+
+    def _out_shapes(self, photos) -> list:
+        """output shapes of a mixed-size batch: the photos' own, or their out_size shapes (at most max_out_pixels in all)"""
+        if self.out_size is None:
+            return [tuple(p.shape) for p in photos]
+        shapes = [self._out_hw(p.shape[0], p.shape[1]) + (3,) for p in photos]
+        px = sum(Ho * Wo for Ho, Wo, _ in shapes)
+        if px > self.max_out_pixels:
+            raise ValueError(f"the batch's outputs have {px} pixels, more than max_out_pixels={self.max_out_pixels}")
+        return shapes
+
+    def _plan_batch(self, table_host: torch.Tensor, photos, outs):
+        if self.out_size is None:
+            plan_mixed(table_host, photos, outs, 64, 64)
+        else:
+            plan_sized(table_host, photos, outs, 64, 64, self.supersample)
+
     def _check_photos(self, photos, device: torch.device, lo: int) -> list:
         """Validates the photos of a mixed-size batch (lo..docs uint8 HWC RGB tensors on `device`, at most max_pixels in all)."""
         if not isinstance(photos, (list, tuple)):
@@ -113,11 +169,13 @@ class DewarpPipeline:
 
     @staticmethod
     def _arena_views(arena: torch.Tensor, photos) -> list:
-        """one [H,W,3] view per photo, packed at 16-byte aligned offsets"""
+        """one [H,W,3] view per photo (tensor or shape), packed at 16-byte aligned offsets"""
         views, off = [], 0
         for p in photos:
-            views.append(arena[off:off + p.numel()].view(p.shape))
-            off = (off + p.numel() + 15) & ~15
+            shape = tuple(p.shape) if isinstance(p, torch.Tensor) else tuple(p)
+            n = shape[0] * shape[1] * shape[2]
+            views.append(arena[off:off + n].view(shape))
+            off = (off + n + 15) & ~15
         return views
 
     def _graph(self, which: str, d: dict, keys, fn):
@@ -158,19 +216,28 @@ class DewarpPipeline:
             return self._run_device_mixed(d)
         with torch.cuda.device(self.dev):
             self._run("sampling", d, self.SAMPLING_KEYS, self._enqueue_sampling)
-            self._run("unwarp", d, ("photo_u8",), self._enqueue_unwarp)
+            if self.out_size is None:
+                self._run("unwarp", d, ("photo_u8",), self._enqueue_unwarp)
+            else:
+                photo = d["photo_u8"]
+                if photo.dtype != torch.uint8 or tuple(photo.shape) != (self.docs, self.H, self.W, 3) or not photo.is_contiguous():
+                    raise ValueError(f"photo_u8: expected a contiguous uint8 tensor {(self.docs, self.H, self.W, 3)}, got "
+                                     f"{photo.dtype} {tuple(photo.shape)}")
+                du = {"photo_u8": photo, "table": self._fixed_table(photo, self.out_u8)}
+                self._run("unwarp", du, ("photo_u8", "table"), self._enqueue_unwarp_sized)
         return self.out_u8
 
     def _run_device_mixed(self, d: dict) -> list:
         photos = self._check_photos(d["photo_u8"], self.dev, self.docs)
+        outs = self._arena_views(self.out_u8, self._out_shapes(photos))
         with torch.cuda.device(self.dev):
             self._run("sampling", d, self.SAMPLING_KEYS, self._enqueue_sampling)
-            outs = self._arena_views(self.out_u8, photos)
             self._ev_table.synchronize()                               # the previous upload has read the pinned table
-            plan_mixed(self._table_host, photos, outs, 64, 64)
+            self._plan_batch(self._table_host, photos, outs)
             self._table.copy_(self._table_host, non_blocking=True)
             self._ev_table.record()
-            self._run("unwarp", {"table": self._table}, ("table",), self._enqueue_unwarp_mixed)
+            self._run("unwarp", {"table": self._table}, ("table",),
+                      self._enqueue_unwarp_mixed if self.out_size is None else self._enqueue_unwarp_sized)
         return outs
 
     # ---- pinned-host inputs -> host uint8 image (H2D and D2H inside the call)
@@ -188,6 +255,8 @@ class DewarpPipeline:
             if self.max_pixels is not None:
                 buf["table"] = torch.empty_like(self._table)
                 slot.update(table_host=torch.empty_like(self._table_host).pin_memory(), ev_table=torch.cuda.Event(), views=None)
+            elif self.out_size is not None:
+                buf["table"] = self._fixed_table(buf["photo_u8"], buf["out_u8"])
             self._slots.append(slot)
         self._submitted = 0
 
@@ -221,7 +290,7 @@ class DewarpPipeline:
                 main.wait_event(s["ev_out"])                       # the download of batch ticket-2 has read this slot's output
             self._run("sampling", s["buf"], self.SAMPLING_KEYS, self._enqueue_sampling)
             main.wait_event(s["ev_photo"])
-            self._run("unwarp", s["buf"], ("photo_u8", "out_u8"), self._enqueue_unwarp)
+            self._run("unwarp", s["buf"], ("photo_u8", "out_u8"), self._enqueue_unwarp if self.out_size is None else self._enqueue_unwarp_sized)
             s["ev_done"].record(main)
             with torch.cuda.stream(self._d2h):
                 self._d2h.wait_event(s["ev_done"])
@@ -232,6 +301,7 @@ class DewarpPipeline:
 
     def _submit_host_mixed(self, h: dict) -> int:
         photos = self._check_photos(h["photo_u8"], torch.device("cpu"), 1)
+        out_shapes = self._out_shapes(photos)
         n = len(photos)
         for k in self.SAMPLING_KEYS:
             want = (n * self.n_batch if k == "x_T" else n,) + tuple(self.buf[k].shape[1:])
@@ -246,7 +316,7 @@ class DewarpPipeline:
             s = self._slots[ticket % 2]
             buf = s["buf"]
             photo_dev = self._arena_views(buf["photo_u8"], photos)
-            out_dev = self._arena_views(buf["out_u8"], photos)
+            out_dev = self._arena_views(buf["out_u8"], out_shapes)
             with torch.cuda.stream(self._h2d):
                 if s["used"]:
                     self._h2d.wait_event(s["ev_done"])             # the kernels of batch ticket-2 have read this slot's inputs
@@ -263,18 +333,18 @@ class DewarpPipeline:
             # the device only waits for batch ticket-2 through events; the HOST rewrites the pinned table now, so the upload of
             # ticket-2 must have read it (normally long done)
             s["ev_table"].synchronize()
-            plan_mixed(s["table_host"], photo_dev, out_dev, 64, 64)
+            self._plan_batch(s["table_host"], photo_dev, out_dev)
             buf["table"].copy_(s["table_host"], non_blocking=True)
             s["ev_table"].record(main)
             main.wait_event(s["ev_photo"])
-            self._run("unwarp", buf, ("table",), self._enqueue_unwarp_mixed)
+            self._run("unwarp", buf, ("table",), self._enqueue_unwarp_mixed if self.out_size is None else self._enqueue_unwarp_sized)
             s["ev_done"].record(main)
             end = out_dev[-1].data_ptr() - buf["out_u8"].data_ptr() + out_dev[-1].numel()
             with torch.cuda.stream(self._d2h):
                 self._d2h.wait_event(s["ev_done"])
                 s["out_host"][:end].copy_(buf["out_u8"][:end], non_blocking=True)
                 s["ev_out"].record()
-            s["views"] = self._arena_views(s["out_host"], photos)
+            s["views"] = self._arena_views(s["out_host"], out_dev)
             s["used"] = True
         return ticket
 

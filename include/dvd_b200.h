@@ -144,6 +144,29 @@ DVD_API int dvd_unwarp_u8_plan(const dvd_unwarp_doc_t* docs_host, int n_docs, in
                                void* table_host, size_t table_bytes, long long* total_tiles);
 /* one launch; table = the uploaded plan; C must equal the planned C (a table planned for another C is ignored: nothing is written) */
 DVD_API int dvd_unwarp_u8_mixed(const void* table, int C, const float* map, void* stream);
+/* Sized uint8 HWC batch: document d dewarps its H x W photo into an Ho x Wo output (any size, per document) in ONE launch, with
+ * the table design of the mixed-size batch above (host plan -> device copy -> launch; a graph captured once serves every plan).
+ * With supersampling factor s the output is the mean of each s x s block of the reference chain evaluated at s*Ho x s*Wo:
+ *   out = trunc(avg_pool2d(grid_sample(photo, fullres_grid(map[d], s*Ho, s*Wo)), s))
+ * s = 1 and Ho x Wo = H x W is dvd_unwarp_u8, byte for byte.  supersample = 0 picks s = min(8, max(1, ceil(H/Ho), ceil(W/Wo))).
+ * A document with H, W, Ho or Wo = 0 is empty (owns no tile; its pointers may be NULL). */
+typedef struct dvd_unwarp_sized_doc {
+  const uint8_t* photo;                 /* [H,W,C] uint8, device   */
+  uint8_t* out;                         /* [Ho,Wo,C] uint8, device */
+  int32_t H, W;                         /* photo                   */
+  int32_t Ho, Wo;                       /* output                  */
+  int32_t supersample;                  /* 0 = auto, 1..8          */
+  int32_t pad;
+} dvd_unwarp_sized_doc_t;
+/* bytes of a sized table for up to max_docs documents */
+DVD_API size_t dvd_unwarp_sized_table_bytes(int max_docs);
+/* host only: validates (C in 1..4, sizes >= 0, supersample in 0..8, H*W*C and Ho*Wo*C < 2^31, non-NULL pointers of non-empty
+ * documents, table_bytes large enough, map size) and fills table_host; *total_tiles (may be NULL) = the tiles of the batch,
+ * supersample_out[d] (may be NULL) = the factor chosen for document d. */
+DVD_API int dvd_unwarp_u8_sized_plan(const dvd_unwarp_sized_doc_t* docs_host, int n_docs, int C, int mh, int mw, float affine,
+                                     void* table_host, size_t table_bytes, long long* total_tiles, int32_t* supersample_out);
+/* one launch; a table planned for another C is ignored (nothing is written) */
+DVD_API int dvd_unwarp_u8_sized(const void* table, int C, const float* map, void* stream);
 /* WP:14-23,50-73 register_model2 / SpatialTransformer2: generic bilinear grid_sample,
  * align_corners=True, zeros padding.  img [B,C,H,W], grid [B,2,Ho,Wo] (ch0=x, ch1=y), out [B,C,Ho,Wo]. */
 DVD_API int dvd_grid_sample_f32(const float* img, const float* grid, float* out, int B, int C, int H, int W,
