@@ -52,6 +52,10 @@ class SizedUnwarpDoc(C.Structure):
                 ("supersample", C.c_int32), ("pad", C.c_int32)]
 
 
+class Y512Doc(C.Structure):
+    _fields_ = [("photo", _vp), ("H", C.c_int32), ("W", C.c_int32)]
+
+
 # name -> (restype, argtypes); mirrors include/dvd_b200.h one to one
 _i, _f, _sz = C.c_int, C.c_float, C.c_size_t
 _WP = C.POINTER(Weights)
@@ -70,6 +74,9 @@ SIGNATURES = {
     "dvd_unwarp_u8_sized_plan": (_i, [C.POINTER(SizedUnwarpDoc), _i, _i, _i, _i, _f, _vp, _sz, C.POINTER(C.c_longlong),
                                       C.POINTER(C.c_int32)]),
     "dvd_unwarp_u8_sized": (_i, [_vp, _i, _vp, _vp]),
+    "dvd_y512_table_bytes": (_sz, [_i]),
+    "dvd_y512_u8_plan": (_i, [C.POINTER(Y512Doc), _i, _vp, _sz]),
+    "dvd_y512_u8": (_i, [_vp, _vp, _vp]),
     "dvd_grid_sample_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "dvd_fullres_grid_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _f, _vp]),
     "dvd_workspace_bytes": (_sz, [_i, _i, _i]),

@@ -12,6 +12,10 @@ once per set of buffers, serves every composition of sizes.
 With ``out_size`` the dewarped pages come out at a requested size instead of the photo's: a ``(Ho, Wo)`` tuple, or a callable
 ``(H, W) -> (Ho, Wo)`` evaluated per photo.  The unwarp step is then the sized launch (supersampled when shrinking), so only the
 smaller pages are written and downloaded.
+
+With ``y512_from_photo=True`` the denoiser's 512x512 input is computed from ``photo_u8`` on the GPU (the reference loader's
+``cv2.resize(photo, (512, 512), INTER_LINEAR) / 255``, byte for byte) by one launch at the head of the sampling graph; the input
+dicts then carry no ``y512`` and the host path uploads none.
 """
 from __future__ import annotations
 
@@ -23,6 +27,7 @@ import torch
 
 from . import _lib
 from .model import DiT
+from .inputs import launch_y512, plan_y512, table_bytes as y512_table_bytes
 from .sampler import create_gaussian_diffusion
 from .unwarp import AFFINE, plan_mixed, plan_sized, size_arg, sized_table_bytes, supersample_arg, table_bytes
 
@@ -30,8 +35,13 @@ from .unwarp import AFFINE, plan_mixed, plan_sized, size_arg, sized_table_bytes,
 class DewarpPipeline:
     def __init__(self, model: DiT, diffusion_steps: int = 3, n_batch: int = 2, docs: int = 1, height: int = 1500, width: int = 2000,
                  noise_schedule: str = "cosine", precision: str | None = None, max_pixels: int | None = None, out_size=None,
-                 supersample="auto", max_out_pixels: int | None = None):
+                 supersample="auto", max_out_pixels: int | None = None, y512_from_photo: bool = False):
         self.model, self.docs, self.n_batch, self.H, self.W = model, docs, n_batch, height, width
+        # y512 computed from photo_u8 by the first launch of the sampling graph instead of supplied by the caller
+        self.y512_from_photo = bool(y512_from_photo)
+        self._input_keys = self.SAMPLING_KEYS[1:] if self.y512_from_photo else self.SAMPLING_KEYS
+        self._sampling_keys = self.SAMPLING_KEYS + ("prep",) if self.y512_from_photo else self.SAMPLING_KEYS
+        self._sampling = self._enqueue_prep_sampling if self.y512_from_photo else self._enqueue_sampling
         self.max_pixels = max_pixels
         if max_pixels is not None and max_pixels < 1:
             raise ValueError(f"max_pixels must be positive, got {max_pixels}")
@@ -69,8 +79,14 @@ class DewarpPipeline:
                 self._table = z(tb, dt=torch.uint8)
                 self._table_host = torch.empty(tb, dtype=torch.uint8).pin_memory()
                 self._ev_table = torch.cuda.Event()
-            self._fixed_tables = {}            # fixed-size mode with out_size: (photo, out) pointers -> sized table, planned once
-        self.h2d_bytes = sum(v.numel() * v.element_size() for v in self.buf.values())
+                if self.y512_from_photo:                              # run_device's y512 table, planned per batch
+                    self._prep_table = z(y512_table_bytes(docs), dt=torch.uint8)
+                    self._prep_host = torch.empty(y512_table_bytes(docs), dtype=torch.uint8).pin_memory()
+                    self._ev_prep = torch.cuda.Event()
+            # fixed-size mode, planned once per buffer: (photo, out) pointers -> sized unwarp table (with out_size), ("prep", photo)
+            # -> y512 table (with y512_from_photo)
+            self._fixed_tables = {}
+        self.h2d_bytes = sum(v.numel() * v.element_size() for k, v in self.buf.items() if k in self._input_keys + ("photo_u8",))
         self.d2h_bytes = self.out_u8.numel()
         self.use_graph = os.environ.get("DVD_NO_GRAPH", "0") != "1"
         self.kernel_launches = 0           # kernels of libdvd_b200 launched (or replayed) through this pipeline
@@ -98,6 +114,11 @@ class DewarpPipeline:
         self.eng.static_forward(d["y512"], d["mask_cat"], d["mask_y512"], d["line_msk"])
         self.eng.sample(d["x_T"], self.init_flow0, self.tables, self.t_scaled, self.a, self.b, None, self.map64)
 
+    def _enqueue_prep_sampling(self, d: dict):
+        """y512 from the photos planned into the device table d["prep"], then the sampling above."""
+        launch_y512(d["prep"], d["y512"])
+        self._enqueue_sampling(d)
+
     def _enqueue_unwarp(self, d: dict):
         """fused upsample + affine + bilinear unwarp of the full-resolution photo, on the current stream."""
         out = d.get("out_u8", self.out_u8)
@@ -111,6 +132,30 @@ class DewarpPipeline:
     def _enqueue_unwarp_sized(self, d: dict):
         """sized unwarp of the batch planned into the device table d["table"] (one launch whatever the composition)."""
         _lib.check(self.lib.dvd_unwarp_u8_sized(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), "dvd_unwarp_u8_sized")
+
+    def _check_fixed_photo(self, photo: torch.Tensor):
+        if photo.dtype != torch.uint8 or tuple(photo.shape) != (self.docs, self.H, self.W, 3) or not photo.is_contiguous():
+            raise ValueError(f"photo_u8: expected a contiguous uint8 tensor {(self.docs, self.H, self.W, 3)}, got "
+                             f"{photo.dtype} {tuple(photo.shape)}")
+
+    def _fixed_prep_table(self, photo: torch.Tensor) -> torch.Tensor:
+        """device table of the y512 launch of photo [docs,H,W,3], planned and uploaded once per buffer (kept alive like the sized
+        unwarp tables)"""
+        key = ("prep", photo.data_ptr())
+        if key not in self._fixed_tables:
+            nb = y512_table_bytes(self.docs)
+            host = torch.empty(nb, dtype=torch.uint8).pin_memory()
+            plan_y512(host, list(photo.unbind(0)))
+            table = torch.empty(nb, dtype=torch.uint8, device=self.dev)
+            table.copy_(host, non_blocking=True)
+            if len(self._fixed_tables) >= 16:
+                self._fixed_tables.pop(next(iter(self._fixed_tables)))
+            self._fixed_tables[key] = (table, host)
+        return self._fixed_tables[key][0]
+
+    def _no_y512(self, d: dict):
+        if "y512" in d:
+            raise ValueError("this pipeline computes y512 from photo_u8 (y512_from_photo=True); do not pass y512")
 
     def _out_hw(self, H: int, W: int) -> tuple:
         """output size of an H x W photo"""
@@ -215,14 +260,16 @@ class DewarpPipeline:
         if self.max_pixels is not None:
             return self._run_device_mixed(d)
         with torch.cuda.device(self.dev):
-            self._run("sampling", d, self.SAMPLING_KEYS, self._enqueue_sampling)
+            if self.y512_from_photo:
+                self._no_y512(d)
+                self._check_fixed_photo(d["photo_u8"])
+                d = dict(d, y512=self.buf["y512"], prep=self._fixed_prep_table(d["photo_u8"]))
+            self._run("sampling", d, self._sampling_keys, self._sampling)
             if self.out_size is None:
                 self._run("unwarp", d, ("photo_u8",), self._enqueue_unwarp)
             else:
                 photo = d["photo_u8"]
-                if photo.dtype != torch.uint8 or tuple(photo.shape) != (self.docs, self.H, self.W, 3) or not photo.is_contiguous():
-                    raise ValueError(f"photo_u8: expected a contiguous uint8 tensor {(self.docs, self.H, self.W, 3)}, got "
-                                     f"{photo.dtype} {tuple(photo.shape)}")
+                self._check_fixed_photo(photo)
                 du = {"photo_u8": photo, "table": self._fixed_table(photo, self.out_u8)}
                 self._run("unwarp", du, ("photo_u8", "table"), self._enqueue_unwarp_sized)
         return self.out_u8
@@ -231,7 +278,14 @@ class DewarpPipeline:
         photos = self._check_photos(d["photo_u8"], self.dev, self.docs)
         outs = self._arena_views(self.out_u8, self._out_shapes(photos))
         with torch.cuda.device(self.dev):
-            self._run("sampling", d, self.SAMPLING_KEYS, self._enqueue_sampling)
+            if self.y512_from_photo:
+                self._no_y512(d)
+                self._ev_prep.synchronize()                            # the previous upload has read the pinned table
+                plan_y512(self._prep_host, photos)
+                self._prep_table.copy_(self._prep_host, non_blocking=True)
+                self._ev_prep.record()
+                d = dict(d, y512=self.buf["y512"], prep=self._prep_table)
+            self._run("sampling", d, self._sampling_keys, self._sampling)
             self._ev_table.synchronize()                               # the previous upload has read the pinned table
             self._plan_batch(self._table_host, photos, outs)
             self._table.copy_(self._table_host, non_blocking=True)
@@ -255,8 +309,13 @@ class DewarpPipeline:
             if self.max_pixels is not None:
                 buf["table"] = torch.empty_like(self._table)
                 slot.update(table_host=torch.empty_like(self._table_host).pin_memory(), ev_table=torch.cuda.Event(), views=None)
+                if self.y512_from_photo:
+                    buf["prep"] = torch.empty_like(self._prep_table)
+                    slot.update(prep_host=torch.empty_like(self._prep_host).pin_memory(), ev_prep=torch.cuda.Event())
             elif self.out_size is not None:
                 buf["table"] = self._fixed_table(buf["photo_u8"], buf["out_u8"])
+            if self.y512_from_photo and self.max_pixels is None:
+                buf["prep"] = self._fixed_prep_table(buf["photo_u8"])
             self._slots.append(slot)
         self._submitted = 0
 
@@ -268,6 +327,8 @@ class DewarpPipeline:
         Mixed-size mode: h["photo_u8"] is a list of 1..docs uint8 HWC host photos and the other inputs have that many documents
         (x_T that many times n_batch); document slots past the list keep their earlier inputs, are sampled and not unwarped."""
         self._check_weights()
+        if self.y512_from_photo:
+            self._no_y512(h)
         if self.max_pixels is not None:
             return self._submit_host_mixed(h)
         with torch.cuda.device(self.dev):
@@ -280,15 +341,15 @@ class DewarpPipeline:
             with torch.cuda.stream(self._h2d):
                 if s["used"]:
                     self._h2d.wait_event(s["ev_done"])             # the kernels of batch ticket-2 have read this slot's inputs
-                for k in self.SAMPLING_KEYS:
+                for k in self._input_keys:
                     s["buf"][k].copy_(h[k], non_blocking=True)
                 s["ev_in"].record()
                 s["buf"]["photo_u8"].copy_(h["photo_u8"], non_blocking=True)
                 s["ev_photo"].record()
-            main.wait_event(s["ev_in"])
+            main.wait_event(s["ev_photo"] if self.y512_from_photo else s["ev_in"])      # y512 from the photo: sampling reads it
             if s["used"]:
                 main.wait_event(s["ev_out"])                       # the download of batch ticket-2 has read this slot's output
-            self._run("sampling", s["buf"], self.SAMPLING_KEYS, self._enqueue_sampling)
+            self._run("sampling", s["buf"], self._sampling_keys, self._sampling)
             main.wait_event(s["ev_photo"])
             self._run("unwarp", s["buf"], ("photo_u8", "out_u8"), self._enqueue_unwarp if self.out_size is None else self._enqueue_unwarp_sized)
             s["ev_done"].record(main)
@@ -303,7 +364,7 @@ class DewarpPipeline:
         photos = self._check_photos(h["photo_u8"], torch.device("cpu"), 1)
         out_shapes = self._out_shapes(photos)
         n = len(photos)
-        for k in self.SAMPLING_KEYS:
+        for k in self._input_keys:
             want = (n * self.n_batch if k == "x_T" else n,) + tuple(self.buf[k].shape[1:])
             if tuple(h[k].shape) != want:
                 raise ValueError(f"{k}: expected shape {want} for {n} photos, got {tuple(h[k].shape)}")
@@ -320,16 +381,25 @@ class DewarpPipeline:
             with torch.cuda.stream(self._h2d):
                 if s["used"]:
                     self._h2d.wait_event(s["ev_done"])             # the kernels of batch ticket-2 have read this slot's inputs
-                for k in self.SAMPLING_KEYS:
+                for k in self._input_keys:
                     buf[k][:h[k].shape[0]].copy_(h[k], non_blocking=True)
                 s["ev_in"].record()
                 for dst, src in zip(photo_dev, photos):
                     dst.copy_(src, non_blocking=True)
                 s["ev_photo"].record()
-            main.wait_event(s["ev_in"])
+            if self.y512_from_photo:
+                # documents past the batch keep their earlier y512, like their other inputs; the host rewrites the pinned table
+                # once the upload of ticket-2 has read it
+                s["ev_prep"].synchronize()
+                plan_y512(s["prep_host"], photo_dev)
+                buf["prep"].copy_(s["prep_host"], non_blocking=True)
+                s["ev_prep"].record(main)
+                main.wait_event(s["ev_photo"])
+            else:
+                main.wait_event(s["ev_in"])
             if s["used"]:
                 main.wait_event(s["ev_out"])                       # the download of batch ticket-2 has read this slot's output
-            self._run("sampling", buf, self.SAMPLING_KEYS, self._enqueue_sampling)
+            self._run("sampling", buf, self._sampling_keys, self._sampling)
             # the device only waits for batch ticket-2 through events; the HOST rewrites the pinned table now, so the upload of
             # ticket-2 must have read it (normally long done)
             s["ev_table"].synchronize()

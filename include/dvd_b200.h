@@ -167,6 +167,22 @@ DVD_API int dvd_unwarp_u8_sized_plan(const dvd_unwarp_sized_doc_t* docs_host, in
                                      void* table_host, size_t table_bytes, long long* total_tiles, int32_t* supersample_out);
 /* one launch; a table planned for another C is ignored (nothing is written) */
 DVD_API int dvd_unwarp_u8_sized(const void* table, int C, const float* map, void* stream);
+
+/* ---- input preparation: the denoiser's y512 [docs,3,512,512] from the uint8 HWC RGB photo (the reference loader's
+ * cv2.resize(photo, (512, 512), INTER_LINEAR) / 255, byte for byte: OpenCV's fixed-point bilinear resize, then an IEEE division
+ * by 255).  Photos of any sizes (at least 1x1) in ONE launch, with the table design of the mixed-size unwarp: dvd_y512_u8_plan
+ * fills the table in host memory (no CUDA call), the caller copies it to the device, dvd_y512_u8 launches; a CUDA graph captured
+ * once serves every batch planned into the same device table. */
+typedef struct dvd_y512_doc {
+  const uint8_t* photo;                 /* [H,W,3] uint8, device */
+  int32_t H, W;
+} dvd_y512_doc_t;
+/* bytes of a table for up to max_docs documents */
+DVD_API size_t dvd_y512_table_bytes(int max_docs);
+/* host only: validates (H, W >= 1, H*W*3 < 2^31, non-NULL photos, table_bytes large enough) and fills table_host */
+DVD_API int dvd_y512_u8_plan(const dvd_y512_doc_t* docs_host, int n_docs, void* table_host, size_t table_bytes);
+/* one launch; writes documents 0..n_docs-1 of y512 [>= n_docs,3,512,512] fp32 and nothing else */
+DVD_API int dvd_y512_u8(const void* table, float* y512, void* stream);
 /* WP:14-23,50-73 register_model2 / SpatialTransformer2: generic bilinear grid_sample,
  * align_corners=True, zeros padding.  img [B,C,H,W], grid [B,2,Ho,Wo] (ch0=x, ch1=y), out [B,C,Ho,Wo]. */
 DVD_API int dvd_grid_sample_f32(const float* img, const float* grid, float* out, int B, int C, int H, int W,
