@@ -131,3 +131,23 @@ def ptr(t):
 def stream_ptr():
     import torch
     return _vp(torch.cuda.current_stream().cuda_stream)
+
+
+class PlannedTable:
+    """The table of a launch that the host plans (dvd_*_plan) and the device reads: a pinned host block, its device copy and an
+    event.  upload() rewrites the pinned block only once the previous upload has read it, so one table serves batch after batch
+    (and keeps the device address that a captured graph reads)."""
+
+    def __init__(self, nbytes: int, device):
+        import torch
+        self.host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
+        self.dev = torch.empty(nbytes, dtype=torch.uint8, device=device)
+        self.event = torch.cuda.Event()
+
+    def upload(self, plan):
+        """plan(host) fills the pinned block, whose copy to the device is enqueued on the current stream; returns the device table."""
+        self.event.synchronize()
+        plan(self.host)
+        self.dev.copy_(self.host, non_blocking=True)
+        self.event.record()
+        return self.dev

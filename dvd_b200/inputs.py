@@ -69,11 +69,7 @@ def photo_to_y512(photo, out: torch.Tensor | None = None) -> torch.Tensor:
         out = torch.empty(shape, dtype=torch.float32, device=dev)
     elif out.dtype != torch.float32 or tuple(out.shape) != shape or not out.is_contiguous() or out.device != dev:
         raise ValueError(f"out must be a contiguous float32 tensor {shape} on {dev}, got {out.dtype} {tuple(out.shape)} on {out.device}")
-    nbytes = table_bytes(len(photos))
-    table_host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
-    plan_y512(table_host, photos)
     with torch.cuda.device(dev):
-        table = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        table.copy_(table_host, non_blocking=True)           # the pinned block is not reused before this copy has run
+        table = _lib.PlannedTable(table_bytes(len(photos)), dev).upload(lambda host: plan_y512(host, photos))
         launch_y512(table, out)
     return out

@@ -61,6 +61,15 @@ class DewarpPipeline:
         self.diffusion = create_gaussian_diffusion(steps=diffusion_steps, noise_schedule=noise_schedule, predict_xstart=True,
                                                    rescale_timesteps=True, rescale_learned_sigmas=True, timestep_respacing="")
         self.lib = _lib.lib()
+        # the unwarp: the batched fixed-size launch, or one launch over a table planned per batch (mixed size, out_size)
+        if out_size is not None:
+            self._plan_unwarp = lambda host, photos, outs: plan_sized(host, photos, outs, 64, 64, self.supersample)
+            self._unwarp_launch, self._unwarp_bytes = "dvd_unwarp_u8_sized", sized_table_bytes(docs)
+        elif max_pixels is not None:
+            self._plan_unwarp = lambda host, photos, outs: plan_mixed(host, photos, outs, 64, 64)
+            self._unwarp_launch, self._unwarp_bytes = "dvd_unwarp_u8_mixed", table_bytes(docs)
+        else:
+            self._plan_unwarp = None
         with torch.cuda.device(self.dev):
             self._bind_engine()
             z = lambda *s, dt=torch.float32: torch.zeros(s, dtype=dt, device=self.dev)
@@ -73,19 +82,7 @@ class DewarpPipeline:
             self.init_flow0 = z(docs, 2, 64, 64)                       # evaluation.py:180 (use_init_flow=False)
             self.map64 = z(docs, 2, 64, 64)
             self.out_u8 = z(*oimg, dt=torch.uint8)
-            self.out_host = torch.empty(oimg, dtype=torch.uint8).pin_memory()
-            if max_pixels is not None:                                # run_device's unwarp table (host plan -> device copy)
-                tb = table_bytes(docs) if out_size is None else sized_table_bytes(docs)
-                self._table = z(tb, dt=torch.uint8)
-                self._table_host = torch.empty(tb, dtype=torch.uint8).pin_memory()
-                self._ev_table = torch.cuda.Event()
-                if self.y512_from_photo:                              # run_device's y512 table, planned per batch
-                    self._prep_table = z(y512_table_bytes(docs), dt=torch.uint8)
-                    self._prep_host = torch.empty(y512_table_bytes(docs), dtype=torch.uint8).pin_memory()
-                    self._ev_prep = torch.cuda.Event()
-            # fixed-size mode, planned once per buffer: (photo, out) pointers -> sized unwarp table (with out_size), ("prep", photo)
-            # -> y512 table (with y512_from_photo)
-            self._fixed_tables = {}
+            self._device_tables = self._planned_tables()              # run_device's
         self.h2d_bytes = sum(v.numel() * v.element_size() for k, v in self.buf.items() if k in self._input_keys + ("photo_u8",))
         self.d2h_bytes = self.out_u8.numel()
         self.use_graph = os.environ.get("DVD_NO_GRAPH", "0") != "1"
@@ -108,6 +105,15 @@ class DewarpPipeline:
             with torch.cuda.device(self.dev):
                 self._bind_engine()
 
+    def _planned_tables(self) -> dict:
+        """the host-planned launch tables of one batch in flight: "unwarp" (mixed size or out_size) and "prep" (y512_from_photo)"""
+        tables = {}
+        if self._plan_unwarp is not None:
+            tables["unwarp"] = _lib.PlannedTable(self._unwarp_bytes, self.dev)
+        if self.y512_from_photo:
+            tables["prep"] = _lib.PlannedTable(y512_table_bytes(self.docs), self.dev)
+        return tables
+
     # ---- device-resident inputs: dict with y512, mask_cat, mask_y512, line_msk, x_T, photo_u8 (all on self.dev)
     def _enqueue_sampling(self, d: dict):
         """static conditioning -> S-step DDIM loop -> hypothesis mean (map64), on the current stream."""
@@ -120,80 +126,77 @@ class DewarpPipeline:
         self._enqueue_sampling(d)
 
     def _enqueue_unwarp(self, d: dict):
-        """fused upsample + affine + bilinear unwarp of the full-resolution photo, on the current stream."""
-        out = d.get("out_u8", self.out_u8)
-        _lib.check(self.lib.dvd_unwarp_u8(_lib.ptr(d["photo_u8"]), _lib.ptr(self.map64), _lib.ptr(out), self.docs, 3,
+        """fused upsample + affine + bilinear unwarp of the full-resolution photos d["photo_u8"] into d["out_u8"], on the current
+        stream."""
+        _lib.check(self.lib.dvd_unwarp_u8(_lib.ptr(d["photo_u8"]), _lib.ptr(self.map64), _lib.ptr(d["out_u8"]), self.docs, 3,
                                           self.H, self.W, 64, 64, AFFINE, _lib.stream_ptr()), "dvd_unwarp_u8")
 
-    def _enqueue_unwarp_mixed(self, d: dict):
-        """mixed-size unwarp of the batch planned into the device table d["table"] (one launch whatever the composition)."""
-        _lib.check(self.lib.dvd_unwarp_u8_mixed(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), "dvd_unwarp_u8_mixed")
+    def _enqueue_unwarp_table(self, d: dict):
+        """mixed-size or sized unwarp of the batch planned into the device table d["table"] (one launch whatever the composition)."""
+        fn = self._unwarp_launch
+        _lib.check(getattr(self.lib, fn)(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), fn)
 
-    def _enqueue_unwarp_sized(self, d: dict):
-        """sized unwarp of the batch planned into the device table d["table"] (one launch whatever the composition)."""
-        _lib.check(self.lib.dvd_unwarp_u8_sized(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), "dvd_unwarp_u8_sized")
+    def _sample(self, d: dict, photos, tables: dict):
+        """the sampling graph on the current stream; with y512_from_photo its first launch reads a y512 table planned from `photos`"""
+        if self.y512_from_photo:
+            d = dict(d, prep=tables["prep"].upload(lambda host: plan_y512(host, photos)))
+        self._run("sampling", d, self._sampling_keys, self._sampling)
 
-    def _check_fixed_photo(self, photo: torch.Tensor):
-        if photo.dtype != torch.uint8 or tuple(photo.shape) != (self.docs, self.H, self.W, 3) or not photo.is_contiguous():
-            raise ValueError(f"photo_u8: expected a contiguous uint8 tensor {(self.docs, self.H, self.W, 3)}, got "
-                             f"{photo.dtype} {tuple(photo.shape)}")
-
-    def _fixed_prep_table(self, photo: torch.Tensor) -> torch.Tensor:
-        """device table of the y512 launch of photo [docs,H,W,3], planned and uploaded once per buffer (kept alive like the sized
-        unwarp tables)"""
-        key = ("prep", photo.data_ptr())
-        if key not in self._fixed_tables:
-            nb = y512_table_bytes(self.docs)
-            host = torch.empty(nb, dtype=torch.uint8).pin_memory()
-            plan_y512(host, list(photo.unbind(0)))
-            table = torch.empty(nb, dtype=torch.uint8, device=self.dev)
-            table.copy_(host, non_blocking=True)
-            if len(self._fixed_tables) >= 16:
-                self._fixed_tables.pop(next(iter(self._fixed_tables)))
-            self._fixed_tables[key] = (table, host)
-        return self._fixed_tables[key][0]
-
-    def _no_y512(self, d: dict):
-        if "y512" in d:
-            raise ValueError("this pipeline computes y512 from photo_u8 (y512_from_photo=True); do not pass y512")
+    def _unwarp(self, photos, outs, tables: dict):
+        """the unwarp graph on the current stream: photos -> outs with the rows of map64"""
+        if self._plan_unwarp is None:
+            self._run("unwarp", {"photo_u8": photos, "out_u8": outs}, ("photo_u8", "out_u8"), self._enqueue_unwarp)
+        else:
+            table = tables["unwarp"].upload(lambda host: self._plan_unwarp(host, photos, outs))
+            self._run("unwarp", {"table": table}, ("table",), self._enqueue_unwarp_table)
 
     def _out_hw(self, H: int, W: int) -> tuple:
         """output size of an H x W photo"""
         return size_arg(self.out_size(H, W) if callable(self.out_size) else self.out_size, f"out_size for a {H}x{W} photo")
 
-    def _fixed_table(self, photo: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
-        """device table of the sized launch photo [docs,H,W,3] -> out [docs,Ho,Wo,3], planned and uploaded once per buffer pair
-        (a graph captured with it keeps it alive through its input dict)"""
-        key = (photo.data_ptr(), out.data_ptr())
-        if key not in self._fixed_tables:
-            nb = sized_table_bytes(self.docs)
-            host = torch.empty(nb, dtype=torch.uint8).pin_memory()
-            plan_sized(host, list(photo.unbind(0)), list(out.unbind(0)), 64, 64, self.supersample)
-            table = torch.empty(nb, dtype=torch.uint8, device=self.dev)
-            table.copy_(host, non_blocking=True)
-            if len(self._fixed_tables) >= 16:
-                self._fixed_tables.pop(next(iter(self._fixed_tables)))
-            self._fixed_tables[key] = (table, host)                  # the pinned block stays alive until its upload has run
-        return self._fixed_tables[key][0]
+    def _place(self, buf: torch.Tensor, docs):
+        """a batch in `buf`: fixed-size mode, the [docs,...] buffer itself; mixed-size mode, one view per document (a tensor or a
+        shape) packed into the arena `buf`"""
+        return buf if self.max_pixels is None else self._arena_views(buf, docs)
 
-    def _out_shapes(self, photos) -> list:
-        """output shapes of a mixed-size batch: the photos' own, or their out_size shapes (at most max_out_pixels in all)"""
-        if self.out_size is None:
-            return [tuple(p.shape) for p in photos]
+    def _outputs(self, buf: torch.Tensor, photos):
+        """where the pages of a batch go in `buf`; in mixed-size mode with out_size, their shapes hold at most max_out_pixels"""
+        if self.max_pixels is None or self.out_size is None:
+            return self._place(buf, photos)
         shapes = [self._out_hw(p.shape[0], p.shape[1]) + (3,) for p in photos]
         px = sum(Ho * Wo for Ho, Wo, _ in shapes)
         if px > self.max_out_pixels:
             raise ValueError(f"the batch's outputs have {px} pixels, more than max_out_pixels={self.max_out_pixels}")
-        return shapes
+        return self._arena_views(buf, shapes)
 
-    def _plan_batch(self, table_host: torch.Tensor, photos, outs):
-        if self.out_size is None:
-            plan_mixed(table_host, photos, outs, 64, 64)
-        else:
-            plan_sized(table_host, photos, outs, 64, 64, self.supersample)
+    def _check_inputs(self, d: dict, on_device: bool):
+        """Validates the inputs of one batch and returns its photos.  A host dict carries 1..docs photos (fixed-size mode: docs) on
+        the CPU, a device dict exactly docs photos and contiguous fp32 sampling inputs on the pipeline's device; the other inputs
+        have one row per photo (x_T n_batch rows)."""
+        if self.y512_from_photo and "y512" in d:
+            raise ValueError("this pipeline computes y512 from photo_u8 (y512_from_photo=True); do not pass y512")
+        photos = self._check_photos(d["photo_u8"], self.dev if on_device else torch.device("cpu"), self.docs if on_device else 1)
+        n = len(photos)
+        for k in self._input_keys:
+            t = d[k]
+            want = (n * self.n_batch if k == "x_T" else n,) + tuple(self.buf[k].shape[1:])
+            if tuple(t.shape) != want:
+                raise ValueError(f"{k}: expected shape {want} for {n} photos, got {tuple(t.shape)}")
+            if on_device and (t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.dev):
+                raise ValueError(f"{k}: expected a contiguous float32 tensor on {self.dev}, got {t.dtype} on {t.device}")
+        return photos
 
-    def _check_photos(self, photos, device: torch.device, lo: int) -> list:
-        """Validates the photos of a mixed-size batch (lo..docs uint8 HWC RGB tensors on `device`, at most max_pixels in all)."""
+    def _check_photos(self, photos, device: torch.device, lo: int):
+        """Validates the photos of a batch on `device`: fixed-size mode, one contiguous uint8 tensor [docs,H,W,3]; mixed-size mode,
+        lo..docs uint8 HWC RGB tensors with at most max_pixels in all (returned as a list)."""
+        if self.max_pixels is None:
+            want = (self.docs, self.H, self.W, 3)
+            if (not isinstance(photos, torch.Tensor) or photos.dtype != torch.uint8 or tuple(photos.shape) != want
+                    or not photos.is_contiguous() or photos.device != device):
+                raise ValueError(f"photo_u8: expected a contiguous uint8 tensor {want} on {device}, got "
+                                 f"{getattr(photos, 'dtype', type(photos))} {tuple(getattr(photos, 'shape', ()))} "
+                                 f"on {getattr(photos, 'device', None)}")
+            return photos
         if not isinstance(photos, (list, tuple)):
             raise ValueError("mixed-size mode (max_pixels) takes photo_u8 as a list of uint8 HWC tensors")
         if not lo <= len(photos) <= self.docs:
@@ -252,71 +255,35 @@ class DewarpPipeline:
 
     def run_device(self, d: dict):
         """The ~230 kernel launches of one batch are captured once per set of input buffers into two CUDA graphs (sampling,
-        unwarp) and replayed (the library never allocates or synchronises, so every entry point is capturable).
+        unwarp) and replayed (the library never allocates or synchronises, so every entry point is capturable).  Returns the
+        device output, overwritten by the next call.
 
         Mixed-size mode: d["photo_u8"] is a list of exactly `docs` uint8 HWC photos on the pipeline's device (read in place);
-        returns a list of views into the device output arena, overwritten by the next call."""
+        returns a list of views into the device output arena."""
         self._check_weights()
-        if self.max_pixels is not None:
-            return self._run_device_mixed(d)
+        photos = self._check_inputs(d, on_device=True)
         with torch.cuda.device(self.dev):
+            outs = self._outputs(self.out_u8, photos)
             if self.y512_from_photo:
-                self._no_y512(d)
-                self._check_fixed_photo(d["photo_u8"])
-                d = dict(d, y512=self.buf["y512"], prep=self._fixed_prep_table(d["photo_u8"]))
-            self._run("sampling", d, self._sampling_keys, self._sampling)
-            if self.out_size is None:
-                self._run("unwarp", d, ("photo_u8",), self._enqueue_unwarp)
-            else:
-                photo = d["photo_u8"]
-                self._check_fixed_photo(photo)
-                du = {"photo_u8": photo, "table": self._fixed_table(photo, self.out_u8)}
-                self._run("unwarp", du, ("photo_u8", "table"), self._enqueue_unwarp_sized)
-        return self.out_u8
-
-    def _run_device_mixed(self, d: dict) -> list:
-        photos = self._check_photos(d["photo_u8"], self.dev, self.docs)
-        outs = self._arena_views(self.out_u8, self._out_shapes(photos))
-        with torch.cuda.device(self.dev):
-            if self.y512_from_photo:
-                self._no_y512(d)
-                self._ev_prep.synchronize()                            # the previous upload has read the pinned table
-                plan_y512(self._prep_host, photos)
-                self._prep_table.copy_(self._prep_host, non_blocking=True)
-                self._ev_prep.record()
-                d = dict(d, y512=self.buf["y512"], prep=self._prep_table)
-            self._run("sampling", d, self._sampling_keys, self._sampling)
-            self._ev_table.synchronize()                               # the previous upload has read the pinned table
-            self._plan_batch(self._table_host, photos, outs)
-            self._table.copy_(self._table_host, non_blocking=True)
-            self._ev_table.record()
-            self._run("unwarp", {"table": self._table}, ("table",),
-                      self._enqueue_unwarp_mixed if self.out_size is None else self._enqueue_unwarp_sized)
+                d = dict(d, y512=self.buf["y512"])
+            self._sample(d, photos, self._device_tables)
+            self._unwarp(photos, outs, self._device_tables)
         return outs
 
     # ---- pinned-host inputs -> host uint8 image (H2D and D2H inside the call)
     def _make_slots(self):
-        """Two sets of device input / output buffers + copy streams: the uploads of batch i+1 and the download of batch i run
-        underneath the kernels of the batch in between (the kernels themselves stay on the caller's stream, one batch at a time)."""
+        """Two sets of device input / output buffers, planned tables + copy streams: the uploads of batch i+1 and the download of
+        batch i run underneath the kernels of the batch in between (the kernels themselves stay on the caller's stream, one batch
+        at a time)."""
         self._h2d = torch.cuda.Stream(device=self.dev)
         self._d2h = torch.cuda.Stream(device=self.dev)
         self._slots = []
         for _ in range(2):
             buf = {k: torch.empty_like(v) for k, v in self.buf.items()}
             buf["out_u8"] = torch.empty_like(self.out_u8)
-            slot = {"buf": buf, "out_host": torch.empty_like(self.out_host).pin_memory(), "used": False,
-                    "ev_in": torch.cuda.Event(), "ev_photo": torch.cuda.Event(), "ev_done": torch.cuda.Event(), "ev_out": torch.cuda.Event()}
-            if self.max_pixels is not None:
-                buf["table"] = torch.empty_like(self._table)
-                slot.update(table_host=torch.empty_like(self._table_host).pin_memory(), ev_table=torch.cuda.Event(), views=None)
-                if self.y512_from_photo:
-                    buf["prep"] = torch.empty_like(self._prep_table)
-                    slot.update(prep_host=torch.empty_like(self._prep_host).pin_memory(), ev_prep=torch.cuda.Event())
-            elif self.out_size is not None:
-                buf["table"] = self._fixed_table(buf["photo_u8"], buf["out_u8"])
-            if self.y512_from_photo and self.max_pixels is None:
-                buf["prep"] = self._fixed_prep_table(buf["photo_u8"])
-            self._slots.append(slot)
+            self._slots.append({"buf": buf, "out_host": torch.empty(self.out_u8.shape, dtype=torch.uint8, pin_memory=True),
+                                "tables": self._planned_tables(), "result": None, "used": False, "ev_in": torch.cuda.Event(),
+                                "ev_photo": torch.cuda.Event(), "ev_done": torch.cuda.Event(), "ev_out": torch.cuda.Event()})
         self._submitted = 0
 
     def submit_host(self, h: dict) -> int:
@@ -327,94 +294,41 @@ class DewarpPipeline:
         Mixed-size mode: h["photo_u8"] is a list of 1..docs uint8 HWC host photos and the other inputs have that many documents
         (x_T that many times n_batch); document slots past the list keep their earlier inputs, are sampled and not unwarped."""
         self._check_weights()
-        if self.y512_from_photo:
-            self._no_y512(h)
-        if self.max_pixels is not None:
-            return self._submit_host_mixed(h)
+        photos = self._check_inputs(h, on_device=False)
         with torch.cuda.device(self.dev):
             if self._slots is None:
                 self._make_slots()
             main = torch.cuda.current_stream()
             ticket = self._submitted
-            self._submitted += 1
-            s = self._slots[ticket % 2]
-            with torch.cuda.stream(self._h2d):
-                if s["used"]:
-                    self._h2d.wait_event(s["ev_done"])             # the kernels of batch ticket-2 have read this slot's inputs
-                for k in self._input_keys:
-                    s["buf"][k].copy_(h[k], non_blocking=True)
-                s["ev_in"].record()
-                s["buf"]["photo_u8"].copy_(h["photo_u8"], non_blocking=True)
-                s["ev_photo"].record()
-            main.wait_event(s["ev_photo"] if self.y512_from_photo else s["ev_in"])      # y512 from the photo: sampling reads it
-            if s["used"]:
-                main.wait_event(s["ev_out"])                       # the download of batch ticket-2 has read this slot's output
-            self._run("sampling", s["buf"], self._sampling_keys, self._sampling)
-            main.wait_event(s["ev_photo"])
-            self._run("unwarp", s["buf"], ("photo_u8", "out_u8"), self._enqueue_unwarp if self.out_size is None else self._enqueue_unwarp_sized)
-            s["ev_done"].record(main)
-            with torch.cuda.stream(self._d2h):
-                self._d2h.wait_event(s["ev_done"])
-                s["out_host"].copy_(s["buf"]["out_u8"], non_blocking=True)
-                s["ev_out"].record()
-            s["used"] = True
-        return ticket
-
-    def _submit_host_mixed(self, h: dict) -> int:
-        photos = self._check_photos(h["photo_u8"], torch.device("cpu"), 1)
-        out_shapes = self._out_shapes(photos)
-        n = len(photos)
-        for k in self._input_keys:
-            want = (n * self.n_batch if k == "x_T" else n,) + tuple(self.buf[k].shape[1:])
-            if tuple(h[k].shape) != want:
-                raise ValueError(f"{k}: expected shape {want} for {n} photos, got {tuple(h[k].shape)}")
-        with torch.cuda.device(self.dev):
-            if self._slots is None:
-                self._make_slots()
-            main = torch.cuda.current_stream()
-            ticket = self._submitted
-            self._submitted += 1
             s = self._slots[ticket % 2]
             buf = s["buf"]
-            photo_dev = self._arena_views(buf["photo_u8"], photos)
-            out_dev = self._arena_views(buf["out_u8"], out_shapes)
+            photo_dev, out_dev = self._place(buf["photo_u8"], photos), self._outputs(buf["out_u8"], photos)
+            self._submitted += 1
             with torch.cuda.stream(self._h2d):
                 if s["used"]:
                     self._h2d.wait_event(s["ev_done"])             # the kernels of batch ticket-2 have read this slot's inputs
                 for k in self._input_keys:
                     buf[k][:h[k].shape[0]].copy_(h[k], non_blocking=True)
                 s["ev_in"].record()
-                for dst, src in zip(photo_dev, photos):
-                    dst.copy_(src, non_blocking=True)
+                if self.max_pixels is None:
+                    photo_dev.copy_(photos, non_blocking=True)
+                else:
+                    for dst, src in zip(photo_dev, photos):
+                        dst.copy_(src, non_blocking=True)
                 s["ev_photo"].record()
-            if self.y512_from_photo:
-                # documents past the batch keep their earlier y512, like their other inputs; the host rewrites the pinned table
-                # once the upload of ticket-2 has read it
-                s["ev_prep"].synchronize()
-                plan_y512(s["prep_host"], photo_dev)
-                buf["prep"].copy_(s["prep_host"], non_blocking=True)
-                s["ev_prep"].record(main)
-                main.wait_event(s["ev_photo"])
-            else:
-                main.wait_event(s["ev_in"])
+            main.wait_event(s["ev_photo"] if self.y512_from_photo else s["ev_in"])      # y512 from the photo: sampling reads it
             if s["used"]:
                 main.wait_event(s["ev_out"])                       # the download of batch ticket-2 has read this slot's output
-            self._run("sampling", buf, self._sampling_keys, self._sampling)
-            # the device only waits for batch ticket-2 through events; the HOST rewrites the pinned table now, so the upload of
-            # ticket-2 must have read it (normally long done)
-            s["ev_table"].synchronize()
-            self._plan_batch(s["table_host"], photo_dev, out_dev)
-            buf["table"].copy_(s["table_host"], non_blocking=True)
-            s["ev_table"].record(main)
+            self._sample(buf, photo_dev, s["tables"])
             main.wait_event(s["ev_photo"])
-            self._run("unwarp", buf, ("table",), self._enqueue_unwarp_mixed if self.out_size is None else self._enqueue_unwarp_sized)
+            self._unwarp(photo_dev, out_dev, s["tables"])
             s["ev_done"].record(main)
-            end = out_dev[-1].data_ptr() - buf["out_u8"].data_ptr() + out_dev[-1].numel()
+            end = out_dev[-1].data_ptr() - buf["out_u8"].data_ptr() + out_dev[-1].numel()       # through the batch's last page
             with torch.cuda.stream(self._d2h):
                 self._d2h.wait_event(s["ev_done"])
-                s["out_host"][:end].copy_(buf["out_u8"][:end], non_blocking=True)
+                s["out_host"].view(-1)[:end].copy_(buf["out_u8"].view(-1)[:end], non_blocking=True)
                 s["ev_out"].record()
-            s["views"] = self._arena_views(s["out_host"], out_dev)
+            s["result"] = self._place(s["out_host"], out_dev)
             s["used"] = True
         return ticket
 
@@ -423,7 +337,7 @@ class DewarpPipeline:
         pinned arena) is reused by the second-next submit."""
         s = self._slots[ticket % 2]
         s["ev_out"].synchronize()
-        return s["out_host"] if self.max_pixels is None else s["views"]
+        return s["result"]
 
     def run_host(self, h: dict):
         """Synchronous form: host inputs in, host uint8 image(s) out."""

@@ -109,17 +109,19 @@ def size_arg(size, what: str = "size") -> tuple:
     return int(size[0]), int(size[1])
 
 
-def _dewarp_sized(map64: torch.Tensor, photos, outs, supersample: int, affine: float):
-    """one sized launch: photos[i] -> outs[i] with map row i"""
+def _dewarp_planned(map64: torch.Tensor, photos, outs, sized: bool, supersample: int, affine: float):
+    """one launch over a planned table: photos[i] -> outs[i] with map row i; the sized launch when `sized`, else the mixed-size one"""
     if not photos:
         return
-    Cc = photos[0].shape[2]
-    nbytes = sized_table_bytes(len(photos))
-    table_host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
-    plan_sized(table_host, photos, outs, map64.shape[2], map64.shape[3], supersample, affine, Cc)
-    table = torch.empty(nbytes, dtype=torch.uint8, device=map64.device)
-    table.copy_(table_host, non_blocking=True)                 # the pinned block is not reused before this copy has run
-    _lib.check(_lib.lib().dvd_unwarp_u8_sized(_lib.ptr(table), Cc, _lib.ptr(map64), _lib.stream_ptr()), "dvd_unwarp_u8_sized")
+    Cc, mh, mw = photos[0].shape[2], map64.shape[2], map64.shape[3]
+    if sized:
+        nbytes, launch = sized_table_bytes(len(photos)), "dvd_unwarp_u8_sized"
+        plan = lambda host: plan_sized(host, photos, outs, mh, mw, supersample, affine, Cc)
+    else:
+        nbytes, launch = table_bytes(len(photos)), "dvd_unwarp_u8_mixed"
+        plan = lambda host: plan_mixed(host, photos, outs, mh, mw, affine, Cc)
+    table = _lib.PlannedTable(nbytes, map64.device).upload(plan)
+    _lib.check(getattr(_lib.lib(), launch)(_lib.ptr(table), Cc, _lib.ptr(map64), _lib.stream_ptr()), launch)
 
 
 def _dewarp_mixed(map64: torch.Tensor, photos, affine: float, size=None, supersample: int = 0) -> list:
@@ -132,25 +134,16 @@ def _dewarp_mixed(map64: torch.Tensor, photos, affine: float, size=None, supersa
                              f"{p.dtype} {tuple(p.shape)} on {p.device}")
         if p.shape[2] != photos[0].shape[2]:
             raise ValueError(f"photo {i} has {p.shape[2]} channels, photo 0 has {photos[0].shape[2]}")
-    if size is not None:
+    if size is None:
+        outs = [torch.empty_like(p) for p in photos]
+    else:
         per_photo = isinstance(size, list) and (not size or isinstance(size[0], (tuple, list)))
         sizes = list(size) if per_photo else [size] * len(photos)
         if len(sizes) != len(photos):
             raise ValueError(f"size: {len(sizes)} sizes for {len(photos)} photos")
         sizes = [size_arg(s, f"size of photo {i}") for i, s in enumerate(sizes)]
         outs = [torch.empty((Ho, Wo, p.shape[2]), dtype=torch.uint8, device=p.device) for p, (Ho, Wo) in zip(photos, sizes)]
-        _dewarp_sized(map64, photos, outs, supersample, affine)
-        return outs
-    if not photos:
-        return []
-    Cc = photos[0].shape[2]
-    outs = [torch.empty_like(p) for p in photos]
-    nbytes = table_bytes(len(photos))
-    table_host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
-    plan_mixed(table_host, photos, outs, map64.shape[2], map64.shape[3], affine, Cc)
-    table = torch.empty(nbytes, dtype=torch.uint8, device=map64.device)
-    table.copy_(table_host, non_blocking=True)                 # the pinned block is not reused before this copy has run
-    _lib.check(_lib.lib().dvd_unwarp_u8_mixed(_lib.ptr(table), Cc, _lib.ptr(map64), _lib.stream_ptr()), "dvd_unwarp_u8_mixed")
+    _dewarp_planned(map64, photos, outs, size is not None, supersample, affine)
     return outs
 
 
@@ -193,7 +186,7 @@ def dewarp_fullres(map64: torch.Tensor, photo, out: torch.Tensor | None = None, 
             raise ValueError(f"out must be a contiguous uint8 tensor {(B, Ho, Wo, Cc)} on {photo.device}, got {out.dtype} "
                              f"{tuple(out.shape)}")
         with torch.cuda.device(photo.device):
-            _dewarp_sized(map64, list(photo.unbind(0)), list(out.unbind(0)), ss, affine)
+            _dewarp_planned(map64, list(photo.unbind(0)), list(out.unbind(0)), True, ss, affine)
         return out
     map64 = map64.float().contiguous()
     l = _lib.lib()

@@ -256,6 +256,16 @@ def test_pipeline_fixed_size(dev, model, out_size):
     d["photo_u8"] = d["photo_u8"].float()
     with pytest.raises(ValueError):
         pipe.run_device(d)
+    # the pipeline that takes y512 checks its inputs as well: a photo of the wrong size, a misshapen x_T and a one-document input
+    # that would broadcast to both documents
+    d = _device(_host(batches[0], True), dev)
+    for k, bad in (("photo_u8", d["photo_u8"][:, 1:].contiguous()), ("x_T", d["x_T"][:2]), ("x_T", d["x_T"].double())):
+        with pytest.raises(ValueError):
+            ref.run_device(dict(d, **{k: bad}))
+    h = _host(batches[0], True)
+    for k in ("photo_u8", "mask_cat"):
+        with pytest.raises(ValueError):
+            ref.submit_host(dict(h, **{k: h[k][:1]}))
 
 
 @pytest.mark.gpu
