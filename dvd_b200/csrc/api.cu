@@ -144,6 +144,20 @@ extern "C" int dvd_test_attention(const float* q, const float* k, const float* v
   return pair_to_f32(o16, x3 ? olo : nullptr, o, n, st);
 }
 
+// The tensor-core attention on caller-prepared 16-bit operands, exactly the launch dvd_denoise_step makes (no conversion, no
+// transpose): one context goes through attention_tc (which picks the kernel), two to four through one attention_tc_multi launch.
+extern "C" int dvd_test_attention_tc(const void* q, int ldq, const void* const* k, int ldk, const void* const* vt, void* const* o,
+                                     void* const* o_lo, int ldo, const int* kv_div, int nctx, int nsamp, int heads, int T, int d,
+                                     float scale, int f16, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  DVD_REQUIRE(nctx >= 1 && nctx <= 4, "test_attention_tc: nctx must be 1..4 (got %d)", nctx);
+  DVD_REQUIRE(k && vt && o && kv_div, "test_attention_tc: null context array");
+  __nv_bfloat16* const* oo = reinterpret_cast<__nv_bfloat16* const*>(o);
+  __nv_bfloat16* const* ol = reinterpret_cast<__nv_bfloat16* const*>(o_lo);
+  if (nctx == 1) return attention_tc(q, ldq, k[0], ldk, vt[0], oo[0], ol ? ol[0] : nullptr, ldo, nsamp, heads, T, d, scale, kv_div[0], f16, st);
+  return attention_tc_multi(q, ldq, k, ldk, vt, oo, ol, ldo, kv_div, nctx, nsamp, heads, T, d, scale, f16, st);
+}
+
 // The decoder's depthwise 3x3 + folded BN + ReLU of the tensor modes on its own: [N,1024,C] bf16 (in_lo non-NULL: bf16 pairs) in and
 // out, the same launch dvd_denoise_step makes.
 extern "C" int dvd_test_dwconv(const void* in_hi, const void* in_lo, const float* w9, const float* scale, const float* shift, void* out_hi,

@@ -322,9 +322,13 @@ static int launch_attention_pair(const CUtensorMap& tmQ, const CUtensorMap& tmK,
 
 int attention_pair(const void* q, int ldq, const void* k, int ldk, const void* vt, __nv_bfloat16* o, __nv_bfloat16* o_lo, int ldo, int nsamp,
                    int heads, int T, float scale, int kv_div, int f16, cudaStream_t st) {
-  DVD_REQUIRE(q && k && vt && o && kv_div > 0 && nsamp % kv_div == 0 && nsamp <= 65535, "attention_pair: bad arguments");
-  DVD_REQUIRE(T % (2 * PQ) == 0 && ldo % 8 == 0 && (reinterpret_cast<uintptr_t>(o) & 15) == 0 && (reinterpret_cast<uintptr_t>(o_lo) & 15) == 0,
-              "attention_pair: bad shape / alignment");
+  DVD_REQUIRE(q && k && vt && o, "attention_pair: null pointer");
+  DVD_REQUIRE(nsamp > 0 && nsamp <= 65535, "attention_pair: nsamp %d outside 1..65535", nsamp);
+  DVD_REQUIRE(kv_div > 0 && nsamp % kv_div == 0, "attention_pair: nsamp %d is not a multiple of kv_div %d", nsamp, kv_div);
+  DVD_REQUIRE(T % (2 * PQ) == 0, "attention_pair: T %d is not a multiple of %d", T, 2 * PQ);
+  DVD_REQUIRE(ldo % 8 == 0, "attention_pair: ldo %d is not a multiple of 8", ldo);
+  DVD_REQUIRE((reinterpret_cast<uintptr_t>(o) & 15) == 0, "attention_pair: o must be 16-byte aligned");
+  DVD_REQUIRE((reinterpret_cast<uintptr_t>(o_lo) & 15) == 0, "attention_pair: o_lo must be 16-byte aligned");
   const int nkv = nsamp / kv_div;
   CUtensorMap tmQ, tmK, tmVt;
   int rc = make_tmap_bf16_2d(&tmQ, q, (uint64_t)nsamp * T, (uint64_t)heads * PD, (uint64_t)ldq, PQ, 64); if (rc) return rc;

@@ -302,21 +302,26 @@ int attention_tc_multi(const void* q, int ldq, const void* const* k, int ldk, co
                        int f16, cudaStream_t st) {
   DVD_REQUIRE(q && k && vt && o && kv_div && nctx >= 1 && nctx <= ACTX, "attention_tc_multi: bad arguments");
   DVD_REQUIRE((d == 64 || d == 256) && T % 128 == 0 && nsamp > 0, "attention_tc: bad shape d=%d T=%d", d, T);
-  DVD_REQUIRE(ldo % 8 == 0 && (long long)nsamp * nctx <= 65535, "attention_tc: bad ldo / batch");
+  DVD_REQUIRE(ldo % 8 == 0, "attention_tc: ldo %d is not a multiple of 8", ldo);
+  DVD_REQUIRE((long long)nsamp * nctx <= 65535, "attention_tc: nsamp %d x nctx %d exceeds 65535 grid slices", nsamp, nctx);
+  // every argument is checked before the first tensor map is encoded (a driver call)
+  for (int i = 0; i < nctx; ++i) {
+    DVD_REQUIRE(k[i] && vt[i] && o[i], "attention_tc: context %d: null pointer", i);
+    DVD_REQUIRE(kv_div[i] > 0 && nsamp % kv_div[i] == 0, "attention_tc: context %d: nsamp %d is not a multiple of kv_div %d", i, nsamp, kv_div[i]);
+    DVD_REQUIRE((reinterpret_cast<uintptr_t>(o[i]) & 15) == 0, "attention_tc: context %d: o must be 16-byte aligned", i);
+    DVD_REQUIRE(!o_lo || (reinterpret_cast<uintptr_t>(o_lo[i]) & 15) == 0, "attention_tc: context %d: o_lo must be 16-byte aligned", i);
+  }
   CUtensorMap tmQ;
   AttnCtx cx;
   memset(&cx, 0, sizeof(cx));
   // (fp16 and bf16 tiles are both plain 16-bit elements for TMA)
   int rc = make_tmap_bf16_2d(&tmQ, q, (uint64_t)nsamp * T, (uint64_t)heads * d, (uint64_t)ldq, AQ, 64); if (rc) return rc;
   for (int i = 0; i < nctx; ++i) {
-    DVD_REQUIRE(k[i] && vt[i] && o[i] && kv_div[i] > 0 && nsamp % kv_div[i] == 0 && (reinterpret_cast<uintptr_t>(o[i]) & 15) == 0,
-                "attention_tc: bad context %d", i);
     const int nkv = nsamp / kv_div[i];
     rc = make_tmap_bf16_2d(&cx.tmK[i], k[i], (uint64_t)nkv * T, (uint64_t)heads * d, (uint64_t)ldk, AKV, 64); if (rc) return rc;
     rc = make_tmap_bf16_2d(&cx.tmVt[i], vt[i], (uint64_t)nkv * heads * d, (uint64_t)T, (uint64_t)T, d, 64); if (rc) return rc;
     cx.out[i] = o[i]; cx.kv_div[i] = kv_div[i];
     cx.out_lo[i] = o_lo ? o_lo[i] : nullptr;
-    DVD_REQUIRE((reinterpret_cast<uintptr_t>(cx.out_lo[i]) & 15) == 0, "attention_tc: o_lo must be 16-byte aligned");
   }
   if (d == 64) return f16 ? launch_attention_t<64, true>(tmQ, cx, nctx, ldo, nsamp, heads, T, scale, st)
                           : launch_attention_t<64, false>(tmQ, cx, nctx, ldo, nsamp, heads, T, scale, st);

@@ -252,6 +252,14 @@ DVD_API int dvd_test_gemm(const float* A, const float* W, const float* bias, flo
 DVD_API int dvd_test_attention(const float* q, const float* k, const float* v, float* o, int batch, int heads,
                        int T, int d, float scale, int precision, void* scratch, size_t scratch_bytes,
                        void* stream);
+/* Tensor-core attention on caller-prepared 16-bit operands, exactly the launch dvd_denoise_step makes:
+ * q [nsamp*T, ldq]; context i: k[i] [nsamp/kv_div[i]*T, ldk], vt[i] = V^T [nsamp/kv_div[i], heads*d, T], o[i] (+ o_lo[i]) [nsamp*T, ldo].
+ * nctx == 1: the kernel attention_tc selects (the CTA pair for d = 256 unless DVD_ATTN_V1=1); nctx 2..4: one multi-context launch.
+ * f16: IEEE fp16 operands (DVD_PREC_BF16X3), else bf16.  k, vt, o, o_lo (may be NULL) and kv_div are HOST arrays of nctx entries.
+ * Every argument is checked before any CUDA call. */
+DVD_API int dvd_test_attention_tc(const void* q, int ldq, const void* const* k, int ldk, const void* const* vt, void* const* o,
+                                  void* const* o_lo, int ldo, const int* kv_div, int nctx, int nsamp, int heads, int T, int d,
+                                  float scale, int f16, void* stream);
 /* Depthwise 3x3 (pad 1) over the 32x32 token grid + folded BN + ReLU as the decoder runs it in the tensor modes: in_hi / in_lo
  * [N,1024,C] bf16 (value = hi + lo; in_lo NULL: hi alone), w9 [9,C] fp32 (tap ky*3+kx), scale / shift [C] fp32, out_hi / out_lo
  * [N,1024,C] bf16 pair of the result (out_lo may be NULL).  C must be a multiple of 64, N > 0, every pointer 16-byte aligned. */

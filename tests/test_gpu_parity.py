@@ -514,10 +514,13 @@ def test_sampling_S10_thresholds_fp32(dev, models, golden_dir):
     assert float((out - torch.from_numpy(g["sample"])).abs().max()) < 2e-3
 
 
+@pytest.mark.parametrize("docs", [3, 17])
 @pytest.mark.parametrize("prec", ["fp32", "bf16", "bf16x3"])
-def test_document_batch_equals_single_documents(dev, models, prec):
-    """Documents are independent: a batch of 3 documents gives the same maps as three separate calls."""
-    inps = [synth.make_doc_inputs(d, with_photo=False) for d in (0, 1, 5)]
+def test_document_batch_equals_single_documents(dev, models, prec, docs):
+    """Documents are independent: a batch of documents gives the same maps as separate calls.  17 documents are 34 samples, more
+    than the 32 of one fp32 attention chunk: the cross attention's second chunk reads K / V from document 16 (kv_div = 2), and the
+    self-attention (136 samples) runs in five chunks."""
+    inps = [synth.make_doc_inputs(d, with_photo=False) for d in ((0, 1, 5) if docs == 3 else range(docs))]
     cat = {k: torch.cat([i[k] for i in inps]) for k in inps[0]}
     both, _ = _sample(models[prec], cat)
     for j, i in enumerate(inps):
