@@ -56,6 +56,10 @@ class Y512Doc(C.Structure):
     _fields_ = [("photo", _vp), ("H", C.c_int32), ("W", C.c_int32)]
 
 
+class JpegDoc(C.Structure):
+    _fields_ = [("file_host", _vp), ("bytes", C.c_int64), ("file", _vp), ("out", _vp)]
+
+
 # name -> (restype, argtypes); mirrors include/dvd_b200.h one to one
 _i, _f, _sz = C.c_int, C.c_float, C.c_size_t
 _WP = C.POINTER(Weights)
@@ -77,6 +81,10 @@ SIGNATURES = {
     "dvd_y512_table_bytes": (_sz, [_i]),
     "dvd_y512_u8_plan": (_i, [C.POINTER(Y512Doc), _i, _vp, _sz]),
     "dvd_y512_u8": (_i, [_vp, _vp, _vp]),
+    "dvd_jpeg_table_bytes": (_sz, [_i]),
+    "dvd_jpeg_workspace_bytes": (_sz, [_i, C.c_longlong, C.c_longlong]),
+    "dvd_jpeg_plan": (_i, [C.POINTER(JpegDoc), _i, _vp, _sz, _sz, C.POINTER(C.c_int32)]),
+    "dvd_jpeg_decode": (_i, [_vp, _vp, _vp]),
     "dvd_grid_sample_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "dvd_fullres_grid_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _f, _vp]),
     "dvd_workspace_bytes": (_sz, [_i, _i, _i]),

@@ -26,7 +26,7 @@ if EXTRA:                                                   # instrumented build
     FLAGS += EXTRA
     BUILD = os.path.join(CSRC, "build_trace")
     LIB = os.path.join(HERE, "libdvd_b200_trace.so")
-SOURCES = ["api.cu", "unwarp.cu", "gemm_simt.cu", "misc.cu", "gemm_tc.cu", "gemm_pair.cu", "attn_tc.cu", "attn_pair.cu", "denoiser.cu", "prep.cu"]
+SOURCES = ["api.cu", "unwarp.cu", "gemm_simt.cu", "misc.cu", "gemm_tc.cu", "gemm_pair.cu", "attn_tc.cu", "attn_pair.cu", "denoiser.cu", "prep.cu", "jpeg.cu"]
 
 
 def _headers():

@@ -16,6 +16,11 @@ smaller pages are written and downloaded.
 With ``y512_from_photo=True`` the denoiser's 512x512 input is computed from ``photo_u8`` on the GPU (the reference loader's
 ``cv2.resize(photo, (512, 512), INTER_LINEAR) / 255``, byte for byte) by one launch at the head of the sampling graph; the input
 dicts then carry no ``y512`` and the host path uploads none.
+
+With ``max_jpeg_bytes=N`` the host path takes the camera's JPEG files instead of decoded photos: host dicts carry ``photo_jpeg``, a
+list of bytes-like files of at most N bytes each (fixed-size mode: exactly ``docs``, each ``height`` x ``width`` after its EXIF
+orientation).  Only the compressed bytes are uploaded; the decode (``inputs.decode_jpeg``'s launches, byte-equal to
+``cv2.imdecode``) heads the sampling graph and writes the photos where ``photo_u8`` would have been uploaded.
 """
 from __future__ import annotations
 
@@ -27,7 +32,8 @@ import torch
 
 from . import _lib
 from .model import DiT
-from .inputs import launch_y512, plan_y512, table_bytes as y512_table_bytes
+from .inputs import (jpeg_hw, jpeg_table_bytes, jpeg_workspace_bytes, launch_jpeg, launch_y512, pack_jpeg, plan_jpeg, plan_y512,
+                     table_bytes as y512_table_bytes)
 from .sampler import create_gaussian_diffusion
 from .unwarp import AFFINE, plan_mixed, plan_sized, size_arg, sized_table_bytes, supersample_arg, table_bytes
 
@@ -35,7 +41,8 @@ from .unwarp import AFFINE, plan_mixed, plan_sized, size_arg, sized_table_bytes,
 class DewarpPipeline:
     def __init__(self, model: DiT, diffusion_steps: int = 3, n_batch: int = 2, docs: int = 1, height: int = 1500, width: int = 2000,
                  noise_schedule: str = "cosine", precision: str | None = None, max_pixels: int | None = None, out_size=None,
-                 supersample="auto", max_out_pixels: int | None = None, y512_from_photo: bool = False):
+                 supersample="auto", max_out_pixels: int | None = None, y512_from_photo: bool = False,
+                 max_jpeg_bytes: int | None = None):
         self.model, self.docs, self.n_batch, self.H, self.W = model, docs, n_batch, height, width
         # y512 computed from photo_u8 by the first launch of the sampling graph instead of supplied by the caller
         self.y512_from_photo = bool(y512_from_photo)
@@ -45,6 +52,10 @@ class DewarpPipeline:
         self.max_pixels = max_pixels
         if max_pixels is not None and max_pixels < 1:
             raise ValueError(f"max_pixels must be positive, got {max_pixels}")
+        # host path: JPEG files of at most max_jpeg_bytes each, decoded by the first launches of the sampling graph
+        self.max_jpeg_bytes = max_jpeg_bytes
+        if max_jpeg_bytes is not None and max_jpeg_bytes < 1:
+            raise ValueError(f"max_jpeg_bytes must be positive, got {max_jpeg_bytes}")
         # output size (None: the photo's).  Fixed-size mode: one (Ho, Wo) for the batch; mixed-size mode: per photo, into an arena
         # of max_out_pixels (default max_pixels)
         self.out_size, self.supersample = out_size, supersample_arg(supersample)
@@ -83,7 +94,14 @@ class DewarpPipeline:
             self.map64 = z(docs, 2, 64, 64)
             self.out_u8 = z(*oimg, dt=torch.uint8)
             self._device_tables = self._planned_tables()              # run_device's
-        self.h2d_bytes = sum(v.numel() * v.element_size() for k, v in self.buf.items() if k in self._input_keys + ("photo_u8",))
+            if max_jpeg_bytes is not None:
+                # one decode workspace: the kernels run one batch at a time on the caller's stream
+                px = docs * height * width if max_pixels is None else max_pixels
+                self._jpeg_arena = docs * ((max_jpeg_bytes + 15) & ~15)
+                self._jpeg_ws = torch.empty(jpeg_workspace_bytes(docs, px, self._jpeg_arena), dtype=torch.uint8, device=self.dev)
+        # bytes uploaded per batch: the inputs and the photos, or at most the compressed files
+        photo_bytes = self.buf["photo_u8"].numel() if max_jpeg_bytes is None else self._jpeg_arena
+        self.h2d_bytes = sum(v.numel() * v.element_size() for k, v in self.buf.items() if k in self._input_keys) + photo_bytes
         self.d2h_bytes = self.out_u8.numel()
         self.use_graph = os.environ.get("DVD_NO_GRAPH", "0") != "1"
         self.kernel_launches = 0           # kernels of libdvd_b200 launched (or replayed) through this pipeline
@@ -112,6 +130,8 @@ class DewarpPipeline:
             tables["unwarp"] = _lib.PlannedTable(self._unwarp_bytes, self.dev)
         if self.y512_from_photo:
             tables["prep"] = _lib.PlannedTable(y512_table_bytes(self.docs), self.dev)
+        if self.max_jpeg_bytes is not None:
+            tables["jpeg"] = _lib.PlannedTable(jpeg_table_bytes(self.docs), self.dev)
         return tables
 
     # ---- device-resident inputs: dict with y512, mask_cat, mask_y512, line_msk, x_T, photo_u8 (all on self.dev)
@@ -125,6 +145,11 @@ class DewarpPipeline:
         launch_y512(d["prep"], d["y512"])
         self._enqueue_sampling(d)
 
+    def _enqueue_decode_sampling(self, d: dict):
+        """the JPEG decode planned into the device table d["jpeg_table"] (writes the batch's photos), then the sampling"""
+        launch_jpeg(d["jpeg_table"], self._jpeg_ws)
+        self._sampling(d)
+
     def _enqueue_unwarp(self, d: dict):
         """fused upsample + affine + bilinear unwarp of the full-resolution photos d["photo_u8"] into d["out_u8"], on the current
         stream."""
@@ -136,11 +161,18 @@ class DewarpPipeline:
         fn = self._unwarp_launch
         _lib.check(getattr(self.lib, fn)(_lib.ptr(d["table"]), 3, _lib.ptr(self.map64), _lib.stream_ptr()), fn)
 
-    def _sample(self, d: dict, photos, tables: dict):
-        """the sampling graph on the current stream; with y512_from_photo its first launch reads a y512 table planned from `photos`"""
+    def _sample(self, d: dict, photos, tables: dict, jpeg=None):
+        """the sampling graph on the current stream; with y512_from_photo its first launch reads a y512 table planned from `photos`.
+        jpeg = (files, device arena, offsets): the graph begins with the decode of the files into `photos`."""
         if self.y512_from_photo:
             d = dict(d, prep=tables["prep"].upload(lambda host: plan_y512(host, photos)))
-        self._run("sampling", d, self._sampling_keys, self._sampling)
+        if jpeg is None:
+            self._run("sampling", d, self._sampling_keys, self._sampling)
+            return
+        files, arena, offsets = jpeg
+        outs = list(photos.unbind(0)) if isinstance(photos, torch.Tensor) else photos
+        d = dict(d, jpeg_table=tables["jpeg"].upload(lambda host: plan_jpeg(files, host, self._jpeg_ws.numel(), arena, offsets, outs)))
+        self._run("decode_sampling", d, self._sampling_keys + ("jpeg_table",), self._enqueue_decode_sampling)
 
     def _unwarp(self, photos, outs, tables: dict):
         """the unwarp graph on the current stream: photos -> outs with the rows of map64"""
@@ -175,7 +207,12 @@ class DewarpPipeline:
         have one row per photo (x_T n_batch rows)."""
         if self.y512_from_photo and "y512" in d:
             raise ValueError("this pipeline computes y512 from photo_u8 (y512_from_photo=True); do not pass y512")
-        photos = self._check_photos(d["photo_u8"], self.dev if on_device else torch.device("cpu"), self.docs if on_device else 1)
+        if self.max_jpeg_bytes is not None and not on_device:
+            if "photo_u8" in d:
+                raise ValueError("this pipeline takes JPEG files on the host path (max_jpeg_bytes): pass photo_jpeg, not photo_u8")
+            photos = self._check_jpeg(d.get("photo_jpeg"))
+        else:
+            photos = self._check_photos(d["photo_u8"], self.dev if on_device else torch.device("cpu"), self.docs if on_device else 1)
         n = len(photos)
         for k in self._input_keys:
             t = d[k]
@@ -214,6 +251,31 @@ class DewarpPipeline:
         if px > self.max_pixels:
             raise ValueError(f"the batch has {px} pixels, more than max_pixels={self.max_pixels}")
         return list(photos)
+
+    def _check_jpeg(self, files) -> list:
+        """Validates the JPEG files of a host batch (fixed-size mode: docs files of height x width; mixed-size mode: 1..docs files
+        with at most max_pixels in all; each at most max_jpeg_bytes and one the decoder takes); returns the photo shapes [H,W,3]."""
+        if not isinstance(files, (list, tuple)):
+            raise ValueError("photo_jpeg: expected a list of JPEG files (bytes-like)")
+        lo = self.docs if self.max_pixels is None else 1
+        if not lo <= len(files) <= self.docs:
+            raise ValueError(f"{len(files)} JPEG files: this call takes {lo}..{self.docs}" if lo < self.docs else
+                             f"{len(files)} JPEG files: this call takes exactly {self.docs}")
+        for i, f in enumerate(files):
+            try:
+                n = memoryview(f).nbytes
+            except TypeError:
+                raise ValueError(f"photo_jpeg {i}: expected a bytes-like JPEG file, got {type(f).__name__}") from None
+            if n > self.max_jpeg_bytes:
+                raise ValueError(f"photo_jpeg {i} has {n} bytes, more than max_jpeg_bytes={self.max_jpeg_bytes}")
+        hw = jpeg_hw(files)
+        if self.max_pixels is None:
+            for i, s in enumerate(hw):
+                if s != (self.H, self.W):
+                    raise ValueError(f"photo_jpeg {i} decodes to {s[0]}x{s[1]}, this pipeline takes {self.H}x{self.W}")
+        elif sum(H * W for H, W in hw) > self.max_pixels:
+            raise ValueError(f"the batch has {sum(H * W for H, W in hw)} pixels, more than max_pixels={self.max_pixels}")
+        return [(H, W, 3) for H, W in hw]
 
     @staticmethod
     def _arena_views(arena: torch.Tensor, photos) -> list:
@@ -281,6 +343,9 @@ class DewarpPipeline:
         for _ in range(2):
             buf = {k: torch.empty_like(v) for k, v in self.buf.items()}
             buf["out_u8"] = torch.empty_like(self.out_u8)
+            if self.max_jpeg_bytes is not None:                   # the compressed files: pinned staging and device copy
+                buf["jpeg"] = torch.empty(self._jpeg_arena, dtype=torch.uint8, device=self.dev)
+                buf["jpeg_host"] = torch.empty(self._jpeg_arena, dtype=torch.uint8, pin_memory=True)
             self._slots.append({"buf": buf, "out_host": torch.empty(self.out_u8.shape, dtype=torch.uint8, pin_memory=True),
                                 "tables": self._planned_tables(), "result": None, "used": False, "ev_in": torch.cuda.Event(),
                                 "ev_photo": torch.cuda.Event(), "ev_done": torch.cuda.Event(), "ev_out": torch.cuda.Event()})
@@ -292,7 +357,10 @@ class DewarpPipeline:
         its upload also runs underneath this batch's own sampling.
 
         Mixed-size mode: h["photo_u8"] is a list of 1..docs uint8 HWC host photos and the other inputs have that many documents
-        (x_T that many times n_batch); document slots past the list keep their earlier inputs, are sampled and not unwarped."""
+        (x_T that many times n_batch); document slots past the list keep their earlier inputs, are sampled and not unwarped.
+
+        With max_jpeg_bytes, h["photo_jpeg"] (a list of JPEG files) replaces h["photo_u8"]: the files are packed into the slot's pinned
+        staging block, uploaded on the copy stream and decoded at the head of the sampling graph."""
         self._check_weights()
         photos = self._check_inputs(h, on_device=False)
         with torch.cuda.device(self.dev):
@@ -302,7 +370,15 @@ class DewarpPipeline:
             ticket = self._submitted
             s = self._slots[ticket % 2]
             buf = s["buf"]
-            photo_dev, out_dev = self._place(buf["photo_u8"], photos), self._outputs(buf["out_u8"], photos)
+            photo_dev = self._place(buf["photo_u8"], photos)
+            out_dev = self._outputs(buf["out_u8"], photo_dev if self.max_jpeg_bytes is not None else photos)
+            jpeg = None
+            if self.max_jpeg_bytes is not None:
+                if s["used"]:
+                    s["ev_photo"].synchronize()                    # the upload of batch ticket-2 has read the staging block
+                files = h["photo_jpeg"]
+                offsets = pack_jpeg(files, buf["jpeg_host"])
+                jpeg = (files, buf["jpeg"], offsets)
             self._submitted += 1
             with torch.cuda.stream(self._h2d):
                 if s["used"]:
@@ -310,16 +386,20 @@ class DewarpPipeline:
                 for k in self._input_keys:
                     buf[k][:h[k].shape[0]].copy_(h[k], non_blocking=True)
                 s["ev_in"].record()
-                if self.max_pixels is None:
+                if jpeg is not None:
+                    end = offsets[-1] + memoryview(files[-1]).nbytes
+                    buf["jpeg"][:end].copy_(buf["jpeg_host"][:end], non_blocking=True)
+                elif self.max_pixels is None:
                     photo_dev.copy_(photos, non_blocking=True)
                 else:
                     for dst, src in zip(photo_dev, photos):
                         dst.copy_(src, non_blocking=True)
                 s["ev_photo"].record()
-            main.wait_event(s["ev_photo"] if self.y512_from_photo else s["ev_in"])      # y512 from the photo: sampling reads it
+            # y512 from the photo, or the decode at the head of the sampling graph: sampling reads the photo upload
+            main.wait_event(s["ev_photo"] if self.y512_from_photo or jpeg is not None else s["ev_in"])
             if s["used"]:
                 main.wait_event(s["ev_out"])                       # the download of batch ticket-2 has read this slot's output
-            self._sample(buf, photo_dev, s["tables"])
+            self._sample(buf, photo_dev, s["tables"], jpeg)
             main.wait_event(s["ev_photo"])
             self._unwarp(photo_dev, out_dev, s["tables"])
             s["ev_done"].record(main)

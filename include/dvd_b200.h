@@ -183,6 +183,30 @@ DVD_API size_t dvd_y512_table_bytes(int max_docs);
 DVD_API int dvd_y512_u8_plan(const dvd_y512_doc_t* docs_host, int n_docs, void* table_host, size_t table_bytes);
 /* one launch; writes documents 0..n_docs-1 of y512 [>= n_docs,3,512,512] fp32 and nothing else */
 DVD_API int dvd_y512_u8(const void* table, float* y512, void* stream);
+/* ---- input decode: baseline / extended sequential 8-bit Huffman JPEG files (one interleaved scan; YCbCr 4:4:4, 4:2:2, 4:2:0 or
+ * grayscale; with or without restart intervals) to uint8 HWC RGB, byte-equal to cv2.imdecode(buf, IMREAD_COLOR)[..., ::-1]: the EXIF
+ * orientation is applied.  dvd_jpeg_plan parses the headers on the host (no CUDA call, never the entropy-coded bytes) and fills a
+ * table; the caller copies it to the device and dvd_jpeg_decode enqueues a fixed sequence of launches that depends on the device only,
+ * so a CUDA graph captured once serves every batch planned into the same device table.  A corrupt scan inside a well-formed file
+ * decodes to unspecified pixels of that document only. */
+typedef struct dvd_jpeg_doc {
+  const uint8_t* file_host;             /* the JPEG file, host                                  */
+  int64_t bytes;                        /* its length                                           */
+  const uint8_t* file;                  /* the same bytes, device (the compressed arena)        */
+  uint8_t* out;                         /* [Ho,Wo,3] uint8 RGB, device (Ho x Wo after orientation) */
+} dvd_jpeg_doc_t;
+/* bytes of a table for up to max_docs documents */
+DVD_API size_t dvd_jpeg_table_bytes(int max_docs);
+/* workspace for up to max_docs documents with at most max_pixels pixels and max_jpeg_bytes bytes IN ALL, each with sides within
+ * about 1:5 (dvd_jpeg_plan checks the batch it is given against the workspace it will use) */
+DVD_API size_t dvd_jpeg_workspace_bytes(int max_docs, long long max_pixels, long long max_jpeg_bytes);
+/* host only: parses and validates every file (a file the decoder does not take is rejected with the reason), writes out_hw[2d],
+ * out_hw[2d+1] = the output height and width of document d (may be NULL) and fills table_host.  With table_host NULL it only
+ * validates and reports sizes (the device pointers and the workspace are not looked at). */
+DVD_API int dvd_jpeg_plan(const dvd_jpeg_doc_t* docs_host, int n_docs, void* table_host, size_t table_bytes, size_t workspace_bytes,
+                          int32_t* out_hw);
+/* the decode of the uploaded plan; workspace: 256-byte aligned, at least the workspace_bytes the plan was given */
+DVD_API int dvd_jpeg_decode(const void* table, void* workspace, void* stream);
 /* WP:14-23,50-73 register_model2 / SpatialTransformer2: generic bilinear grid_sample,
  * align_corners=True, zeros padding.  img [B,C,H,W], grid [B,2,Ho,Wo] (ch0=x, ch1=y), out [B,C,Ho,Wo]. */
 DVD_API int dvd_grid_sample_f32(const float* img, const float* grid, float* out, int B, int C, int H, int W,
